@@ -3,7 +3,7 @@
 Adam) on synthetic periodic 2-D RVE meshes -- BASELINE.json configs[1]
 ("config_train_no_div.yml ... synthetic meshes batch 32, 1 B200").
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--config 4] [--lean]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--config 4] [--lean] [--dump-outputs DIR]
 
 One JSON line on stdout (rank 0).  See DESIGN.md "Measurement" for every field.
   value        whole-job nodes/s, inputs resident in HBM, K steps, CUDA events, max over ranks
@@ -37,7 +37,6 @@ sys.path.insert(0, ROOT)
 import torch  # noqa: E402
 
 B_DEFAULT, NODES_DEFAULT, T_STEPS = 32, 1024, 10
-REFERENCE_TIME_BUDGET_S = 420.0  # the reference arm shortens its run only if the full one would exceed this
 
 
 def parse():
@@ -58,7 +57,18 @@ def parse():
                     help="1 = configs[1] (default line); 4 = configs[4]: epoch over a >= 10k-mesh on-disk dataset, sharded")
     ap.add_argument("--meshes", type=int, default=10240, help="--config 4: dataset size")
     ap.add_argument("--distinct", type=int, default=128, help="--config 4: distinct mesh geometries generated")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed training step returned (loss terms, prediction, "
+                         "parameters and gradients after the optimizer step) as DIR/<name>.npy, at most 64 MB in all "
+                         "(rank 0; the inputs are seeded, so two builds run with the same arguments can be compared file by file; "
+                         "--impl reference writes the same files for the oracle port, after the same number of steps when "
+                         "--warmup >= 3; not with --config 4)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.config != 1:
+        ap.error("--dump-outputs writes the outputs of the configs[1] training step; --config 4 times whole epochs")
+    return args
 
 
 # ---------------------------------------------------------------------------------------
@@ -78,8 +88,9 @@ def oracle_case_from(samples):
     return O, O.collate(graphs), O.dataset_stats(graphs)
 
 
-def oracle_train_rate(n_graphs, nodes, divergence, steps, warmup, device="cpu", budget_s=None):
-    """fwd + loss + bwd + torch.optim.Adam of the oracle port on `device`; returns a dict."""
+def oracle_train_rate(n_graphs, nodes, divergence, steps, warmup, device="cpu", dump=None):
+    """fwd + loss + bwd + torch.optim.Adam of the oracle port on `device`, max(1, warmup) warm-up steps then `steps` timed
+    ones; returns a dict.  With `dump`, writes the last timed step's outputs there (dump_outputs)."""
     O, batch, stats = oracle_case(n_graphs, nodes)
     if device == "cpu":
         torch.set_num_threads(os.cpu_count() or 1)
@@ -91,27 +102,21 @@ def oracle_train_rate(n_graphs, nodes, divergence, steps, warmup, device="cpu", 
     params = {k: v.clone().to(device).requires_grad_(True) for k, v in sd.items()}
     opt = torch.optim.Adam(list(params.values()), lr=1e-3)
 
+    last = {}
+
     def step():
         total, nmse, div, pred = O.train_loss(params, batch, stats, T_STEPS, bool(divergence), 10.0)
         opt.zero_grad()
         total.backward()
         opt.step()
-        return total
+        last.update(loss=total.detach(), nmse=nmse.detach(), div=div.detach(), local_stress=pred.detach())
 
     def sync():
         if device != "cpu":
             torch.cuda.synchronize()
 
-    t_first = time.perf_counter()
-    step()
-    sync()
-    t_first = time.perf_counter() - t_first
-    shortened = None
-    if budget_s is not None and t_first * (steps + warmup) > budget_s:  # host too slow for the full run: say so
-        k = max(1, int(budget_s / t_first) - 1)
-        shortened = {"requested_steps": steps, "requested_warmup": warmup}
-        warmup, steps = min(warmup, 1), max(1, k - 1)
-    for _ in range(max(0, warmup - 1)):
+    warmup = max(1, warmup)
+    for _ in range(warmup):
         step()
     sync()
     if device == "cpu":
@@ -127,9 +132,14 @@ def oracle_train_rate(n_graphs, nodes, divergence, steps, warmup, device="cpu", 
         e1.record()
         torch.cuda.synchronize()
         dt = e0.elapsed_time(e1) * 1e-3 / steps
+    if dump:
+        out = {k: v.cpu().numpy() for k, v in last.items()}
+        for k, p in params.items():
+            out["param." + k] = p.detach().cpu().numpy()
+            out["grad." + k] = p.grad.cpu().numpy()
+        dump_outputs(dump, out)
     return {"value": batch.num_nodes / dt, "s_per_step": dt, "nodes": int(batch.num_nodes), "graphs": n_graphs,
-            "steps": steps, "warmup": warmup, "cores": torch.get_num_threads() if device == "cpu" else None,
-            "shortened": shortened}
+            "steps": steps, "warmup": warmup, "cores": torch.get_num_threads() if device == "cpu" else None}
 
 
 def oracle_forward_ms(n_graphs, nodes, device, reps):
@@ -170,6 +180,30 @@ def emit(line):
     out.flush()
 
 
+DUMP_LIMIT_BYTES = 64 * 10**6
+
+
+def dump_outputs(folder, arrays, limit=DUMP_LIMIT_BYTES):
+    """Write every array as folder/<name>.npy, float64 kept, everything else as float32, at most `limit` bytes of files
+    in all.  Arrays are written smallest first; one that no longer fits whole keeps a sample of its rows (along axis 0)
+    drawn from a generator seeded with 0 and sorted, so the same shapes always give the same rows."""
+    import numpy as np
+    header = 1024  # reserved for each .npy header
+    os.makedirs(folder, exist_ok=True)
+    left = limit
+    for name, a in sorted(arrays.items(), key=lambda kv: (np.size(kv[1]), kv[0])):
+        a = np.asarray(a)
+        a = a if a.dtype == np.float64 else a.astype(np.float32)
+        if a.nbytes + header > left:
+            rows = max(0, left - header) // (a.nbytes // a.shape[0]) if a.ndim and a.shape[0] else 0
+            if rows == 0:
+                raise ValueError(f"--dump-outputs: {name} {a.shape} does not fit the {limit}-byte limit")
+            a = a[np.sort(np.random.default_rng(0).choice(a.shape[0], rows, replace=False))]
+        path = os.path.join(folder, name + ".npy")
+        np.save(path, a)
+        left -= os.path.getsize(path)
+
+
 METRIC = "mesh nodes/sec, P-GNN training step (fwd+loss+bwd+Adam)"
 
 
@@ -178,7 +212,7 @@ def run_reference(args, rank):
     32-mesh batch per step, the same steps and warm-up.  Rank 0 only."""
     if rank != 0:
         return
-    r = oracle_train_rate(args.batch, args.nodes, args.divergence, args.steps, args.warmup, "cpu", REFERENCE_TIME_BUDGET_S)
+    r = oracle_train_rate(args.batch, args.nodes, args.divergence, args.steps, args.warmup, "cpu", args.dump_outputs)
     sample = (f"the full configs[1] batch: {r['graphs']} meshes x ~{args.nodes} nodes ({r['nodes']} nodes) per step, "
               f"{r['warmup']} warm-up + {r['steps']} timed steps, {r['s_per_step']:.2f} s/step")
     line = {
@@ -190,8 +224,6 @@ def run_reference(args, rank):
         "e2e": {"value": r["value"], "unit": "nodes/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
         "note": "oracle port (pure-torch CPU restatement of the reference path); the reference needs torch_geometric",
     }
-    if r["shortened"]:
-        line["shortened"] = {**r["shortened"], "why": f"the full run would exceed {REFERENCE_TIME_BUDGET_S:.0f} s on this host"}
     emit(line)
 
 
@@ -275,7 +307,18 @@ class Arm:
         self.opt.zero_grad(set_to_none=True)
         loss.backward()
         self.opt.step()
+        # detached: holding `pred` itself would keep the step's autograd state (the saved workspace) alive
+        self.last = {"loss": loss.detach(), "nmse": nmse.detach(), "div": dv.detach(), "local_stress": pred.detach()}
         return loss
+
+    def last_outputs(self):
+        """What the last train_step handed its caller, as host arrays: the loss terms, the standardised prediction
+        (nodes x 3) and every parameter and its gradient after the optimizer step (state_dict names)."""
+        out = {k: v.cpu().numpy() for k, v in self.last.items()}
+        for k, p in self.model.named_parameters():
+            out["param." + k] = p.detach().cpu().numpy()
+            out["grad." + k] = p.grad.cpu().numpy()
+        return out
 
     def params_identical_across_ranks(self):
         """SURVEY 8e: identical parameters on all ranks after every step (checked once, after the timed regions)."""
@@ -777,6 +820,8 @@ def main():
     time.sleep(0.25)
     ms, t0, t1, launches = time_resident(arm, resident, args.steps, args.warmup, world)  # launches: timed steps only
     clk = clocks.stop(t0, t1)
+    if args.dump_outputs and rank == 0:  # before the passes below train the same model further
+        dump_outputs(args.dump_outputs, arm.last_outputs())
     ms_k, ksteps, ktimes = kernel_pass(arm, resident, args.steps, world)
     h2d = batcher.host_bytes(host[0], with_op)
     e2e_ms, nodes_e2e = time_e2e(arm, host, args.steps, args.warmup, world, with_op)
