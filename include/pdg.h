@@ -129,13 +129,22 @@ int pdg_ws_offset(int64_t n_nodes, int64_t n_edges, int steps, int flags, int wh
 
 /* ---- model backward: d loss / d params given d loss / d local_stress [N,3] ----------
  * grads_flat: PDG_PARAM_ELEMS floats, state_dict order, overwritten (not accumulated).
- * Inputs (mean_stress, pos, ...) are not differentiated (the reference never does).
+ * pdg_backward differentiates the parameters only; pdg_backward_inputs, with the same arguments, also writes the
+ * gradients of the differentiable inputs of models.py:140-162 into each non-NULL output (overwritten, not
+ * accumulated; the parameter gradients are the same bits either way):
+ *   grad_mean_stress [N,3], grad_pos [N,2], grad_edge_attr [E] in the caller's (PyG) edge order.
+ * nodes_types is an integer input and has no gradient.  pdg_backward is pdg_backward_inputs with three NULLs.
  * Replaces torch autograd through models.py:288-326. */
 size_t pdg_backward_ws_bytes(int64_t n_nodes, int64_t n_edges, int steps);
 int pdg_backward(const pdg_params_t* params, const pdg_norm_t* norm, const float* mean_stress, const float* pos,
                  const int64_t* nodes_types, const float* edge_attr, const void* plan, int64_t n_nodes,
                  int64_t n_edges, int steps, int flags, int precision, void* fwd_ws, void* bwd_ws, size_t bwd_ws_bytes,
                  const float* grad_local_stress, float* grads_flat, void* stream);
+int pdg_backward_inputs(const pdg_params_t* params, const pdg_norm_t* norm, const float* mean_stress, const float* pos,
+                        const int64_t* nodes_types, const float* edge_attr, const void* plan, int64_t n_nodes,
+                        int64_t n_edges, int steps, int flags, int precision, void* fwd_ws, void* bwd_ws,
+                        size_t bwd_ws_bytes, const float* grad_local_stress, float* grads_flat,
+                        float* grad_mean_stress, float* grad_pos, float* grad_edge_attr, void* stream);
 
 /* ---- loss: per-graph NMSE + divergence regulariser, batch means ---------------------
  * Replaces the per-graph Python loop of train() (gnn_train.py:162-202):

@@ -58,6 +58,8 @@ _SIGS = {
     "pdg_backward_ws_bytes": (_sz, [_i64, _i64, _i32]),
     "pdg_backward": (_i32, [C.POINTER(PdgParams), C.POINTER(PdgNorm), _vp, _vp, _vp, _vp, _vp, _i64, _i64, _i32, _i32,
                             _i32, _vp, _vp, _sz, _vp, _vp, _vp]),
+    "pdg_backward_inputs": (_i32, [C.POINTER(PdgParams), C.POINTER(PdgNorm), _vp, _vp, _vp, _vp, _vp, _i64, _i64, _i32,
+                                   _i32, _i32, _vp, _vp, _sz, _vp, _vp, _vp, _vp, _vp, _vp]),
     "pdg_opdiv_plan_bytes": (_sz, [_i64, _i64]),
     "pdg_opdiv_tmp_bytes": (_sz, [_i64, _i64]),
     "pdg_opdiv_plan_build": (_i32, [_vp, _vp, _i64, _vp, _i64, _i64, _vp, _vp, _sz, _vp]),

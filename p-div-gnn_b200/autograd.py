@@ -2,7 +2,7 @@
 
 Nothing here computes; it validates inputs, builds / caches the device graph plan,
 allocates the workspace from torch's caching allocator (so stream semantics hold) and
-calls ``pdg_forward`` / ``pdg_backward`` on the current CUDA stream.
+calls ``pdg_forward`` / ``pdg_backward_inputs`` on the current CUDA stream.
 """
 from __future__ import annotations
 
@@ -149,31 +149,37 @@ class _EPDFunction(torch.autograd.Function):
     @staticmethod
     def backward(ctx, grad_out):
         L = _lib.lib()
-        if not hasattr(L, "pdg_backward") or getattr(L.pdg_backward, "argtypes", None) is None:
-            raise RuntimeError("libpdivgnn.so was built without pdg_backward")
+        if not hasattr(L, "pdg_backward_inputs") or getattr(L.pdg_backward_inputs, "argtypes", None) is None:
+            raise RuntimeError("libpdivgnn.so was built without pdg_backward_inputs")
         model, plan, mean_stress, pos, types, edge_attr, flags, steps, prec, params, ws, norm = ctx.pdg
         dev = grad_out.device
         n, e = plan.n_nodes, plan.n_edges
         grad_out = _lib.require_cuda(grad_out, "grad_local_stress", torch.float32)
+        need = ctx.needs_input_grad  # slots 2, 3, 5: mean_stress, pos, edge_attr
         with torch.cuda.device(dev):
             flat = torch.empty(_lib.PDG_PARAM_ELEMS, dtype=torch.float32, device=dev)
+            g_ms = torch.empty((n, 3), dtype=torch.float32, device=dev) if need[2] else None
+            g_pos = torch.empty((n, 2), dtype=torch.float32, device=dev) if need[3] else None
+            g_ea = torch.empty(e, dtype=torch.float32, device=dev) if need[5] else None
             bws_bytes = L.pdg_backward_ws_bytes(n, e, steps)
             bws = torch.empty(_bucket(bws_bytes), dtype=torch.uint8, device=dev)
             ps = _params_struct(params)
-            _lib.check(L.pdg_backward(C.byref(ps), C.byref(norm), _lib.ptr(mean_stress), _lib.ptr(pos), _lib.ptr(types),
-                                      _lib.ptr(edge_attr), _lib.ptr(plan.buf), n, e, steps, flags, prec, _lib.ptr(ws),
-                                      _lib.ptr(bws), bws_bytes, _lib.ptr(grad_out), _lib.ptr(flat),
-                                      _lib.stream_ptr(dev)), "pdg_backward")
+            _lib.check(L.pdg_backward_inputs(C.byref(ps), C.byref(norm), _lib.ptr(mean_stress), _lib.ptr(pos),
+                                             _lib.ptr(types), _lib.ptr(edge_attr), _lib.ptr(plan.buf), n, e, steps, flags,
+                                             prec, _lib.ptr(ws), _lib.ptr(bws), bws_bytes, _lib.ptr(grad_out),
+                                             _lib.ptr(flat), _lib.ptr(g_ms), _lib.ptr(g_pos), _lib.ptr(g_ea),
+                                             _lib.stream_ptr(dev)), "pdg_backward_inputs")
         dp = getattr(model, "_pdg_dp", None)
-        if dp is not None and dp[0]:  # data parallel: one all-reduce of the flat buffer (dist.py)
+        # data parallel: one all-reduce of the flat buffer (dist.py); input gradients stay rank-local, as in torch DDP
+        if dp is not None and dp[0]:
             from .dist import allreduce_flat_
             allreduce_flat_(flat, dp[1], getattr(model, "_pdg_peer", None))
         grads, off = [], 0
-        for p in params:
-            grads.append(flat[off:off + p.numel()].view(p.shape))
+        for i, p in enumerate(params):
+            grads.append(flat[off:off + p.numel()].view(p.shape) if need[10 + i] else None)
             off += p.numel()
         ctx.pdg = None
-        return (None,) * 10 + tuple(grads)
+        return (None, None, g_ms, g_pos, None, g_ea) + (None,) * 4 + tuple(grads)
 
 
 # ---- CUDA-graph replay of the inference forward (small-N latency) ------------------------------------------------------
@@ -246,8 +252,10 @@ def epd_forward(model, mesh_graph, scale_output: bool, scale_input: bool, zero_c
         | (_lib.FLAG_ZERO_CHECK if zero_check else 0)
     prec = _lib.PREC_BF16 if getattr(model, "precision", "fp32") in ("bf16", "fp16", "tc16") else _lib.PREC_FP32
     params = param_list(model)
-    # grad mode is off inside Function.forward, so decide here whether the backward state must be kept
-    need_grad = torch.is_grad_enabled() and any(p.requires_grad for p in params)
+    # grad mode is off inside Function.forward, so decide here whether the backward state must be kept: a frozen model
+    # (no parameter requires grad) differentiated with respect to its inputs keeps it too
+    need_grad = torch.is_grad_enabled() and (mean_stress.requires_grad or pos.requires_grad or edge_attr.requires_grad
+                                             or any(p.requires_grad for p in params))
     if not need_grad and (getattr(model, "cuda_graphs", False) or _GRAPHS_ENV) and not torch.cuda.is_current_stream_capturing():
         return _forward_graphed(model, plan, mean_stress, pos, types, edge_attr, flags, model.message_passing_steps, prec,
                                 params)

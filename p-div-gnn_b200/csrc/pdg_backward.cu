@@ -721,14 +721,18 @@ __global__ void __launch_bounds__(NT, 1) k_node_pre_bwd(NodePreBwdArgs a) {
 }
 
 // ---- encoder backward (node: NODE=1, edge: NODE=0) -------------------------------------------
-template <int NODE>
+// IG: also write the input gradient dfeat = dh0 W0 of every row, un-standardised (models.py:140-162):
+//   node  gi0 = d/d mean_stress [N,3] (features 0-2), gi1 = d/d pos [N,2] (features 3-4), either may be null;
+//   edge  gi0 = d/d edge_attr [E] at perm[row] (PyG edge order; perm is a permutation: plain stores).
+// The <NODE, false> instances are the parameter-gradient-only kernels, unchanged.
+template <int NODE, bool IG>
 __global__ void __launch_bounds__(NT, 1)
 k_encoder_bwd(const float* __restrict__ g_in, const float* __restrict__ y_raw, const float* __restrict__ scal,
               const float* __restrict__ lnw, const float* __restrict__ mean_stress, const float* __restrict__ pos,
               const int64_t* __restrict__ types, const float* __restrict__ edge_attr, const int32_t* __restrict__ perm,
               pdg_norm_t nrm, int scale_in, const float* __restrict__ W0, const float* __restrict__ b0,
               const float* __restrict__ W2, float* __restrict__ cta_grads, int off_w0, int off_b0, int off_w2,
-              int off_b2, int R, int n_tiles) {
+              int off_b2, int R, int n_tiles, float* __restrict__ gi0, float* __restrict__ gi1) {
   extern __shared__ __align__(16) float smem[];
   float* T0 = smem;
   float* T1 = T0 + TM * LDS;
@@ -828,6 +832,30 @@ k_encoder_bwd(const float* __restrict__ g_in, const float* __restrict__ y_raw, c
 #pragma unroll
         for (int j = 0; j < NF; ++j) dW0[j] = fmaf(d, feat[r * 8 + j], dW0[j]);
       }
+    } else if (IG) {  // warps 4-7, idle in the walk above: dfeat[r] = dh0[r] W0, one warp per row, lane = 4 channels
+      constexpr int NI = NODE ? 5 : 1;  // feature 5 (nodes_types) is an integer input: no gradient
+      for (int r = (tid - H) >> 5; r < nvalid; r += (NT - H) / 32) {
+        const float4 d = *reinterpret_cast<const float4*>(T0 + r * LDS + c4);
+        float s[NI];
+#pragma unroll
+        for (int j = 0; j < NI; ++j) {
+          s[j] = fmaf(d.w, w0[3][j], fmaf(d.z, w0[2][j], fmaf(d.y, w0[1][j], d.x * w0[0][j])));
+#pragma unroll
+          for (int o = 16; o > 0; o >>= 1) s[j] += __shfl_xor_sync(0xffffffffu, s[j], o);
+        }
+        if ((tid & 31) == 0) {
+          const int row = row0 + r;
+          if (NODE) {
+            const float sm = scale_in ? nrm.std_mean_stress : 1.f, sp = scale_in ? nrm.std_pos : 1.f;
+            if (gi0 != nullptr) {
+              gi0[row * 3 + 0] = s[0] / sm; gi0[row * 3 + 1] = s[1 % NI] / sm; gi0[row * 3 + 2] = s[2 % NI] / sm;
+            }
+            if (gi1 != nullptr) { gi1[row * 2 + 0] = s[3 % NI] / sp; gi1[row * 2 + 1] = s[4 % NI] / sp; }
+          } else {
+            gi0[perm[row]] = s[0] / (scale_in ? nrm.std_edge_weight : 1.f);
+          }
+        }
+      }
     }
     __syncthreads();
   }
@@ -918,15 +946,16 @@ extern "C" size_t pdg_backward_ws_bytes(int64_t n_nodes, int64_t n_edges, int st
   return BwdWs(n_nodes, n_edges, steps, g, nullptr).total;
 }
 
-extern "C" int pdg_backward(const pdg_params_t* params, const pdg_norm_t* norm, const float* mean_stress,
-                            const float* pos, const int64_t* nodes_types, const float* edge_attr, const void* plan,
-                            int64_t n_nodes, int64_t n_edges, int steps, int flags, int precision, void* fwd_ws,
-                            void* bwd_ws, size_t bwd_ws_bytes, const float* grad_local_stress, float* grads_flat,
-                            void* stream_) {
+extern "C" int pdg_backward_inputs(const pdg_params_t* params, const pdg_norm_t* norm, const float* mean_stress,
+                                   const float* pos, const int64_t* nodes_types, const float* edge_attr, const void* plan,
+                                   int64_t n_nodes, int64_t n_edges, int steps, int flags, int precision, void* fwd_ws,
+                                   void* bwd_ws, size_t bwd_ws_bytes, const float* grad_local_stress, float* grads_flat,
+                                   float* grad_mean_stress, float* grad_pos, float* grad_edge_attr, void* stream_) {
   cudaStream_t st = (cudaStream_t)stream_;
   if (steps < 1 || steps > 62) { set_error("pdg_backward: steps=%d unsupported", steps); return -1; }
   if (!(flags & PDG_FLAG_SAVE)) { set_error("pdg_backward: forward was not run with PDG_FLAG_SAVE"); return -1; }
   if (precision != PDG_PREC_FP32 && precision != PDG_PREC_BF16) { set_error("pdg_backward: unknown precision mode %d", precision); return -1; }
+  const bool ig_node = grad_mean_stress != nullptr || grad_pos != nullptr, ig_edge = grad_edge_attr != nullptr;
   int G = num_sms();
   if (G > MAXP) G = MAXP;
   const bool tcm = precision == PDG_PREC_BF16;
@@ -946,8 +975,8 @@ extern "C" int pdg_backward(const pdg_params_t* params, const pdg_norm_t* norm, 
   if (set_smem_b((const void*)k_node_update_bwd, SMEM_B3T)) return -2;
   if (set_smem_b((const void*)k_edge_step_bwd, SMEM_B3T)) return -2;
   if (set_smem_b((const void*)k_node_pre_bwd, SMEM_B3T)) return -2;
-  if (set_smem_b((const void*)k_encoder_bwd<1>, SMEM_B3T)) return -2;
-  if (set_smem_b((const void*)k_encoder_bwd<0>, SMEM_B3T)) return -2;
+  if (set_smem_b(ig_node ? (const void*)k_encoder_bwd<1, true> : (const void*)k_encoder_bwd<1, false>, SMEM_B3T)) return -2;
+  if (set_smem_b(ig_edge ? (const void*)k_encoder_bwd<0, true> : (const void*)k_encoder_bwd<0, false>, SMEM_B3T)) return -2;
 
   PDG_CUDA_CHECK(cudaMemsetAsync(B.cta_grads, 0, (size_t)G * GRADP * sizeof(float), st));
   PDG_CUDA_CHECK(cudaMemsetAsync(grads_flat, 0, (size_t)PDG_PARAM_ELEMS * sizeof(float), st));
@@ -1059,11 +1088,12 @@ extern "C" int pdg_backward(const pdg_params_t* params, const pdg_norm_t* norm, 
     ScopedTimer tm_(KC_ENC_BWD, st);
     if (tcm) {
       if (launch_node_encoder_bwd_tc(B.gx, W.y_nenc, scal(0), P[NE_LNW], mean_stress, pos, nodes_types, norm, scale_in, P[NE_W0],
-                                     P[NE_B0], B.cta_grads, N, nt_n, grid_n, W.img, st)) return -2;
+                                     P[NE_B0], B.cta_grads, gs, grad_mean_stress, grad_pos, N, nt_n, grid_n, W.img, st)) return -2;
     } else {
-      PDG_CUDA_CHECK(launch_pdl(k_encoder_bwd<1>, dim3(grid_n), dim3(NT), SMEM_B3T, st, B.gx, W.y_nenc, scal(0), P[NE_LNW], mean_stress,
-                                pos, nodes_types, nullptr, nullptr, *norm, scale_in, P[NE_W0], P[NE_B0], P[NE_W2], B.cta_grads,
-                                param_offset(NE_W0), param_offset(NE_B0), param_offset(NE_W2), param_offset(NE_B2), N, nt_n));
+      PDG_CUDA_CHECK(launch_pdl(ig_node ? k_encoder_bwd<1, true> : k_encoder_bwd<1, false>, dim3(grid_n), dim3(NT), SMEM_B3T, st, B.gx,
+                                W.y_nenc, scal(0), P[NE_LNW], mean_stress, pos, nodes_types, nullptr, nullptr, *norm, scale_in, P[NE_W0],
+                                P[NE_B0], P[NE_W2], B.cta_grads, param_offset(NE_W0), param_offset(NE_B0), param_offset(NE_W2),
+                                param_offset(NE_B2), N, nt_n, grad_mean_stress, grad_pos));
     }
   }
   PDG_LAUNCH_CHECK();
@@ -1071,12 +1101,12 @@ extern "C" int pdg_backward(const pdg_params_t* params, const pdg_norm_t* norm, 
     ScopedTimer tm_(KC_ENC_BWD, st);
     if (tcm) {
       if (launch_edge_encoder_bwd_tc(B.ge, W.y_eenc, scal(1), P[EE_LNW], edge_attr, perm, norm, scale_in, P[EE_W0], P[EE_B0],
-                                     B.cta_grads, E, nt_e, grid_e, W.img, st)) return -2;
+                                     B.cta_grads, gs, grad_edge_attr, E, nt_e, grid_e, W.img, st)) return -2;
     } else {
-      k_encoder_bwd<0><<<grid_e, NT, SMEM_B3T, st>>>(B.ge, W.y_eenc, scal(1), P[EE_LNW], nullptr, nullptr, nullptr, edge_attr,
-                                                     perm, *norm, scale_in, P[EE_W0], P[EE_B0], P[EE_W2], B.cta_grads,
-                                                     param_offset(EE_W0), param_offset(EE_B0), param_offset(EE_W2),
-                                                     param_offset(EE_B2), E, nt_e);
+      (ig_edge ? k_encoder_bwd<0, true> : k_encoder_bwd<0, false>)<<<grid_e, NT, SMEM_B3T, st>>>(
+          B.ge, W.y_eenc, scal(1), P[EE_LNW], nullptr, nullptr, nullptr, edge_attr, perm, *norm, scale_in, P[EE_W0], P[EE_B0],
+          P[EE_W2], B.cta_grads, param_offset(EE_W0), param_offset(EE_B0), param_offset(EE_W2), param_offset(EE_B2), E, nt_e,
+          grad_edge_attr, nullptr);
     }
   }
   PDG_LAUNCH_CHECK();
@@ -1086,4 +1116,14 @@ extern "C" int pdg_backward(const pdg_params_t* params, const pdg_norm_t* norm, 
   }
   PDG_LAUNCH_CHECK();
   return 0;
+}
+
+extern "C" int pdg_backward(const pdg_params_t* params, const pdg_norm_t* norm, const float* mean_stress,
+                            const float* pos, const int64_t* nodes_types, const float* edge_attr, const void* plan,
+                            int64_t n_nodes, int64_t n_edges, int steps, int flags, int precision, void* fwd_ws,
+                            void* bwd_ws, size_t bwd_ws_bytes, const float* grad_local_stress, float* grads_flat,
+                            void* stream) {
+  return pdg_backward_inputs(params, norm, mean_stress, pos, nodes_types, edge_attr, plan, n_nodes, n_edges, steps, flags,
+                             precision, fwd_ws, bwd_ws, bwd_ws_bytes, grad_local_stress, grads_flat, nullptr, nullptr, nullptr,
+                             stream);
 }

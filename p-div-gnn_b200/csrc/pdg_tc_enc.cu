@@ -130,10 +130,17 @@ struct EdgeEncBwdArgs {
   const float* W0;
   const float* b0;
   float* cta_grads;
+  const float* gs;        // IG: device {S, 1/S} of k_grad_scale (the incoming gradient carries S)
+  float* g_edge_attr;     // IG: d loss / d edge_attr [E], PyG edge order
   int E, n_tiles;
 };
 constexpr int TC_SMEM_EDGE_ENC_BWD = 3 * tc::TILE_BF16_BYTES + TM * 4 + 4 * H * 4 + 512 + 2048;
+constexpr int TC_SMEM_EDGE_ENC_BWD_IG = TC_SMEM_EDGE_ENC_BWD + H * 4;  // + W0 [128]
 
+// IG: also write d loss / d edge_attr = (dh0 . W0) / std_edge_weight / S at perm[row], formed from the fp32 TMEM values of
+// dh0; the half-1 thread of a row hands its partial sum to the half-0 thread through its own (then dead) bytes of the h0
+// tile.  The <false> instance is unchanged.
+template <bool IG>
 __global__ void __launch_bounds__(NT, 1)
 k_edge_encoder_bwd_tc(EdgeEncBwdArgs a, const uint8_t* __restrict__ imgW2) {
   extern __shared__ uint8_t smem_raw[];
@@ -143,10 +150,12 @@ k_edge_encoder_bwd_tc(EdgeEncBwdArgs a, const uint8_t* __restrict__ imgW2) {
   uint8_t* T1 = T0 + tc::TILE_BF16_BYTES;   // h0
   float* feat = reinterpret_cast<float*>(T1 + tc::TILE_BF16_BYTES);
   float* comb = feat + TM;  // [4][H]
-  uint64_t* bars = reinterpret_cast<uint64_t*>(comb + 4 * H);
+  float* w0s = comb + 4 * H;  // IG: [H]
+  uint64_t* bars = reinterpret_cast<uint64_t*>(w0s + (IG ? H : 0));
   uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 2);
   const TcThread t;
   float* cg = a.cta_grads + (size_t)blockIdx.x * GRADP;
+  if (IG && t.tid < H) w0s[t.tid] = a.W0[t.tid];
   const uint32_t tmem = tc_setup_enc(bars, 2, tmem_slot, 256);
   const uint32_t ACC = tmem, WORK = tmem + 128;
   if (t.tid == 0) {
@@ -155,6 +164,7 @@ k_edge_encoder_bwd_tc(EdgeEncBwdArgs a, const uint8_t* __restrict__ imgW2) {
   }
   pdl_sync();  // scal / g_in / y_raw come from the preceding kernels
   const float c1 = a.scal[0], c2 = a.scal[1], mu = a.scal[2], rstd = a.scal[3];
+  const float iea = IG ? a.gs[1] / (a.scale_in ? a.std : 1.f) : 0.f;
   const int ch = t.tid & 15;
   float w0[8], b0[8], lw[8];
 #pragma unroll
@@ -206,6 +216,7 @@ k_edge_encoder_bwd_tc(EdgeEncBwdArgs a, const uint8_t* __restrict__ imgW2) {
     tc::mbar_wait(&bars[1], ph);
     tc::fence_after_sync();
     __syncthreads();  // every column walker is done with dy before the epilogue overwrites T0 with dh0
+    float gi = 0.f;
 #pragma unroll
     for (int hh = 0; hh < 2; ++hh) {
       float v[32];
@@ -218,10 +229,19 @@ k_edge_encoder_bwd_tc(EdgeEncBwdArgs a, const uint8_t* __restrict__ imgW2) {
 #pragma unroll
         for (int j = 0; j < 8; ++j) d[j] = h[j] > 0.f ? v[c8 * 8 + j] : 0.f;
         row_store8(T0, t.row, t.half, hh * 4 + c8, d);
+        if (IG) {
+          const float* w = w0s + t.half * 64 + hh * 32 + c8 * 8;  // warp-uniform: broadcast
+          const float4 wa = *reinterpret_cast<const float4*>(w), wb = *reinterpret_cast<const float4*>(w + 4);
+          gi = fmaf(d[0], wa.x, gi); gi = fmaf(d[1], wa.y, gi); gi = fmaf(d[2], wa.z, gi); gi = fmaf(d[3], wa.w, gi);
+          gi = fmaf(d[4], wb.x, gi); gi = fmaf(d[5], wb.y, gi); gi = fmaf(d[6], wb.z, gi); gi = fmaf(d[7], wb.w, gi);
+        }
       }
     }
+    if (IG && t.half == 1) *reinterpret_cast<float*>(T1 + tc::sw128_chunk(t.row, 8)) = gi;  // read above by this thread only
     tc::fence_before_sync();
     __syncthreads();
+    if (IG && t.half == 0 && t.row < nvalid)
+      a.g_edge_attr[a.perm[row0 + t.row]] = (gi + *reinterpret_cast<const float*>(T1 + tc::sw128_chunk(t.row, 8))) * iea;
     {  // db0 = colsum(dh0), dW0[c] = sum_r dh0[r][c] * feat[r]   (thread = channel pair x 32-row quarter)
       const int cp = t.tid & 63, q = t.tid >> 6;
       float s0 = 0.f, s1 = 0.f, u0 = 0.f, u1 = 0.f;
@@ -262,11 +282,17 @@ int launch_edge_encoder_tc(const float* edge_attr, const int32_t* perm, const pd
 }
 int launch_edge_encoder_bwd_tc(const float* g_in, const float* y_raw, const float* scal, const float* lnw, const float* edge_attr,
                                const int32_t* perm, const pdg_norm_t* nrm, int scale_in, const float* W0, const float* b0,
-                               float* cta_grads, int E, int n_tiles, int grid, const uint8_t* img, cudaStream_t st) {
-  cudaError_t e = cudaFuncSetAttribute((const void*)k_edge_encoder_bwd_tc, cudaFuncAttributeMaxDynamicSharedMemorySize, TC_SMEM_EDGE_ENC_BWD);
+                               float* cta_grads, const float* gs, float* grad_edge_attr, int E, int n_tiles, int grid,
+                               const uint8_t* img, cudaStream_t st) {
+  const bool ig = grad_edge_attr != nullptr;
+  const void* fn = ig ? (const void*)k_edge_encoder_bwd_tc<true> : (const void*)k_edge_encoder_bwd_tc<false>;
+  const int smem = ig ? TC_SMEM_EDGE_ENC_BWD_IG : TC_SMEM_EDGE_ENC_BWD;
+  cudaError_t e = cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
   if (e != cudaSuccess) { set_error("k_edge_encoder_bwd_tc smem attribute: %s", cudaGetErrorString(e)); return -2; }
-  EdgeEncBwdArgs a{g_in, y_raw, scal, lnw, edge_attr, perm, nrm->mean_edge_weight, nrm->std_edge_weight, scale_in, W0, b0, cta_grads, E, n_tiles};
-  e = launch_pdl(k_edge_encoder_bwd_tc, dim3(grid), dim3(NT), TC_SMEM_EDGE_ENC_BWD, st, a, img + (size_t)IMG_EE_W2 * tc::TILE_BF16_BYTES);
+  EdgeEncBwdArgs a{g_in, y_raw, scal, lnw, edge_attr, perm, nrm->mean_edge_weight, nrm->std_edge_weight, scale_in, W0, b0, cta_grads,
+                   gs, grad_edge_attr, E, n_tiles};
+  e = launch_pdl(ig ? k_edge_encoder_bwd_tc<true> : k_edge_encoder_bwd_tc<false>, dim3(grid), dim3(NT), smem, st, a,
+                 img + (size_t)IMG_EE_W2 * tc::TILE_BF16_BYTES);
   if (e != cudaSuccess) { set_error("k_edge_encoder_bwd_tc launch: %s", cudaGetErrorString(e)); return -2; }
   return 0;
 }

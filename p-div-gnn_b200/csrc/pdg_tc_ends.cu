@@ -181,10 +181,18 @@ struct NodeEncBwdArgs {
   const float* W0;
   const float* b0;
   float* cta_grads;
+  const float* gs;        // IG: device {S, 1/S} of k_grad_scale (the incoming gradient carries S)
+  float* g_mean_stress;   // IG: d loss / d mean_stress [N,3] or null
+  float* g_pos;           // IG: d loss / d pos [N,2] or null
   int N, n_tiles;
 };
 constexpr int TC_SMEM_NODE_ENC_BWD = 3 * tc::TILE_BF16_BYTES + TM * 8 * 4 + 4 * H * 4 + 512 + 2048;
+constexpr int TC_SMEM_NODE_ENC_BWD_IG = TC_SMEM_NODE_ENC_BWD + H * 8 * 4;  // + W0 staged as [128][8] (features 0-4 used)
 
+// IG: also write the input gradient dfeat = dh0 W0 (features 0-4, un-standardised, times 1/S), formed from the fp32 TMEM
+// values of dh0.  Each thread owns 64 channels of one row; the half-1 thread hands its five partial sums to the half-0
+// thread of the row through its own (then dead) 128 bytes of the h0 tile.  The <false> instance is unchanged.
+template <bool IG>
 __global__ void __launch_bounds__(NT, 1)
 k_node_encoder_bwd_tc(NodeEncBwdArgs a, const uint8_t* __restrict__ imgW2) {
   extern __shared__ uint8_t smem_raw[];
@@ -194,10 +202,15 @@ k_node_encoder_bwd_tc(NodeEncBwdArgs a, const uint8_t* __restrict__ imgW2) {
   uint8_t* T1 = T0 + tc::TILE_BF16_BYTES;   // h0
   float* feat = reinterpret_cast<float*>(T1 + tc::TILE_BF16_BYTES);  // [TM][8]
   float* comb = feat + TM * 8;  // [4][H]
-  uint64_t* bars = reinterpret_cast<uint64_t*>(comb + 4 * H);
+  float* w0s = comb + 4 * H;    // IG: [H][8]
+  uint64_t* bars = reinterpret_cast<uint64_t*>(w0s + (IG ? H * 8 : 0));
   uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 2);
   const TcThread t;
   float* cg = a.cta_grads + (size_t)blockIdx.x * GRADP;
+  if (IG && t.tid < H) {
+#pragma unroll
+    for (int j = 0; j < 8; ++j) w0s[t.tid * 8 + j] = j < 5 ? a.W0[t.tid * 6 + j] : 0.f;
+  }
   const uint32_t tmem = tc_setup_ends(bars, 2, tmem_slot, 256);
   const uint32_t ACC = tmem, WORK = tmem + 128;
   if (t.tid == 0) {
@@ -215,6 +228,8 @@ k_node_encoder_bwd_tc(NodeEncBwdArgs a, const uint8_t* __restrict__ imgW2) {
   }
   pdl_sync();  // scal / g_in come from the preceding kernels
   const float c1 = a.scal[0], c2 = a.scal[1], mu = a.scal[2], rstd = a.scal[3];
+  const float ims = IG ? a.gs[1] / (a.scale_in ? a.nrm.std_mean_stress : 1.f) : 0.f;
+  const float ipos = IG ? a.gs[1] / (a.scale_in ? a.nrm.std_pos : 1.f) : 0.f;
   float db2[2] = {0.f, 0.f}, db0[2] = {0.f, 0.f}, dw0[6][2];
 #pragma unroll
   for (int j = 0; j < 6; ++j) { dw0[j][0] = 0.f; dw0[j][1] = 0.f; }
@@ -271,6 +286,7 @@ k_node_encoder_bwd_tc(NodeEncBwdArgs a, const uint8_t* __restrict__ imgW2) {
     tc::mbar_wait(&bars[1], ph);
     tc::fence_after_sync();
     __syncthreads();  // every column walker is done with dy before the epilogue overwrites T0 with dh0
+    float gi[5] = {0.f, 0.f, 0.f, 0.f, 0.f};
 #pragma unroll
     for (int hh = 0; hh < 2; ++hh) {
       float v[32];
@@ -283,10 +299,37 @@ k_node_encoder_bwd_tc(NodeEncBwdArgs a, const uint8_t* __restrict__ imgW2) {
 #pragma unroll
         for (int j = 0; j < 8; ++j) d[j] = h[j] > 0.f ? v[c8 * 8 + j] : 0.f;
         row_store8(T0, t.row, t.half, hh * 4 + c8, d);
+        if (IG) {
+#pragma unroll
+          for (int j = 0; j < 8; ++j) {
+            const float* w = w0s + (t.half * 64 + hh * 32 + c8 * 8 + j) * 8;  // warp-uniform: broadcast
+            const float4 w03 = *reinterpret_cast<const float4*>(w);
+            gi[0] = fmaf(d[j], w03.x, gi[0]); gi[1] = fmaf(d[j], w03.y, gi[1]); gi[2] = fmaf(d[j], w03.z, gi[2]);
+            gi[3] = fmaf(d[j], w03.w, gi[3]); gi[4] = fmaf(d[j], w[4], gi[4]);
+          }
+        }
       }
+    }
+    if (IG && t.half == 1) {  // chunks 8-9 of this row of T1: read above by this thread only
+      *reinterpret_cast<float4*>(T1 + tc::sw128_chunk(t.row, 8)) = make_float4(gi[0], gi[1], gi[2], gi[3]);
+      *reinterpret_cast<float*>(T1 + tc::sw128_chunk(t.row, 9)) = gi[4];
     }
     tc::fence_before_sync();
     __syncthreads();
+    if (IG && t.half == 0 && t.row < nvalid) {
+      const float4 p03 = *reinterpret_cast<const float4*>(T1 + tc::sw128_chunk(t.row, 8));
+      const float p4 = *reinterpret_cast<const float*>(T1 + tc::sw128_chunk(t.row, 9));
+      const int row = row0 + t.row;
+      if (a.g_mean_stress != nullptr) {
+        a.g_mean_stress[row * 3 + 0] = (gi[0] + p03.x) * ims;
+        a.g_mean_stress[row * 3 + 1] = (gi[1] + p03.y) * ims;
+        a.g_mean_stress[row * 3 + 2] = (gi[2] + p03.z) * ims;
+      }
+      if (a.g_pos != nullptr) {
+        a.g_pos[row * 2 + 0] = (gi[3] + p03.w) * ipos;
+        a.g_pos[row * 2 + 1] = (gi[4] + p4) * ipos;
+      }
+    }
     {  // db0 = colsum(dh0), dW0[c][j] = sum_r dh0[r][c] * feat[r][j]   (thread = channel pair x 32-row quarter)
       const int cp = t.tid & 63, q = t.tid >> 6;
       float s0 = 0.f, s1 = 0.f, u[6][2];
@@ -623,10 +666,17 @@ int launch_node_encoder_tc(const float* mean_stress, const float* pos, const int
 }
 int launch_node_encoder_bwd_tc(const float* g_in, const float* y_raw, const float* scal, const float* lnw, const float* mean_stress,
                                const float* pos, const int64_t* types, const pdg_norm_t* nrm, int scale_in, const float* W0,
-                               const float* b0, float* cta_grads, int N, int n_tiles, int grid, const uint8_t* img, cudaStream_t st) {
-  if (ends_attr((const void*)k_node_encoder_bwd_tc, TC_SMEM_NODE_ENC_BWD, "k_node_encoder_bwd_tc")) return -2;
-  NodeEncBwdArgs a{g_in, y_raw, scal, lnw, mean_stress, pos, types, *nrm, scale_in, W0, b0, cta_grads, N, n_tiles};
-  return ends_launch(launch_pdl(k_node_encoder_bwd_tc, dim3(grid), dim3(NT), TC_SMEM_NODE_ENC_BWD, st, a, ends_img(img, IMG_NE_W2)),
+                               const float* b0, float* cta_grads, const float* gs, float* grad_mean_stress, float* grad_pos, int N,
+                               int n_tiles, int grid, const uint8_t* img, cudaStream_t st) {
+  NodeEncBwdArgs a{g_in, y_raw, scal, lnw, mean_stress, pos, types, *nrm, scale_in, W0, b0, cta_grads, gs, grad_mean_stress, grad_pos,
+                   N, n_tiles};
+  if (grad_mean_stress != nullptr || grad_pos != nullptr) {
+    if (ends_attr((const void*)k_node_encoder_bwd_tc<true>, TC_SMEM_NODE_ENC_BWD_IG, "k_node_encoder_bwd_tc")) return -2;
+    return ends_launch(launch_pdl(k_node_encoder_bwd_tc<true>, dim3(grid), dim3(NT), TC_SMEM_NODE_ENC_BWD_IG, st, a,
+                                  ends_img(img, IMG_NE_W2)), "k_node_encoder_bwd_tc");
+  }
+  if (ends_attr((const void*)k_node_encoder_bwd_tc<false>, TC_SMEM_NODE_ENC_BWD, "k_node_encoder_bwd_tc")) return -2;
+  return ends_launch(launch_pdl(k_node_encoder_bwd_tc<false>, dim3(grid), dim3(NT), TC_SMEM_NODE_ENC_BWD, st, a, ends_img(img, IMG_NE_W2)),
                      "k_node_encoder_bwd_tc");
 }
 int launch_decoder_tc(const float* base, const float* yprev, const double* prev_parts, double prev_count, const float* lnw,

@@ -160,7 +160,8 @@ int launch_node_encoder_tc(const float* mean_stress, const float* pos, const int
                            int n_tiles, int grid, const uint8_t* img, cudaStream_t st);
 int launch_node_encoder_bwd_tc(const float* g_in, const float* y_raw, const float* scal, const float* lnw, const float* mean_stress,
                                const float* pos, const int64_t* types, const pdg_norm_t* nrm, int scale_in, const float* W0,
-                               const float* b0, float* cta_grads, int N, int n_tiles, int grid, const uint8_t* img, cudaStream_t st);
+                               const float* b0, float* cta_grads, const float* gs, float* grad_mean_stress, float* grad_pos, int N,
+                               int n_tiles, int grid, const uint8_t* img, cudaStream_t st);
 int launch_decoder_tc(const float* base, const float* yprev, const double* prev_parts, double prev_count, const float* lnw,
                       const float* lnb, float* x_out, const float* d1, const float* D2, const float* d2, float* hd_out,
                       float out_scale, float out_shift, float* out, const int* nzflag, int N, int n_tiles, int grid,
@@ -173,7 +174,8 @@ int launch_edge_encoder_tc(const float* edge_attr, const int32_t* perm, const pd
                            const uint8_t* img, cudaStream_t st);  // pdg_tc_enc.cu
 int launch_edge_encoder_bwd_tc(const float* g_in, const float* y_raw, const float* scal, const float* lnw, const float* edge_attr,
                                const int32_t* perm, const pdg_norm_t* nrm, int scale_in, const float* W0, const float* b0,
-                               float* cta_grads, int E, int n_tiles, int grid, const uint8_t* img, cudaStream_t st);
+                               float* cta_grads, const float* gs, float* grad_edge_attr, int E, int n_tiles, int grid,
+                               const uint8_t* img, cudaStream_t st);
 int launch_node_pre_tc(const NodePreArgs& a, const uint8_t* img, int n_tiles, cudaStream_t st);          // pdg_tc_node.cu
 int launch_node_update_tc(const NodeUpdArgs& a, const uint8_t* img, int grid, cudaStream_t st);
 int launch_node_update_bwd_tc(const NodeUpdBwdArgs& a, const uint8_t* img, int grid, cudaStream_t st);
