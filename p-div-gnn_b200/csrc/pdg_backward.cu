@@ -899,12 +899,16 @@ __global__ void k_grad_reduce(const float* __restrict__ cta_grads, int G, float*
 }
 
 // Power-of-two gradient scale of the fp16 tensor-core backward (the GradScaler of gnn_train.py:111,204-207 moved inside
-// the operator and decided on the device): gs[0] = S = 2^(8 - e) with max|g| in [2^(e-1), 2^e), gs[1] = 1/S.  Every
-// gradient-valued fp16 tile / row of the backward then sits around 2^8 x (its size relative to d loss / d local_stress):
-// measured along the chain the tiles span 1e-5 .. 4 of that maximum, i.e. 2.5e-3 .. 1e3 after scaling -- inside fp16's
-// normal range [6.1e-5, 65504] with 2^6 of headroom (conversions saturate, nothing becomes inf).  Zero / non-finite
-// gradients: S = 1.  One block; deterministic (max is order-free).
-__global__ void __launch_bounds__(1024) k_grad_scale(const float* __restrict__ g, int n, float* __restrict__ gs) {
+// the operator and decided on the device).  The decoder backward builds its first fp16 tile from g * gscale * S, where
+// gscale is the output de-standardisation factor (std_local_stress with PDG_FLAG_SCALE_OUTPUT, else 1), so S is chosen
+// from that product: gs[0] = S = 2^(8 - e) with max|g| * |gscale| in [2^(e-1), 2^e), gs[1] = 1/S.  Every gradient-valued
+// fp16 tile / row of the backward then sits around 2^8 x (its size relative to d loss / d(standardised output)),
+// whatever std_local_stress is: measured along the chain the tiles span 1e-5 .. 4 of that maximum, i.e. 2.5e-3 .. 1e3
+// after scaling -- inside fp16's normal range [6.1e-5, 65504] with 2^6 of headroom (conversions saturate, nothing
+// becomes inf).  The product is formed in double, so it neither overflows nor rounds across a power of two, and S
+// follows a power-of-two rescaling of g exactly.  Every consumer (k_grad_reduce, the input-gradient epilogues) removes
+// S alone: gscale is part of the chain rule, S is not.  Zero / non-finite: S = 1.  One block; deterministic.
+__global__ void __launch_bounds__(1024) k_grad_scale(const float* __restrict__ g, int n, float gscale, float* __restrict__ gs) {
   pdl_sync();
   __shared__ float red[32];
   float m = 0.f;
@@ -917,8 +921,9 @@ __global__ void __launch_bounds__(1024) k_grad_scale(const float* __restrict__ g
     for (int w = 1; w < 32; ++w) m = fmaxf(m, red[w]);
     int e = 0;
     float S = 1.f, inv = 1.f;
-    if (m > 0.f && isfinite(m)) {
-      frexpf(m, &e);  // m = f * 2^e, f in [0.5, 1)
+    const double mt = (double)m * fabs((double)gscale);
+    if (mt > 0.0 && isfinite(mt)) {
+      frexp(mt, &e);  // mt = f * 2^e, f in [0.5, 1)
       int k = 8 - e;
       k = k > 100 ? 100 : (k < -100 ? -100 : k);
       S = ldexpf(1.f, k);
@@ -986,7 +991,7 @@ extern "C" int pdg_backward_inputs(const pdg_params_t* params, const pdg_norm_t*
   const float gscale = (flags & PDG_FLAG_SCALE_OUTPUT) ? norm->std_local_stress : 1.f;
   const float* gs = nullptr;
   if (tcm) {  // fp16 gradient tiles: scale the incoming gradient to a fixed magnitude, unscale in k_grad_reduce
-    PDG_CUDA_CHECK(launch_pdl(k_grad_scale, dim3(1), dim3(1024), 0, st, grad_local_stress, N * PDG_OUT, B.gs));
+    PDG_CUDA_CHECK(launch_pdl(k_grad_scale, dim3(1), dim3(1024), 0, st, grad_local_stress, N * PDG_OUT, gscale, B.gs));
     PDG_LAUNCH_CHECK();
     gs = B.gs;
   }

@@ -9,7 +9,8 @@
 //     well inside fp16's range; every conversion saturates (cvt.rn.satfinite) so nothing can become inf;
 //   * gradient-valued tiles / rows (dy, d-hidden, g_agg, dhm / dhn) span ~6 decades along the backward chain and are
 //     tiny in absolute terms (1e-3 .. 1e-9): pdg_backward multiplies d loss / d local_stress by a power of two S chosen
-//     on the device so that its largest element sits at 2^8 (k_grad_scale), the whole -- linear -- backward runs on
+//     on the device so that the largest element of the decoder's first gradient tile, g * gscale (gscale =
+//     std_local_stress with scale_output), sits at 2^8 (k_grad_scale), the whole -- linear -- backward runs on
 //     scaled values (fp32 streams included) and k_grad_reduce multiplies the weight gradients by 1/S.  That is the
 //     GradScaler of the reference train loop (gnn_train.py:111,204-207) moved inside the operator, with no host sync.
 //     Values down to 2^-15 of the scaled stream keep at least bf16's relative precision, smaller ones an absolute
