@@ -146,6 +146,21 @@ int pdg_backward_inputs(const pdg_params_t* params, const pdg_norm_t* norm, cons
                         size_t bwd_ws_bytes, const float* grad_local_stress, float* grads_flat,
                         float* grad_mean_stress, float* grad_pos, float* grad_edge_attr, void* stream);
 
+/* ---- model forward-mode derivative (Jacobian-vector product) ---------------------------
+ * tan_local_stress [N,3] (overwritten) = d local_stress / d (mean_stress, pos, edge_attr) applied to the tangents
+ * tan_mean_stress [N,3], tan_pos [N,2], tan_edge_attr [E] (caller's PyG edge order); a NULL tangent is a zero tangent.
+ * nodes_types is an integer input and has no tangent.  fwd_ws is the workspace of a pdg_forward with PDG_FLAG_SAVE
+ * and the same arguments (flags included); it is only read, so a pdg_backward may follow.  jvp_ws: the tangent
+ * workspace, pdg_jvp_ws_bytes.  Returns -1 for precision != PDG_PREC_FP32 (the 16-bit mode has no forward-mode
+ * derivative), flags without PDG_FLAG_SAVE, steps outside 1..62 or a workspace that is too small.
+ * Replaces torch forward-mode AD (torch.func.jvp, torch.autograd.forward_ad) through models.py:288-326. */
+size_t pdg_jvp_ws_bytes(int64_t n_nodes, int64_t n_edges, int steps);
+int pdg_jvp(const pdg_params_t* params, const pdg_norm_t* norm, const float* mean_stress, const float* pos,
+            const int64_t* nodes_types, const float* edge_attr, const void* plan, int64_t n_nodes, int64_t n_edges,
+            int steps, int flags, int precision, const void* fwd_ws, void* jvp_ws, size_t jvp_ws_bytes,
+            const float* tan_mean_stress, const float* tan_pos, const float* tan_edge_attr, float* tan_local_stress,
+            void* stream);
+
 /* ---- loss: per-graph NMSE + divergence regulariser, batch means ---------------------
  * Replaces the per-graph Python loop of train() (gnn_train.py:162-202):
  * normalized_mse_loss_single (:41-57), compute_divergence (:60-92),

@@ -60,6 +60,9 @@ _SIGS = {
                             _i32, _vp, _vp, _sz, _vp, _vp, _vp]),
     "pdg_backward_inputs": (_i32, [C.POINTER(PdgParams), C.POINTER(PdgNorm), _vp, _vp, _vp, _vp, _vp, _i64, _i64, _i32,
                                    _i32, _i32, _vp, _vp, _sz, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "pdg_jvp_ws_bytes": (_sz, [_i64, _i64, _i32]),
+    "pdg_jvp": (_i32, [C.POINTER(PdgParams), C.POINTER(PdgNorm), _vp, _vp, _vp, _vp, _vp, _i64, _i64, _i32, _i32, _i32,
+                       _vp, _vp, _sz, _vp, _vp, _vp, _vp, _vp]),
     "pdg_opdiv_plan_bytes": (_sz, [_i64, _i64]),
     "pdg_opdiv_tmp_bytes": (_sz, [_i64, _i64]),
     "pdg_opdiv_plan_build": (_i32, [_vp, _vp, _i64, _vp, _i64, _i64, _vp, _vp, _sz, _vp]),
@@ -130,8 +133,16 @@ def check(rc: int, what: str):
         raise RuntimeError(f"{what} failed (rc={rc}): {lib().pdg_last_error().decode()}")
 
 
+def raw(t):
+    """The plain tensor under functorch wrappers: inside torch.func transforms (torch.func.jvp), tensors created by the
+    transformed function are wrappers without storage of their own; the library reads and writes the wrapped one."""
+    while torch._C._functorch.is_functorch_wrapped_tensor(t):
+        t = torch._C._functorch.get_unwrapped(t)
+    return t
+
+
 def ptr(t):
-    return None if t is None else C.c_void_p(t.data_ptr())
+    return None if t is None else C.c_void_p(raw(t).data_ptr())
 
 
 def stream_ptr(device=None):

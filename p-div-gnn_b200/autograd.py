@@ -2,7 +2,7 @@
 
 Nothing here computes; it validates inputs, builds / caches the device graph plan,
 allocates the workspace from torch's caching allocator (so stream semantics hold) and
-calls ``pdg_forward`` / ``pdg_backward_inputs`` on the current CUDA stream.
+calls ``pdg_forward`` / ``pdg_backward_inputs`` / ``pdg_jvp`` on the current CUDA stream.
 """
 from __future__ import annotations
 
@@ -11,6 +11,7 @@ import os
 from collections import OrderedDict
 
 import torch
+import torch.autograd.forward_ad as fwAD
 
 from . import _lib
 
@@ -56,7 +57,7 @@ class GraphPlan:
         ptrs = [C.c_void_p() for _ in range(6)]
         _lib.check(L.pdg_plan_views(_lib.ptr(self.buf), self.n_nodes, self.n_edges, *[C.byref(p) for p in ptrs]),
                    "pdg_plan_views")
-        base = self.buf.data_ptr()
+        base = _lib.raw(self.buf).data_ptr()
         e_pad = (self.n_edges + 127) // 128 * 128
         sizes = [e_pad, e_pad, e_pad, self.n_nodes + 1, self.n_nodes + 1, self.n_edges]
         i32 = self.buf.view(torch.int32)
@@ -120,17 +121,20 @@ def _bucket(nbytes: int) -> int:
 def _params_struct(params):
     s = _lib.PdgParams()
     for i, p in enumerate(params):
-        s.p[i] = p.data_ptr()
+        s.p[i] = _lib.raw(p).data_ptr()
     return s
 
 
 class _EPDFunction(torch.autograd.Function):
+    """pdg_forward, pdg_backward_inputs (reverse mode) and pdg_jvp (forward mode).  Written in setup_context style so
+    that torch.func.jvp accepts it; the forward workspace reaches ctx as a second, non-differentiable output."""
+
     @staticmethod
-    def forward(ctx, model, plan, mean_stress, pos, types, edge_attr, flags, steps, prec, need_grad, *params):
+    def forward(model, plan, mean_stress, pos, types, edge_attr, flags, steps, prec, need_grad, need_tan, *params):
         L = _lib.lib()
         dev = mean_stress.device
         n, e = plan.n_nodes, plan.n_edges
-        if need_grad:
+        if need_grad or need_tan:
             flags |= _lib.FLAG_SAVE
         params = [_lib.require_cuda(p.detach(), "parameter", torch.float32) for p in params]
         norm = model._norm_struct()
@@ -142,18 +146,62 @@ class _EPDFunction(torch.autograd.Function):
             _lib.check(L.pdg_forward(C.byref(ps), C.byref(norm), _lib.ptr(mean_stress), _lib.ptr(pos), _lib.ptr(types),
                                      _lib.ptr(edge_attr), _lib.ptr(plan.buf), n, e, steps, flags, prec, _lib.ptr(ws),
                                      ws_bytes, _lib.ptr(out), _lib.stream_ptr(dev)), "pdg_forward")
-        if need_grad:
-            ctx.pdg = (model, plan, mean_stress, pos, types, edge_attr, flags, steps, prec, params, ws, norm)
-        return out
+        return out, ws
 
     @staticmethod
-    def backward(ctx, grad_out):
+    def setup_context(ctx, inputs, output):
+        model, plan, mean_stress, pos, types, edge_attr, flags, steps, prec, need_grad, need_tan, *params = inputs
+        _, ws = output
+        ctx.mark_non_differentiable(ws)
+        # no zero gradient is materialised for the workspace output (a memset of the whole saved state per backward);
+        # tangents that do not exist arrive as None (pdg_jvp reads NULL as a zero tangent)
+        ctx.set_materialize_grads(False)
+        ctx.pdg = None
+        if need_grad or need_tan:
+            params = [_lib.require_cuda(p.detach(), "parameter", torch.float32) for p in params]
+            ctx.pdg = (model, plan, mean_stress, pos, types, edge_attr, flags | _lib.FLAG_SAVE, steps, prec, params, ws,
+                       model._norm_struct())
+        ctx.pdg_need_grad = need_grad
+
+    @staticmethod
+    def jvp(ctx, _model, _plan, t_ms, t_pos, _types, t_ea, *_rest):
+        """Tangent of local_stress from the tangents of mean_stress, pos and edge_attr (pdg_jvp, fp32 mode).
+        Tangents of the parameters were refused in epd_forward; whatever arrives for them here is ignored."""
+        L = _lib.lib()
+        model, plan, mean_stress, pos, types, edge_attr, flags, steps, prec, params, ws, norm = ctx.pdg
+        dev = mean_stress.device
+        n, e = plan.n_nodes, plan.n_edges
+
+        def tangent(t, name, shape):
+            if t is None:
+                return None
+            # tangents may arrive non-contiguous (an expanded load direction) or in another dtype
+            return _lib.require_cuda(t.to(torch.float32), name, torch.float32).reshape(shape)
+        t_ms, t_pos, t_ea = tangent(t_ms, "mean_stress tangent", (n, 3)), tangent(t_pos, "pos tangent", (n, 2)), \
+            tangent(t_ea, "edge_attr tangent", (e,))
+        with torch.cuda.device(dev):
+            jws_bytes = L.pdg_jvp_ws_bytes(n, e, steps)
+            jws = torch.empty(_bucket(jws_bytes), dtype=torch.uint8, device=dev)
+            t_out = torch.empty((n, 3), dtype=torch.float32, device=dev)
+            ps = _params_struct(params)
+            _lib.check(L.pdg_jvp(C.byref(ps), C.byref(norm), _lib.ptr(mean_stress), _lib.ptr(pos), _lib.ptr(types),
+                                 _lib.ptr(edge_attr), _lib.ptr(plan.buf), n, e, steps, flags, prec, _lib.ptr(ws),
+                                 _lib.ptr(jws), jws_bytes, _lib.ptr(t_ms), _lib.ptr(t_pos), _lib.ptr(t_ea),
+                                 _lib.ptr(t_out), _lib.stream_ptr(dev)), "pdg_jvp")
+        if not ctx.pdg_need_grad:
+            ctx.pdg = None  # no backward follows: release the forward workspace now
+        return t_out, None
+
+    @staticmethod
+    def backward(ctx, grad_out, _grad_ws):
         L = _lib.lib()
         if not hasattr(L, "pdg_backward_inputs") or getattr(L.pdg_backward_inputs, "argtypes", None) is None:
             raise RuntimeError("libpdivgnn.so was built without pdg_backward_inputs")
         model, plan, mean_stress, pos, types, edge_attr, flags, steps, prec, params, ws, norm = ctx.pdg
-        dev = grad_out.device
         n, e = plan.n_nodes, plan.n_edges
+        dev = mean_stress.device
+        if grad_out is None:  # local_stress received no gradient: as autograd's materialised zeros
+            grad_out = torch.zeros((n, 3), dtype=torch.float32, device=dev)
         grad_out = _lib.require_cuda(grad_out, "grad_local_stress", torch.float32)
         need = ctx.needs_input_grad  # slots 2, 3, 5: mean_stress, pos, edge_attr
         with torch.cuda.device(dev):
@@ -176,10 +224,10 @@ class _EPDFunction(torch.autograd.Function):
             allreduce_flat_(flat, dp[1], getattr(model, "_pdg_peer", None))
         grads, off = [], 0
         for i, p in enumerate(params):
-            grads.append(flat[off:off + p.numel()].view(p.shape) if need[10 + i] else None)
+            grads.append(flat[off:off + p.numel()].view(p.shape) if need[11 + i] else None)
             off += p.numel()
         ctx.pdg = None
-        return (None, None, g_ms, g_pos, None, g_ea) + (None,) * 4 + tuple(grads)
+        return (None, None, g_ms, g_pos, None, g_ea) + (None,) * 5 + tuple(grads)
 
 
 # ---- CUDA-graph replay of the inference forward (small-N latency) ------------------------------------------------------
@@ -256,8 +304,22 @@ def epd_forward(model, mesh_graph, scale_output: bool, scale_input: bool, zero_c
     # (no parameter requires grad) differentiated with respect to its inputs keeps it too
     need_grad = torch.is_grad_enabled() and (mean_stress.requires_grad or pos.requires_grad or edge_attr.requires_grad
                                              or any(p.requires_grad for p in params))
-    if not need_grad and (getattr(model, "cuda_graphs", False) or _GRAPHS_ENV) and not torch.cuda.is_current_stream_capturing():
+    # forward-mode AD (torch.autograd.forward_ad dual tensors, torch.func.jvp): tangents of the inputs keep the forward
+    # state for pdg_jvp.  Parameters are looked at only while a dual level is open (no cost on the training path), and
+    # through a fresh walk of the module: torch.func.functional_call swaps them under the cached list of param_list.
+    need_tan = False
+    if fwAD._current_level >= 0:
+        need_tan = any(fwAD.unpack_dual(t).tangent is not None for t in (mean_stress, pos, edge_attr))
+        if any(fwAD.unpack_dual(p).tangent is not None for _, p in model.named_parameters()):
+            raise NotImplementedError("pdivgnn_b200: forward-mode derivatives with respect to the parameters are not "
+                                      "implemented; tangents of mean_stress, pos and edge_attr are")
+        if need_tan and prec != _lib.PREC_FP32:
+            raise NotImplementedError("pdivgnn_b200: forward-mode derivatives need precision='fp32'; in the 16-bit mode "
+                                      "per-row derivatives amplify the fp16 rounding beyond its 2e-2 tolerance "
+                                      "(DESIGN.md section 5)")
+    if not (need_grad or need_tan) and (getattr(model, "cuda_graphs", False) or _GRAPHS_ENV) \
+            and not torch.cuda.is_current_stream_capturing():
         return _forward_graphed(model, plan, mean_stress, pos, types, edge_attr, flags, model.message_passing_steps, prec,
                                 params)
     return _EPDFunction.apply(model, plan, mean_stress, pos, types, edge_attr, flags, model.message_passing_steps, prec,
-                              need_grad, *params)
+                              need_grad, need_tan, *params)[0]
