@@ -161,6 +161,21 @@ int pdg_jvp(const pdg_params_t* params, const pdg_norm_t* norm, const float* mea
             const float* tan_mean_stress, const float* tan_pos, const float* tan_edge_attr, float* tan_local_stress,
             void* stream);
 
+/* Batched tangents: one tangent pass carries n_tangents (1..PDG_JVP_MAX_TANGENTS) tangents K.  Tangent k of an input is
+ * contiguous in the layout of pdg_jvp and starts at tan_x + k * x_stride (elements); stride 0 gives every k the same
+ * tangent, NULL a zero tangent.  tan_local_stress [K][N][3].  jvp_ws: pdg_jvp_batched_ws_bytes (K tangent workspaces
+ * of pdg_jvp_ws_bytes each); 0 for K or steps out of range.  Column k has the bits of a pdg_jvp call on tangent k.
+ * Launches the kernels of one pdg_jvp for any K.  Returns -1 for K outside 1..PDG_JVP_MAX_TANGENTS and for every
+ * refusal of pdg_jvp.  pdg_jvp is this call with K = 1. */
+#define PDG_JVP_MAX_TANGENTS 64
+size_t pdg_jvp_batched_ws_bytes(int64_t n_nodes, int64_t n_edges, int steps, int n_tangents);
+int pdg_jvp_batched(const pdg_params_t* params, const pdg_norm_t* norm, const float* mean_stress, const float* pos,
+                    const int64_t* nodes_types, const float* edge_attr, const void* plan, int64_t n_nodes,
+                    int64_t n_edges, int steps, int flags, int precision, const void* fwd_ws, void* jvp_ws,
+                    size_t jvp_ws_bytes, int n_tangents, const float* tan_mean_stress, int64_t ms_stride,
+                    const float* tan_pos, int64_t pos_stride, const float* tan_edge_attr, int64_t ea_stride,
+                    float* tan_local_stress, void* stream);
+
 /* ---- loss: per-graph NMSE + divergence regulariser, batch means ---------------------
  * Replaces the per-graph Python loop of train() (gnn_train.py:162-202):
  * normalized_mse_loss_single (:41-57), compute_divergence (:60-92),

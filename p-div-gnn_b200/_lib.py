@@ -16,6 +16,7 @@ PDG_NUM_PARAMS = 28
 PDG_PARAM_ELEMS = 167299
 FLAG_SCALE_INPUT, FLAG_SCALE_OUTPUT, FLAG_SAVE, FLAG_ZERO_CHECK = 1, 2, 4, 8
 PREC_FP32, PREC_BF16 = 0, 1
+JVP_MAX_TANGENTS = 64  # PDG_JVP_MAX_TANGENTS: tangents of one pdg_jvp_batched call
 
 
 class PdgParams(C.Structure):
@@ -63,6 +64,9 @@ _SIGS = {
     "pdg_jvp_ws_bytes": (_sz, [_i64, _i64, _i32]),
     "pdg_jvp": (_i32, [C.POINTER(PdgParams), C.POINTER(PdgNorm), _vp, _vp, _vp, _vp, _vp, _i64, _i64, _i32, _i32, _i32,
                        _vp, _vp, _sz, _vp, _vp, _vp, _vp, _vp]),
+    "pdg_jvp_batched_ws_bytes": (_sz, [_i64, _i64, _i32, _i32]),
+    "pdg_jvp_batched": (_i32, [C.POINTER(PdgParams), C.POINTER(PdgNorm), _vp, _vp, _vp, _vp, _vp, _i64, _i64, _i32, _i32,
+                               _i32, _vp, _vp, _sz, _i32, _vp, _i64, _vp, _i64, _vp, _i64, _vp, _vp]),
     "pdg_opdiv_plan_bytes": (_sz, [_i64, _i64]),
     "pdg_opdiv_tmp_bytes": (_sz, [_i64, _i64]),
     "pdg_opdiv_plan_build": (_i32, [_vp, _vp, _i64, _vp, _i64, _i64, _vp, _vp, _sz, _vp]),
@@ -135,8 +139,12 @@ def check(rc: int, what: str):
 
 def raw(t):
     """The plain tensor under functorch wrappers: inside torch.func transforms (torch.func.jvp), tensors created by the
-    transformed function are wrappers without storage of their own; the library reads and writes the wrapped one."""
+    transformed function are wrappers without storage of their own; the library reads and writes the wrapped one.
+    A vmap BatchedTensor is refused: its storage holds the whole batch while the library would read one tensor."""
     while torch._C._functorch.is_functorch_wrapped_tensor(t):
+        if torch._C._functorch.is_batchedtensor(t):
+            raise RuntimeError("pdivgnn_b200: a vmap BatchedTensor reached the library; its storage holds the whole "
+                               "batch, so it cannot be passed as one tensor")
         t = torch._C._functorch.get_unwrapped(t)
     return t
 

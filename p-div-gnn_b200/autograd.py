@@ -2,7 +2,7 @@
 
 Nothing here computes; it validates inputs, builds / caches the device graph plan,
 allocates the workspace from torch's caching allocator (so stream semantics hold) and
-calls ``pdg_forward`` / ``pdg_backward_inputs`` / ``pdg_jvp`` on the current CUDA stream.
+calls ``pdg_forward`` / ``pdg_backward_inputs`` / ``pdg_jvp_batched`` on the current CUDA stream.
 """
 from __future__ import annotations
 
@@ -165,32 +165,20 @@ class _EPDFunction(torch.autograd.Function):
 
     @staticmethod
     def jvp(ctx, _model, _plan, t_ms, t_pos, _types, t_ea, *_rest):
-        """Tangent of local_stress from the tangents of mean_stress, pos and edge_attr (pdg_jvp, fp32 mode).
-        Tangents of the parameters were refused in epd_forward; whatever arrives for them here is ignored."""
-        L = _lib.lib()
-        model, plan, mean_stress, pos, types, edge_attr, flags, steps, prec, params, ws, norm = ctx.pdg
-        dev = mean_stress.device
-        n, e = plan.n_nodes, plan.n_edges
-
-        def tangent(t, name, shape):
-            if t is None:
-                return None
-            # tangents may arrive non-contiguous (an expanded load direction) or in another dtype
-            return _lib.require_cuda(t.to(torch.float32), name, torch.float32).reshape(shape)
-        t_ms, t_pos, t_ea = tangent(t_ms, "mean_stress tangent", (n, 3)), tangent(t_pos, "pos tangent", (n, 2)), \
-            tangent(t_ea, "edge_attr tangent", (e,))
-        with torch.cuda.device(dev):
-            jws_bytes = L.pdg_jvp_ws_bytes(n, e, steps)
-            jws = torch.empty(_bucket(jws_bytes), dtype=torch.uint8, device=dev)
-            t_out = torch.empty((n, 3), dtype=torch.float32, device=dev)
-            ps = _params_struct(params)
-            _lib.check(L.pdg_jvp(C.byref(ps), C.byref(norm), _lib.ptr(mean_stress), _lib.ptr(pos), _lib.ptr(types),
-                                 _lib.ptr(edge_attr), _lib.ptr(plan.buf), n, e, steps, flags, prec, _lib.ptr(ws),
-                                 _lib.ptr(jws), jws_bytes, _lib.ptr(t_ms), _lib.ptr(t_pos), _lib.ptr(t_ea),
-                                 _lib.ptr(t_out), _lib.stream_ptr(dev)), "pdg_jvp")
+        """Tangent of local_stress from the tangents of mean_stress, pos and edge_attr (fp32 mode).  Under vmap the
+        tangents are batched and _EPDTangent's vmap rule makes one tangent pass for the whole batch.  Tangents of the
+        parameters were refused in epd_forward; whatever arrives for them here is ignored."""
+        t_out = _EPDTangent.apply(ctx.pdg, t_ms, t_pos, t_ea)
         if not ctx.pdg_need_grad:
             ctx.pdg = None  # no backward follows: release the forward workspace now
         return t_out, None
+
+    @staticmethod
+    def vmap(info, in_dims, *args):
+        """torch reaches this rule only when a model input or parameter is batched at this vmap level: with unbatched
+        primals it skips the level, and batched tangents go to _EPDTangent.vmap."""
+        raise NotImplementedError("pdivgnn_b200: vmap over the model's inputs or parameters is not implemented; batched "
+                                  "tangents are (torch.func.jacfwd, torch.func.vmap over torch.func.jvp)")
 
     @staticmethod
     def backward(ctx, grad_out, _grad_ws):
@@ -228,6 +216,88 @@ class _EPDFunction(torch.autograd.Function):
             off += p.numel()
         ctx.pdg = None
         return (None, None, g_ms, g_pos, None, g_ea) + (None,) * 5 + tuple(grads)
+
+
+def _tangent_shapes(state):
+    plan = state[1]
+    return ((plan.n_nodes, 3), (plan.n_nodes, 2), (plan.n_edges,))
+
+
+class _EPDTangent(torch.autograd.Function):
+    """Tangents of local_stress for K tangents of (mean_stress, pos, edge_attr) in one pdg_jvp_batched pass.  `state` is
+    the forward's ctx tuple.  A tangent is None (zero), of the input's shape (the same for every k) or [K, *shape]; the
+    result is [K, N, 3], or [N, 3] when no tangent has the K dimension.  The vmap rule folds the vmapped dimension into
+    K.  There is no backward: second-order derivatives are not implemented."""
+
+    @staticmethod
+    def forward(state, t_ms, t_pos, t_ea):
+        L = _lib.lib()
+        model, plan, mean_stress, pos, types, edge_attr, flags, steps, prec, params, ws, norm = state
+        dev = mean_stress.device
+        n, e = plan.n_nodes, plan.n_edges
+        ts, shapes = (t_ms, t_pos, t_ea), _tangent_shapes(state)
+        ks = {t.shape[0] for t, s in zip(ts, shapes) if t is not None and t.dim() == len(s) + 1}
+        if len(ks) > 1:
+            raise ValueError(f"pdivgnn_b200: batched tangents disagree on their count: {sorted(ks)}")
+        k = ks.pop() if ks else None
+        args = []
+        for t, s, name in zip(ts, shapes, ("mean_stress", "pos", "edge_attr")):
+            stride = 0
+            if t is not None:
+                # tangents may arrive non-contiguous (an expanded load direction) or in another dtype; one tangent
+                # expanded over K (leading stride 0) is passed once, with stride 0
+                t = t.to(torch.float32)
+                if t.dim() == len(s) + 1 and t.stride(0) != 0:
+                    t, stride = t.reshape(k, *s), t[0].numel()
+                elif t.dim() == len(s) + 1:
+                    t = t[0]
+                t = _lib.require_cuda(t, f"{name} tangent", torch.float32).reshape(-1, *s)
+            args += [t, stride]
+        with torch.cuda.device(dev):
+            jws_bytes = L.pdg_jvp_batched_ws_bytes(n, e, steps, k or 1)
+            jws = torch.empty(_bucket(jws_bytes), dtype=torch.uint8, device=dev)
+            t_out = torch.empty((k or 1, n, 3), dtype=torch.float32, device=dev)
+            ps = _params_struct(params)
+            _lib.check(L.pdg_jvp_batched(C.byref(ps), C.byref(norm), _lib.ptr(mean_stress), _lib.ptr(pos),
+                                         _lib.ptr(types), _lib.ptr(edge_attr), _lib.ptr(plan.buf), n, e, steps, flags,
+                                         prec, _lib.ptr(ws), _lib.ptr(jws), jws_bytes, k or 1,
+                                         _lib.ptr(args[0]), args[1], _lib.ptr(args[2]), args[3], _lib.ptr(args[4]),
+                                         args[5], _lib.ptr(t_out), _lib.stream_ptr(dev)), "pdg_jvp_batched")
+        return t_out if k is not None else t_out[0]
+
+    @staticmethod
+    def setup_context(ctx, inputs, output):
+        pass
+
+    @staticmethod
+    def vmap(info, in_dims, state, *ts):
+        """Moves the vmapped dimension B of every batched tangent to the front and merges it with a K that an inner
+        vmap level already folded in ([B, K, ...] -> [B*K, ...]: nested vmap flattens).  Unbatched tangents keep the
+        input's shape (stride 0 in the kernels).  One pass per at most JVP_MAX_TANGENTS tangents."""
+        shapes = _tangent_shapes(state)
+        b = info.batch_size
+        ts = [t if d is None else t.movedim(d, 0) for t, d in zip(ts, in_dims[1:])]
+        ks = {t.shape[1 if d is not None else 0] for t, d, s in zip(ts, in_dims[1:], shapes)
+              if t is not None and t.dim() == len(s) + 1 + (d is not None)}
+        if len(ks) > 1:
+            raise ValueError(f"pdivgnn_b200: batched tangents disagree on their count: {sorted(ks)}")
+        k = ks.pop() if ks else None
+        flat = []
+        for t, d, s in zip(ts, in_dims[1:], shapes):
+            if t is not None and k is not None and (d is not None or t.dim() == len(s) + 1):
+                if d is None:
+                    t = t.unsqueeze(0)
+                elif t.dim() == len(s) + 1:
+                    t = t.unsqueeze(1)
+                t = t.expand(b, k, *s).reshape(b * k, *s)
+            flat.append(t)
+        total, cap = b * (k or 1), _lib.JVP_MAX_TANGENTS
+        outs = []
+        for i in range(0, total, cap):
+            part = [t[i:i + cap] if t is not None and t.dim() == len(s) + 1 else t for t, s in zip(flat, shapes)]
+            outs.append(_EPDTangent.apply(state, *part))
+        out = outs[0] if len(outs) == 1 else torch.cat(outs)
+        return (out if k is None else out.reshape(b, k, *out.shape[1:])), 0
 
 
 # ---- CUDA-graph replay of the inference forward (small-N latency) ------------------------------------------------------

@@ -6,6 +6,11 @@
 // packed weights, the zero-load flag), recomputes what the forward did not keep (the first-layer masks of the encoders,
 // G = e_t We^T + b1, the message y1) and never writes the forward workspace, so a later pdg_backward is unaffected.
 //
+// One pass carries K tangents (pdg_jvp_batched).  Each has a tangent workspace of the single-tangent layout, one after
+// another at a fixed stride.  The node kernels and the encoders take the tangent index from blockIdx.y; the edge kernel
+// takes a group of tangents, computes the primal part of a tile once and loops over the group.  Tangent k runs the same
+// operations in the same order (same x-grid, so the same partial slot; same GEMMs and masks) as a single-tangent pass.
+//
 // Tangent rules (every one linear in the tangent):
 //   Linear   yd = xd W^T                     (no bias)
 //   ReLU     yd = yd_pre * [y > 0]           (mask = primal OUTPUT > 0, as torch's forward AD of relu)
@@ -17,6 +22,8 @@
 // sum (y - mu) yd} in the slot layout of the forward's, reduced in a fixed order (bit-reproducible).
 // The message LayerNorm is pushed through the receiver sum as in pdg_forward.cu:
 //   aggd = w [(aggrawd - deg mud1) r1 - (aggraw - deg mu1) r1^2 sigmad1].
+#include <algorithm>
+
 #include "pdg_ws.cuh"
 
 namespace pdg {
@@ -27,31 +34,43 @@ constexpr size_t SMEM_J2A = (size_t)(2 * TM * LDS + 2 * BK * H) * sizeof(float) 
 constexpr size_t SMEM_JENC = SMEM_J1A + TM * 16 * sizeof(float);
 constexpr size_t SMEM_JEDGE = (size_t)(3 * TM * LDS + 2 * BKJ * H) * sizeof(float) + 2 * TM * sizeof(int) + 16 * sizeof(double) +
                               8 * sizeof(float) + 4 * sizeof(unsigned) + TM + 1 + 256;
+// per tangent of an edge-kernel group: the LayerNorm tangent statistics {mud, c} and the fp64 partials {t1s, t1c, t2s, t2c}
+constexpr size_t SMEM_JEDGE_TAN = 2 * sizeof(float) + 4 * sizeof(double);
+static_assert(SMEM_JEDGE + PDG_JVP_MAX_TANGENTS * SMEM_JEDGE_TAN <= 227 * 1024, "edge JVP kernel exceeds shared memory");
+
+// tangent k's copy of a tangent-workspace buffer: p + k * (bytes between consecutive tangent workspaces)
+template <class T>
+__device__ __forceinline__ T* tan_at(T* p, size_t off) {
+  return p == nullptr ? p : reinterpret_cast<T*>(reinterpret_cast<uintptr_t>(p) + off);
+}
 
 // Tangent statistics of one LayerNorm instance: mud and c = r^2 sigmad, from the tangent partials and the primal
 // statistics st (ln_stat_block of the same slot).  CTA-wide; sm: >= 2 floats.
 struct LnTan { float mud, c; };
-__device__ __forceinline__ LnTan ln_tan_block(const double* __restrict__ tparts, double count, const LnStat& st, float* sm) {
-  if (threadIdx.x < 32) {
-    constexpr int K = (MAXP + 31) / 32;
-    double2 v[K];
+// one warp: the reduction of ln_tan_block; lane 0 writes {mud, c} to out
+__device__ __forceinline__ void ln_tan_warp(const double* __restrict__ tparts, double count, const LnStat& st, float* out) {
+  const int lane = threadIdx.x & 31;
+  constexpr int K = (MAXP + 31) / 32;
+  double2 v[K];
 #pragma unroll
-    for (int k = 0; k < K; ++k) {
-      const int i = threadIdx.x + 32 * k;
-      v[k] = i < MAXP ? reinterpret_cast<const double2*>(tparts)[i] : make_double2(0.0, 0.0);
-    }
-    double s = 0, sc = 0;
-#pragma unroll
-    for (int k = 0; k < K; ++k) { s += v[k].x; sc += v[k].y; }
-    s = warp_sum(s);
-    sc = warp_sum(sc);
-    if (threadIdx.x == 0) {
-      const double sigma = (double)st.sigma, r = (double)st.rstd;
-      const double sigd = sigma > 0 ? sc / (count * sigma) : 0.0;
-      sm[0] = (float)(s / count);
-      sm[1] = (float)(r * r * sigd);
-    }
+  for (int k = 0; k < K; ++k) {
+    const int i = lane + 32 * k;
+    v[k] = i < MAXP ? reinterpret_cast<const double2*>(tparts)[i] : make_double2(0.0, 0.0);
   }
+  double s = 0, sc = 0;
+#pragma unroll
+  for (int k = 0; k < K; ++k) { s += v[k].x; sc += v[k].y; }
+  s = warp_sum(s);
+  sc = warp_sum(sc);
+  if (lane == 0) {
+    const double sigma = (double)st.sigma, r = (double)st.rstd;
+    const double sigd = sigma > 0 ? sc / (count * sigma) : 0.0;
+    out[0] = (float)(s / count);
+    out[1] = (float)(r * r * sigd);
+  }
+}
+__device__ __forceinline__ LnTan ln_tan_block(const double* __restrict__ tparts, double count, const LnStat& st, float* sm) {
+  if (threadIdx.x < 32) ln_tan_warp(tparts, count, st, sm);
   __syncthreads();
   LnTan t;
   t.mud = sm[0];
@@ -105,8 +124,12 @@ k_node_encoder_jvp(const float* __restrict__ mean_stress, const float* __restric
                    pdg_norm_t nrm, int scale_in, const float* __restrict__ tan_ms, const float* __restrict__ tan_pos,
                    const float* __restrict__ W0, const float* __restrict__ b0, const float* __restrict__ Wt2,
                    const float* __restrict__ y_nenc, const double* __restrict__ parts, double count, float* __restrict__ yd_out,
-                   double* __restrict__ tparts, int N, int n_tiles) {
+                   double* __restrict__ tparts, int N, int n_tiles, int64_t ms_stride, int64_t pos_stride, size_t tws) {
   extern __shared__ __align__(16) float smem[];
+  if (tan_ms != nullptr) tan_ms += blockIdx.y * ms_stride;
+  if (tan_pos != nullptr) tan_pos += blockIdx.y * pos_stride;
+  yd_out = tan_at(yd_out, blockIdx.y * tws);
+  tparts = tan_at(tparts, blockIdx.y * tws);
   float* A = smem;
   float* Ws = A + TM * LDS;
   float* feat = Ws + 2 * BK * H;  // [TM][8] primal features
@@ -187,8 +210,12 @@ __global__ void __launch_bounds__(NT, 1)
 k_edge_encoder_jvp(const float* __restrict__ edge_attr, const int32_t* __restrict__ perm, pdg_norm_t nrm, int scale_in,
                    const float* __restrict__ tan_ea, const float* __restrict__ W0, const float* __restrict__ b0,
                    const float* __restrict__ Wt2, const float* __restrict__ y_eenc, const double* __restrict__ parts,
-                   double count, float* __restrict__ yd_out, double* __restrict__ tparts, int E, int n_tiles) {
+                   double count, float* __restrict__ yd_out, double* __restrict__ tparts, int E, int n_tiles,
+                   int64_t ea_stride, size_t tws) {
   extern __shared__ __align__(16) float smem[];
+  if (tan_ea != nullptr) tan_ea += blockIdx.y * ea_stride;
+  yd_out = tan_at(yd_out, blockIdx.y * tws);
+  tparts = tan_at(tparts, blockIdx.y * tws);
   float* A = smem;
   float* Ws = A + TM * LDS;
   float* feat = Ws + 2 * BK * H;  // [TM]
@@ -242,8 +269,17 @@ __global__ void __launch_bounds__(NT, 1)
 k_node_pre_jvp(const float* __restrict__ yprev, const double* __restrict__ prev_parts, const double* __restrict__ tprev_parts,
                double prev_count, const float* __restrict__ lnw, const float* __restrict__ tbase,
                const float* __restrict__ typrev, float* __restrict__ tx_out, const float* __restrict__ WtA,
-               const float* __restrict__ WtB, float* __restrict__ tPa, float* __restrict__ tPb, int n_tiles) {
+               const float* __restrict__ WtB, float* __restrict__ tPa, float* __restrict__ tPb, int n_tiles, size_t tws) {
   extern __shared__ __align__(16) float smem[];
+  {
+    const size_t off = blockIdx.y * tws;
+    tprev_parts = tan_at(tprev_parts, off);
+    tbase = tan_at(tbase, off);
+    typrev = tan_at(typrev, off);
+    tx_out = tan_at(tx_out, off);
+    tPa = tan_at(tPa, off);
+    tPb = tan_at(tPb, off);
+  }
   float* A = smem;
   float* Ws = A + TM * LDS;
   float* smf = Ws + 2 * BK * H;
@@ -291,7 +327,10 @@ k_node_pre_jvp(const float* __restrict__ yprev, const double* __restrict__ prev_
 //   y1    = relu(relu(G + Pa[recv] + Pb[send]) W2^T + b2)          (recomputed: the forward keeps its segment sums only)
 //   y1d   = [y1 > 0] ((m1 (Gd + Pad[recv] + Pbd[send])) W2^T)    -> segment sums into aggrawd, partials LN1
 //   y2d   = [y2_t > 0] ((m2 (Gd + Pad[send] + Pbd[recv])) W2^T)  -> in place over yd_prev, partials LN2 (not on the last step)
-// Tiles: T0 e_t -> h1 -> y1 -> h2d;  T1 G -> h1d -> y1d;  T2 ed_t -> Gd.  Five GEMMs per tile against the forward's three.
+// A CTA takes a group of C tangents: the primal part (G, both masks, y1) runs once per tile, then each tangent of the
+// group runs Gd, y1d and y2d.
+// Tiles: T0 e_t -> h1 -> y1 (kept for the whole group);  T1 G, then per tangent h1d -> y1d -> h2d;  T2 ed_t -> Gd.
+// Two GEMMs per tile plus three per tangent, against the forward's three.
 // ------------------------------------------------------------------------------------
 struct EdgeJvpArgs {
   // primal state (forward workspace)
@@ -324,6 +363,8 @@ struct EdgeJvpArgs {
   const float* b2;
   double count;
   int E, n_tiles;
+  size_t tws;  // bytes between consecutive tangent workspaces
+  int K, C;    // tangents of the pass; tangents per CTA group (blockIdx.y = group)
 };
 
 // acc = relu(G + P1[idx1[row]] + P2[idx2[row]])  (the arithmetic of k_edge_step's gather_hidden, so the masks are its)
@@ -383,6 +424,40 @@ __device__ __forceinline__ unsigned long long pos_bits(const float (&acc)[8][8])
   return m;
 }
 
+// ed_t = ed_{t-1} + LN-tangent(y2_{t-1}) of one tangent (workspace offset off, statistics tt2 = {mud, c}) on the tile's
+// rows -> T2, and to te_out (in place over ed_{t-1}) when the next step reads it
+__device__ __forceinline__ void load_ed(const EdgeJvpArgs& a, const LnStat& st, const float* tt2, const float4 w, int row0,
+                                        size_t off, float* T2) {
+  const int tid = threadIdx.x;
+  const int c4 = (tid & 31) * 4;
+  LnTan tt;
+  tt.mud = tt2[0];
+  tt.c = tt2[1];
+  const float* tbase = tan_at(a.tbase, off);
+  const float* typrev = tan_at(a.typrev, off);
+  float* te_out = tan_at(a.te_out, off);
+#pragma unroll
+  for (int bt = 0; bt < 4; ++bt) {
+    float4 ly[4], ld[4], lx[4];
+#pragma unroll
+    for (int k = 0; k < 4; ++k) {
+      const size_t g = ((size_t)row0 + (tid >> 5) + (bt * 4 + k) * 8) * H + c4;
+      ly[k] = *reinterpret_cast<const float4*>(a.yprev + g);
+      ld[k] = *reinterpret_cast<const float4*>(typrev + g);
+      lx[k] = tbase != nullptr ? *reinterpret_cast<const float4*>(tbase + g) : make_float4(0.f, 0.f, 0.f, 0.f);
+    }
+#pragma unroll
+    for (int k = 0; k < 4; ++k) {
+      const int r = (tid >> 5) + (bt * 4 + k) * 8;
+      const size_t g = ((size_t)row0 + r) * H + c4;
+      float4 v = ln_tan4(ly[k], ld[k], st, tt, w);
+      v.x += lx[k].x; v.y += lx[k].y; v.z += lx[k].z; v.w += lx[k].w;
+      if (te_out != nullptr) *reinterpret_cast<float4*>(te_out + g) = v;
+      *reinterpret_cast<float4*>(T2 + r * LDS + c4) = v;
+    }
+  }
+}
+
 __global__ void __launch_bounds__(NT, 1) k_edge_step_jvp(EdgeJvpArgs a) {
   extern __shared__ __align__(16) float smem[];
   float* T0 = smem;
@@ -395,15 +470,19 @@ __global__ void __launch_bounds__(NT, 1) k_edge_step_jvp(EdgeJvpArgs a) {
   float* smf = (float*)(red + 16);
   unsigned* seg_masks = (unsigned*)(smf + 8);
   unsigned char* seg_row = (unsigned char*)(seg_masks + 4);  // [TM + 1]
+  // per tangent of the group (SMEM_JEDGE_TAN each, above the 16-byte-aligned end of seg_row)
+  double* tsum = (double*)(((uintptr_t)(seg_row + TM + 1) + 15) & ~(uintptr_t)15);  // [C][4] {t1s, t1c, t2s, t2c}
+  float* ttan = (float*)(tsum + 4 * a.C);                                           // [C][2] {mud, c}
   const int tid = threadIdx.x;
   const int c4 = (tid & 31) * 4;
   const bool upd = a.ty2_out != nullptr;
+  const int k0 = blockIdx.y * a.C, nk = min(a.C, a.K - k0);  // this CTA's tangents: k0 .. k0 + nk - 1
   const LnStat st = ln_stat_block(a.prev_parts, a.count, smf);
-  const LnTan tt = ln_tan_block(a.tprev_parts, a.count, st, smf);
-  const float mu1 = ln_stat_block(a.parts1, a.count, smf).mu;
+  for (int c = tid >> 5; c < nk; c += NT / 32) ln_tan_warp(tan_at(a.tprev_parts, (k0 + c) * a.tws), a.count, st, ttan + 2 * c);
+  for (int i = tid; i < 4 * nk; i += NT) tsum[i] = 0.0;
+  const float mu1 = ln_stat_block(a.parts1, a.count, smf).mu;  // its barriers publish ttan and tsum
   const float mu2 = upd ? ln_stat_block(a.parts2, a.count, smf).mu : 0.f;
   const float4 w = *reinterpret_cast<const float4*>(a.prev_w + c4);
-  double t1s = 0, t1c = 0, t2s = 0, t2c = 0;
   for (int tile = blockIdx.x; tile < a.n_tiles; tile += gridDim.x) {
     const int row0 = tile * TM;
     const int nvalid = min(TM, a.E - row0);
@@ -411,37 +490,18 @@ __global__ void __launch_bounds__(NT, 1) k_edge_step_jvp(EdgeJvpArgs a) {
       recv_s[tid] = a.recv[row0 + tid];
       send_s[tid] = a.send[row0 + tid];
     }
-    // ---- primal e_t rows straight into T0 (asynchronous); tangent ed_t (lazy LN tangent + residual) into T2 ----
+    // ---- primal part, once per tile for the whole group: G = e_t We^T + b1 -> T1, masks, y1 -> T0.  e_t arrives in
+    // T0 asynchronously while the group's first ed_t goes to T2 (the primal part does not touch T2) ----
 #pragma unroll
     for (int it = 0; it < (TM * H / 4) / NT; ++it) {
       const int r = (tid >> 5) + it * 8;
       cp_async16(T0 + r * LDS + c4, a.e_t + ((size_t)row0 + r) * H + c4);
     }
     cp_async_commit();
-#pragma unroll
-    for (int bt = 0; bt < 4; ++bt) {
-      float4 ly[4], ld[4], lx[4];
-#pragma unroll
-      for (int k = 0; k < 4; ++k) {
-        const size_t g = ((size_t)row0 + (tid >> 5) + (bt * 4 + k) * 8) * H + c4;
-        ly[k] = *reinterpret_cast<const float4*>(a.yprev + g);
-        ld[k] = *reinterpret_cast<const float4*>(a.typrev + g);
-        lx[k] = a.tbase != nullptr ? *reinterpret_cast<const float4*>(a.tbase + g) : make_float4(0.f, 0.f, 0.f, 0.f);
-      }
-#pragma unroll
-      for (int k = 0; k < 4; ++k) {
-        const int r = (tid >> 5) + (bt * 4 + k) * 8;
-        const size_t g = ((size_t)row0 + r) * H + c4;
-        float4 v = ln_tan4(ly[k], ld[k], st, tt, w);
-        v.x += lx[k].x; v.y += lx[k].y; v.z += lx[k].z; v.w += lx[k].w;
-        if (a.te_out != nullptr) *reinterpret_cast<float4*>(a.te_out + g) = v;
-        *reinterpret_cast<float4*>(T2 + r * LDS + c4) = v;
-      }
-    }
+    load_ed(a, st, ttan, w, row0, (size_t)k0 * a.tws, T2);
     cp_async_wait<0>();
     __syncthreads();  // recv_s/send_s, T0, T2 visible
     const int nseg = tile_segments(recv_s, nvalid, seg_row, seg_masks);
-    // ---- G = e_t We^T + b1 -> T1;  Gd = ed_t We^T -> T2 ----
     float acc[8][8];
     acc_zero(acc);
     gemm_rowA<BKJ>(T0, a.WtE, H, acc, Ws);
@@ -454,11 +514,7 @@ __global__ void __launch_bounds__(NT, 1) k_edge_step_jvp(EdgeJvpArgs a) {
         for (int j = 0; j < 8; ++j) acc[i][j] += bias1[j];
     }
     acc_store(acc, T1, LDS);
-    acc_zero(acc);
-    gemm_rowA<BKJ>(T2, a.WtE, H, acc, Ws);
-    acc_store(acc, T2, LDS);
-    __syncthreads();  // T1, T2 visible
-    // ---- hidden masks of both evaluations while G is live; h1 -> T0 ----
+    __syncthreads();  // T1 visible
     unsigned long long m2 = 0;
     if (upd) {
       gather_hidden_j(acc, T1, a.Pa, send_s, a.Pb, recv_s);
@@ -467,7 +523,6 @@ __global__ void __launch_bounds__(NT, 1) k_edge_step_jvp(EdgeJvpArgs a) {
     gather_hidden_j(acc, T1, a.Pa, recv_s, a.Pb, send_s);
     const unsigned long long m1 = pos_bits(acc);
     acc_store(acc, T0, LDS);
-    // ---- y1 = relu(h1 W2^T + b2) -> T0 ----
     acc_zero(acc);
     gemm_rowA<BKJ>(T0, a.Wt2, H, acc, Ws);
     {
@@ -478,40 +533,57 @@ __global__ void __launch_bounds__(NT, 1) k_edge_step_jvp(EdgeJvpArgs a) {
 #pragma unroll
         for (int j = 0; j < 8; ++j) acc[i][j] = fmaxf(acc[i][j] + bias2[j], 0.f);
     }
-    acc_store(acc, T0, LDS);
-    // ---- h1d -> T1 (G is dead: both masks are in registers; the GEMM above separated its last reads) ----
-    gather_hidden_tan(acc, T2, a.tPa, recv_s, a.tPb, send_s, m1);
-    acc_store(acc, T1, LDS);
-    acc_zero(acc);
-    gemm_rowA<BKJ>(T1, a.Wt2, H, acc, Ws);  // its first barrier also makes y1 in T0 visible
-    {
-      float s = 0.f, c = 0.f;
-      relu_mask_stats(acc, T0, LDS, mu1, nvalid, s, c);  // y1d, partials of LN1
-      acc_store(acc, T1, LDS);
-      __syncthreads();
-      float u0 = 0.f, u1 = 0.f;
-      tile_segsum_warp<false>(T1, recv_s, seg_row, nseg, a.rowptr, row0, nvalid, a.taggraw, u0, u1);
-      finish_partials(s, c, red, t1s, t1c);  // its barriers also end every read of y1 in T0
-    }
-    // ---- edge-update tangent (skipped on the last step, as in the forward) ----
-    if (upd) {
-      gather_hidden_tan(acc, T2, a.tPa, send_s, a.tPb, recv_s, m2);
-      acc_store(acc, T0, LDS);
+    acc_store(acc, T0, LDS);  // y1 stays in T0 until the group's last tangent; G in T1 is dead (masks are in registers)
+    // ---- tangents of the group ----
+    for (int c = 0; c < nk; ++c) {
+      const size_t off = (size_t)(k0 + c) * a.tws;
+      if (c > 0) load_ed(a, st, ttan + 2 * c, w, row0, off, T2);
+      // ---- Gd = ed_t We^T -> T2 (ed_t of tangent 0 was loaded with e_t) ----
       acc_zero(acc);
-      gemm_rowA<BKJ>(T0, a.Wt2, H, acc, Ws);
-      float s = 0.f, c = 0.f;
-      relu_mask_stats(acc, a.y2_t + (size_t)row0 * H, H, mu2, nvalid, s, c);
-      acc_store(acc, a.ty2_out + (size_t)row0 * H, H);
-      finish_partials(s, c, red, t2s, t2c);
+      gemm_rowA<BKJ>(T2, a.WtE, H, acc, Ws);  // its first barrier also makes y1 in T0 visible
+      acc_store(acc, T2, LDS);
+      __syncthreads();  // T2 visible
+      // ---- h1d -> T1 ----
+      const float* tPa = tan_at(a.tPa, off);
+      const float* tPb = tan_at(a.tPb, off);
+      gather_hidden_tan(acc, T2, tPa, recv_s, tPb, send_s, m1);
+      acc_store(acc, T1, LDS);
+      acc_zero(acc);
+      gemm_rowA<BKJ>(T1, a.Wt2, H, acc, Ws);
+      {
+        float s = 0.f, cc = 0.f;
+        relu_mask_stats(acc, T0, LDS, mu1, nvalid, s, cc);  // y1d, partials of LN1
+        acc_store(acc, T1, LDS);
+        __syncthreads();
+        float u0 = 0.f, u1 = 0.f;
+        tile_segsum_warp<false>(T1, recv_s, seg_row, nseg, a.rowptr, row0, nvalid, tan_at(a.taggraw, off), u0, u1);
+        finish_partials(s, cc, red, tsum[4 * c], tsum[4 * c + 1]);  // its barriers also end every read of T1
+      }
+      // ---- edge-update tangent (skipped on the last step, as in the forward); h2d -> T1, T0 keeps y1 ----
+      if (upd) {
+        gather_hidden_tan(acc, T2, tPa, send_s, tPb, recv_s, m2);
+        acc_store(acc, T1, LDS);
+        acc_zero(acc);
+        gemm_rowA<BKJ>(T1, a.Wt2, H, acc, Ws);
+        float s = 0.f, cc = 0.f;
+        relu_mask_stats(acc, a.y2_t + (size_t)row0 * H, H, mu2, nvalid, s, cc);
+        acc_store(acc, tan_at(a.ty2_out, off) + (size_t)row0 * H, H);
+        finish_partials(s, cc, red, tsum[4 * c + 2], tsum[4 * c + 3]);
+      }
+      __syncthreads();
     }
-    __syncthreads();
   }
   if (tid == 0) {
-    a.tparts1[2 * blockIdx.x] = t1s;
-    a.tparts1[2 * blockIdx.x + 1] = t1c;
-    if (a.tparts2 != nullptr) {
-      a.tparts2[2 * blockIdx.x] = t2s;
-      a.tparts2[2 * blockIdx.x + 1] = t2c;
+    for (int c = 0; c < nk; ++c) {
+      const size_t off = (size_t)(k0 + c) * a.tws;
+      double* p1 = tan_at(a.tparts1, off);
+      p1[2 * blockIdx.x] = tsum[4 * c];
+      p1[2 * blockIdx.x + 1] = tsum[4 * c + 1];
+      if (a.tparts2 != nullptr) {
+        double* p2 = tan_at(a.tparts2, off);
+        p2[2 * blockIdx.x] = tsum[4 * c + 2];
+        p2[2 * blockIdx.x + 1] = tsum[4 * c + 3];
+      }
     }
   }
 }
@@ -526,8 +598,16 @@ k_node_update_jvp(const float* __restrict__ aggraw, const float* __restrict__ ta
                   const float* __restrict__ lnw_e, const float* __restrict__ tx_t, const float* __restrict__ WtA,
                   const float* __restrict__ WtX, const float* __restrict__ hq, const float* __restrict__ Wt2,
                   const float* __restrict__ y3, const double* __restrict__ parts3, double count3, float* __restrict__ ty3_out,
-                  double* __restrict__ tparts3, int N, int n_tiles) {
+                  double* __restrict__ tparts3, int N, int n_tiles, size_t tws) {
   extern __shared__ __align__(16) float smem[];
+  {
+    const size_t off = blockIdx.y * tws;
+    taggraw = tan_at(taggraw, off);
+    tparts1 = tan_at(tparts1, off);
+    tx_t = tan_at(tx_t, off);
+    ty3_out = tan_at(ty3_out, off);
+    tparts3 = tan_at(tparts3, off);
+  }
   float* A0 = smem;
   float* A1 = A0 + TM * LDS;
   float* Ws = A1 + TM * LDS;
@@ -599,8 +679,15 @@ k_decoder_jvp(const float* __restrict__ yprev, const double* __restrict__ prev_p
               double prev_count, const float* __restrict__ lnw, const float* __restrict__ tbase,
               const float* __restrict__ typrev, const float* __restrict__ WtD, const float* __restrict__ hd,
               const float* __restrict__ D2, float out_scale, float* __restrict__ tout, const int* __restrict__ nzflag, int N,
-              int n_tiles) {
+              int n_tiles, size_t tws) {
   extern __shared__ __align__(16) float smem[];
+  {
+    const size_t off = blockIdx.y * tws;
+    tprev_parts = tan_at(tprev_parts, off);
+    tbase = tan_at(tbase, off);
+    typrev = tan_at(typrev, off);
+    tout += (size_t)blockIdx.y * N * PDG_OUT;  // [K][N][3]
+  }
   float* A = smem;
   float* Ws = A + TM * LDS;
   float* smf = Ws + 2 * BK * H;
@@ -658,18 +745,30 @@ static int set_smem_j(const void* fn, size_t bytes) {
 using namespace pdg;
 
 // The tangent workspace has the buffers of a forward without PDG_FLAG_SAVE: ping-pong xd, Pad, Pbd, aggrawd, y3d,
-// ed updated in place, y2d over yd_eenc; its LayerNorm partials hold the tangent partials.
+// ed updated in place, y2d over yd_eenc; its LayerNorm partials hold the tangent partials.  A batched pass keeps K of
+// them one after another (the total is a multiple of 256 bytes, so every copy stays aligned).
 extern "C" size_t pdg_jvp_ws_bytes(int64_t n_nodes, int64_t n_edges, int steps) {
   if (steps < 1 || steps > 62) return 0;
   return FwdWs(n_nodes, n_edges, steps, false, nullptr, false).total;
 }
 
-extern "C" int pdg_jvp(const pdg_params_t* params, const pdg_norm_t* norm, const float* mean_stress, const float* pos,
-                       const int64_t* nodes_types, const float* edge_attr, const void* plan, int64_t n_nodes, int64_t n_edges,
-                       int steps, int flags, int precision, const void* fwd_ws, void* jvp_ws, size_t jvp_ws_bytes,
-                       const float* tan_mean_stress, const float* tan_pos, const float* tan_edge_attr,
-                       float* tan_local_stress, void* stream_) {
+extern "C" size_t pdg_jvp_batched_ws_bytes(int64_t n_nodes, int64_t n_edges, int steps, int n_tangents) {
+  if (n_tangents < 1 || n_tangents > PDG_JVP_MAX_TANGENTS) return 0;
+  return (size_t)n_tangents * pdg_jvp_ws_bytes(n_nodes, n_edges, steps);
+}
+
+extern "C" int pdg_jvp_batched(const pdg_params_t* params, const pdg_norm_t* norm, const float* mean_stress, const float* pos,
+                               const int64_t* nodes_types, const float* edge_attr, const void* plan, int64_t n_nodes,
+                               int64_t n_edges, int steps, int flags, int precision, const void* fwd_ws, void* jvp_ws,
+                               size_t jvp_ws_bytes, int n_tangents, const float* tan_mean_stress, int64_t ms_stride,
+                               const float* tan_pos, int64_t pos_stride, const float* tan_edge_attr, int64_t ea_stride,
+                               float* tan_local_stress, void* stream_) {
   cudaStream_t st = (cudaStream_t)stream_;
+  const int K = n_tangents;
+  if (K < 1 || K > PDG_JVP_MAX_TANGENTS) {
+    set_error("pdg_jvp_batched: n_tangents=%d outside 1..%d", K, PDG_JVP_MAX_TANGENTS);
+    return -1;
+  }
   if (steps < 1 || steps > 62) { set_error("pdg_jvp: steps=%d unsupported", steps); return -1; }
   if (precision != PDG_PREC_FP32) {
     set_error("pdg_jvp: only the fp32 mode (PDG_PREC_FP32) has a forward-mode derivative; the 16-bit mode's per-row "
@@ -680,7 +779,8 @@ extern "C" int pdg_jvp(const pdg_params_t* params, const pdg_norm_t* norm, const
   if (n_nodes <= 0 || n_edges <= 0) { set_error("pdg_jvp: empty graph"); return -1; }
   const FwdWs F(n_nodes, n_edges, steps, true, const_cast<void*>(fwd_ws), false);
   const FwdWs J(n_nodes, n_edges, steps, false, jvp_ws, false);
-  if (jvp_ws_bytes < J.total) { set_error("pdg_jvp: workspace %zu < %zu", jvp_ws_bytes, J.total); return -1; }
+  const size_t tws = J.total;  // bytes between consecutive tangent workspaces
+  if (jvp_ws_bytes < (size_t)K * tws) { set_error("pdg_jvp: workspace %zu < %zu", jvp_ws_bytes, (size_t)K * tws); return -1; }
   const int N = (int)n_nodes, E = (int)n_edges, T = steps;
   int32_t *perm, *recv, *send, *rowptr;
   pdg_plan_views(const_cast<void*>(plan), n_nodes, n_edges, &perm, &recv, &send, &rowptr, nullptr, nullptr);
@@ -688,32 +788,39 @@ extern "C" int pdg_jvp(const pdg_params_t* params, const pdg_norm_t* norm, const
   int sms = num_sms();
   if (sms > MAXP) sms = MAXP;
   const int grid_n = balanced_grid(nt_n, sms), grid_e = balanced_grid(nt_e, sms);
+  // Edge kernel: tangent groups of C over the SMs the x-grid leaves idle.  One group of all K (C = K) shares the primal
+  // part of every tile across the K tangents; more groups spread the tangents of a small graph over idle SMs.
+  int groups = std::min(K, std::max(1, sms / grid_e));
+  const int C = (K + groups - 1) / groups;
+  groups = (K + C - 1) / C;  // no empty group
+  const size_t smem_edge = SMEM_JEDGE + (size_t)C * SMEM_JEDGE_TAN;
   const double cnt_n = (double)N * H, cnt_e = (double)E * H;
   if (set_smem_j((const void*)k_node_encoder_jvp, SMEM_JENC)) return -2;
   if (set_smem_j((const void*)k_edge_encoder_jvp, SMEM_JENC)) return -2;
   if (set_smem_j((const void*)k_node_pre_jvp, SMEM_J1A)) return -2;
-  if (set_smem_j((const void*)k_edge_step_jvp, SMEM_JEDGE)) return -2;
+  if (set_smem_j((const void*)k_edge_step_jvp, smem_edge)) return -2;
   if (set_smem_j((const void*)k_node_update_jvp, SMEM_J2A)) return -2;
   if (set_smem_j((const void*)k_decoder_jvp, SMEM_J1A)) return -2;
 
-  // tangent partials: slots of CTAs that do not exist must read as zero
-  PDG_CUDA_CHECK(cudaMemsetAsync(J.parts, 0, (size_t)(2 + 3 * T) * MAXP * 2 * sizeof(double), st));
+  // tangent partials of all K tangents (one strided memset): slots of CTAs that do not exist must read as zero
+  PDG_CUDA_CHECK(cudaMemset2DAsync(J.parts, tws, 0, (size_t)(2 + 3 * T) * MAXP * 2 * sizeof(double), K, st));
   const int* nzflag = (flags & PDG_FLAG_ZERO_CHECK) ? F.nzflag : nullptr;
   const float* const* P = params->p;
   const float* pk = F.pack;
   const int scale_in = (flags & PDG_FLAG_SCALE_INPUT) ? 1 : 0;
+  const dim3 gn(grid_n, K), ge(grid_e, K);
   {
     ScopedTimer tm_(KC_JVP_NODE_ENC, st);
-    k_node_encoder_jvp<<<grid_n, NT, SMEM_JENC, st>>>(mean_stress, pos, nodes_types, *norm, scale_in, tan_mean_stress, tan_pos,
-                                                      P[NE_W0], P[NE_B0], pk + PackOffsets::NE_W2T, F.y_nenc, F.parts_slot(0),
-                                                      cnt_n, J.y_nenc, J.parts_slot(0), N, nt_n);
+    k_node_encoder_jvp<<<gn, NT, SMEM_JENC, st>>>(mean_stress, pos, nodes_types, *norm, scale_in, tan_mean_stress, tan_pos,
+                                                  P[NE_W0], P[NE_B0], pk + PackOffsets::NE_W2T, F.y_nenc, F.parts_slot(0),
+                                                  cnt_n, J.y_nenc, J.parts_slot(0), N, nt_n, ms_stride, pos_stride, tws);
   }
   PDG_LAUNCH_CHECK();
   {
     ScopedTimer tm_(KC_JVP_EDGE_ENC, st);
-    k_edge_encoder_jvp<<<grid_e, NT, SMEM_JENC, st>>>(edge_attr, perm, *norm, scale_in, tan_edge_attr, P[EE_W0], P[EE_B0],
-                                                      pk + PackOffsets::EE_W2T, F.y_eenc, F.parts_slot(1), cnt_e, J.y_eenc,
-                                                      J.parts_slot(1), E, nt_e);
+    k_edge_encoder_jvp<<<ge, NT, SMEM_JENC, st>>>(edge_attr, perm, *norm, scale_in, tan_edge_attr, P[EE_W0], P[EE_B0],
+                                                  pk + PackOffsets::EE_W2T, F.y_eenc, F.parts_slot(1), cnt_e, J.y_eenc,
+                                                  J.parts_slot(1), E, nt_e, ea_stride, tws);
   }
   PDG_LAUNCH_CHECK();
   for (int t = 0; t < T; ++t) {
@@ -721,13 +828,13 @@ extern "C" int pdg_jvp(const pdg_params_t* params, const pdg_norm_t* norm, const
     {
       ScopedTimer tm_(KC_JVP_NODE_PRE, st);
       const int ps = first ? 0 : slot_ln3(t - 1);
-      k_node_pre_jvp<<<grid_n, NT, SMEM_J1A, st>>>(first ? F.y_nenc : F.y3_[t - 1], F.parts_slot(ps), J.parts_slot(ps), cnt_n,
-                                                   first ? P[NE_LNW] : P[PN_LNW], first ? nullptr : J.x_[t - 1],
-                                                   first ? J.y_nenc : J.y3_[t - 1], J.x_[t], pk + PackOffsets::PE_WAT,
-                                                   pk + PackOffsets::PE_WBT, J.Pa_[t], J.Pb_[t], nt_n);
+      k_node_pre_jvp<<<gn, NT, SMEM_J1A, st>>>(first ? F.y_nenc : F.y3_[t - 1], F.parts_slot(ps), J.parts_slot(ps), cnt_n,
+                                               first ? P[NE_LNW] : P[PN_LNW], first ? nullptr : J.x_[t - 1],
+                                               first ? J.y_nenc : J.y3_[t - 1], J.x_[t], pk + PackOffsets::PE_WAT,
+                                               pk + PackOffsets::PE_WBT, J.Pa_[t], J.Pb_[t], nt_n, tws);
     }
     PDG_LAUNCH_CHECK();
-    PDG_CUDA_CHECK(cudaMemsetAsync(J.aggraw_[t], 0, (size_t)J.N_pad * H * sizeof(float), st));
+    PDG_CUDA_CHECK(cudaMemset2DAsync(J.aggraw_[t], tws, 0, (size_t)J.N_pad * H * sizeof(float), K, st));
     EdgeJvpArgs a;
     const int ps = first ? 1 : slot_ln2(t - 1);
     a.yprev = first ? F.y_eenc : F.y2_[t - 1];
@@ -759,28 +866,41 @@ extern "C" int pdg_jvp(const pdg_params_t* params, const pdg_norm_t* norm, const
     a.count = cnt_e;
     a.E = E;
     a.n_tiles = nt_e;
+    a.tws = tws;
+    a.K = K;
+    a.C = C;
     {
       ScopedTimer tm_(KC_JVP_EDGE_STEP, st);
-      k_edge_step_jvp<<<grid_e, NT, SMEM_JEDGE, st>>>(a);
+      k_edge_step_jvp<<<dim3(grid_e, groups), NT, smem_edge, st>>>(a);
     }
     PDG_LAUNCH_CHECK();
     {
       ScopedTimer tm_(KC_JVP_NODE_UPD, st);
-      k_node_update_jvp<<<grid_n, NT, SMEM_J2A, st>>>(F.aggraw_[t], J.aggraw_[t], rowptr, F.parts_slot(slot_ln1(t)),
-                                                      J.parts_slot(slot_ln1(t)), cnt_e, P[PE_LNW], J.x_[t],
-                                                      pk + PackOffsets::PN_WAT, pk + PackOffsets::PN_WXT, F.hq_[t],
-                                                      pk + PackOffsets::PN_W2T, F.y3_[t], F.parts_slot(slot_ln3(t)), cnt_n,
-                                                      J.y3_[t], J.parts_slot(slot_ln3(t)), N, nt_n);
+      k_node_update_jvp<<<gn, NT, SMEM_J2A, st>>>(F.aggraw_[t], J.aggraw_[t], rowptr, F.parts_slot(slot_ln1(t)),
+                                                  J.parts_slot(slot_ln1(t)), cnt_e, P[PE_LNW], J.x_[t],
+                                                  pk + PackOffsets::PN_WAT, pk + PackOffsets::PN_WXT, F.hq_[t],
+                                                  pk + PackOffsets::PN_W2T, F.y3_[t], F.parts_slot(slot_ln3(t)), cnt_n,
+                                                  J.y3_[t], J.parts_slot(slot_ln3(t)), N, nt_n, tws);
     }
     PDG_LAUNCH_CHECK();
   }
   const bool scale_out = (flags & PDG_FLAG_SCALE_OUTPUT) != 0;
   {
     ScopedTimer tm_(KC_JVP_DECODER, st);
-    k_decoder_jvp<<<grid_n, NT, SMEM_J1A, st>>>(F.y3_[T - 1], F.parts_slot(slot_ln3(T - 1)), J.parts_slot(slot_ln3(T - 1)), cnt_n,
-                                                P[PN_LNW], J.x_[T - 1], J.y3_[T - 1], pk + PackOffsets::ND_W0T, F.hd, P[ND_W2],
-                                                scale_out ? norm->std_local_stress : 1.f, tan_local_stress, nzflag, N, nt_n);
+    k_decoder_jvp<<<gn, NT, SMEM_J1A, st>>>(F.y3_[T - 1], F.parts_slot(slot_ln3(T - 1)), J.parts_slot(slot_ln3(T - 1)), cnt_n,
+                                            P[PN_LNW], J.x_[T - 1], J.y3_[T - 1], pk + PackOffsets::ND_W0T, F.hd, P[ND_W2],
+                                            scale_out ? norm->std_local_stress : 1.f, tan_local_stress, nzflag, N, nt_n, tws);
   }
   PDG_LAUNCH_CHECK();
   return 0;
+}
+
+extern "C" int pdg_jvp(const pdg_params_t* params, const pdg_norm_t* norm, const float* mean_stress, const float* pos,
+                       const int64_t* nodes_types, const float* edge_attr, const void* plan, int64_t n_nodes, int64_t n_edges,
+                       int steps, int flags, int precision, const void* fwd_ws, void* jvp_ws, size_t jvp_ws_bytes,
+                       const float* tan_mean_stress, const float* tan_pos, const float* tan_edge_attr,
+                       float* tan_local_stress, void* stream) {
+  return pdg_jvp_batched(params, norm, mean_stress, pos, nodes_types, edge_attr, plan, n_nodes, n_edges, steps, flags,
+                         precision, fwd_ws, jvp_ws, jvp_ws_bytes, 1, tan_mean_stress, 0, tan_pos, 0, tan_edge_attr, 0,
+                         tan_local_stress, stream);
 }
