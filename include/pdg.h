@@ -176,6 +176,25 @@ int pdg_jvp_batched(const pdg_params_t* params, const pdg_norm_t* norm, const fl
                     const float* tan_pos, int64_t pos_stride, const float* tan_edge_attr, int64_t ea_stride,
                     float* tan_local_stress, void* stream);
 
+/* ---- batched reverse-mode derivative (vector-Jacobian products) of the inputs -----------------------
+ * For n_cotangents (1..PDG_VJP_MAX_COTANGENTS) cotangents K of local_stress, grad_local_stress [K][N][3], writes
+ * d <u_k, local_stress> / d (mean_stress, pos, edge_attr) into each non-NULL output (overwritten, not accumulated):
+ * grad_mean_stress [K][N][3], grad_pos [K][N][2], grad_edge_attr [K][E] in the caller's (PyG) edge order.  No parameter
+ * gradient is formed.  fwd_ws is the workspace of a pdg_forward with PDG_FLAG_SAVE and the same arguments (flags
+ * included); it is only read, so a pdg_backward may follow.  vjp_ws: pdg_vjp_batched_ws_bytes (K cotangent workspaces
+ * of the data-gradient buffers of the backward; 0 for K or steps out of range).  Column k has the bits of the input
+ * gradients of pdg_backward_inputs with cotangent k, the same flags and PDG_PREC_FP32.  Launches the same kernels for
+ * any K.  Returns -1 for K outside 1..PDG_VJP_MAX_COTANGENTS, precision != PDG_PREC_FP32, flags without PDG_FLAG_SAVE,
+ * steps outside 1..62, a workspace that is too small, three NULL outputs and an empty graph.
+ * Replaces torch.func.jacrev / torch.func.vmap over torch.func.vjp through models.py:288-326. */
+#define PDG_VJP_MAX_COTANGENTS 64
+size_t pdg_vjp_batched_ws_bytes(int64_t n_nodes, int64_t n_edges, int steps, int n_cotangents);
+int pdg_vjp_batched(const pdg_params_t* params, const pdg_norm_t* norm, const float* mean_stress, const float* pos,
+                    const int64_t* nodes_types, const float* edge_attr, const void* plan, int64_t n_nodes,
+                    int64_t n_edges, int steps, int flags, int precision, const void* fwd_ws, void* vjp_ws,
+                    size_t vjp_ws_bytes, int n_cotangents, const float* grad_local_stress, float* grad_mean_stress,
+                    float* grad_pos, float* grad_edge_attr, void* stream);
+
 /* ---- loss: per-graph NMSE + divergence regulariser, batch means ---------------------
  * Replaces the per-graph Python loop of train() (gnn_train.py:162-202):
  * normalized_mse_loss_single (:41-57), compute_divergence (:60-92),

@@ -17,6 +17,7 @@ PDG_PARAM_ELEMS = 167299
 FLAG_SCALE_INPUT, FLAG_SCALE_OUTPUT, FLAG_SAVE, FLAG_ZERO_CHECK = 1, 2, 4, 8
 PREC_FP32, PREC_BF16 = 0, 1
 JVP_MAX_TANGENTS = 64  # PDG_JVP_MAX_TANGENTS: tangents of one pdg_jvp_batched call
+VJP_MAX_COTANGENTS = 64  # PDG_VJP_MAX_COTANGENTS: cotangents of one pdg_vjp_batched call
 
 
 class PdgParams(C.Structure):
@@ -67,6 +68,9 @@ _SIGS = {
     "pdg_jvp_batched_ws_bytes": (_sz, [_i64, _i64, _i32, _i32]),
     "pdg_jvp_batched": (_i32, [C.POINTER(PdgParams), C.POINTER(PdgNorm), _vp, _vp, _vp, _vp, _vp, _i64, _i64, _i32, _i32,
                                _i32, _vp, _vp, _sz, _i32, _vp, _i64, _vp, _i64, _vp, _i64, _vp, _vp]),
+    "pdg_vjp_batched_ws_bytes": (_sz, [_i64, _i64, _i32, _i32]),
+    "pdg_vjp_batched": (_i32, [C.POINTER(PdgParams), C.POINTER(PdgNorm), _vp, _vp, _vp, _vp, _vp, _i64, _i64, _i32, _i32,
+                               _i32, _vp, _vp, _sz, _i32, _vp, _vp, _vp, _vp, _vp]),
     "pdg_opdiv_plan_bytes": (_sz, [_i64, _i64]),
     "pdg_opdiv_tmp_bytes": (_sz, [_i64, _i64]),
     "pdg_opdiv_plan_build": (_i32, [_vp, _vp, _i64, _vp, _i64, _i64, _vp, _vp, _sz, _vp]),
@@ -137,16 +141,35 @@ def check(rc: int, what: str):
         raise RuntimeError(f"{what} failed (rc={rc}): {lib().pdg_last_error().decode()}")
 
 
+def _refuse_legacy_batched(t):
+    if torch._C._functorch.is_legacy_batchedtensor(t):
+        raise NotImplementedError("pdivgnn_b200: torch.autograd.grad(..., is_grads_batched=True) is not supported (its "
+                                  "legacy vmap passes tensors without storage); use torch.func.jacrev or "
+                                  "torch.func.vmap over torch.func.vjp, which run all cotangents in one adjoint pass")
+
+
 def raw(t):
     """The plain tensor under functorch wrappers: inside torch.func transforms (torch.func.jvp), tensors created by the
     transformed function are wrappers without storage of their own; the library reads and writes the wrapped one.
-    A vmap BatchedTensor is refused: its storage holds the whole batch while the library would read one tensor."""
+    A vmap BatchedTensor is refused: its storage holds the whole batch while the library would read one tensor.  So is a
+    tensor of the legacy vmap behind torch.autograd.grad(..., is_grads_batched=True), which has no storage at all."""
+    _refuse_legacy_batched(t)
     while torch._C._functorch.is_functorch_wrapped_tensor(t):
         if torch._C._functorch.is_batchedtensor(t):
             raise RuntimeError("pdivgnn_b200: a vmap BatchedTensor reached the library; its storage holds the whole "
                                "batch, so it cannot be passed as one tensor")
         t = torch._C._functorch.get_unwrapped(t)
+        _refuse_legacy_batched(t)
     return t
+
+
+def is_vmapped(t):
+    """True when t carries a torch.func.vmap level (a BatchedTensor under any functorch wrappers)."""
+    while torch._C._functorch.is_functorch_wrapped_tensor(t):
+        if torch._C._functorch.is_batchedtensor(t):
+            return True
+        t = torch._C._functorch.get_unwrapped(t)
+    return False
 
 
 def ptr(t):

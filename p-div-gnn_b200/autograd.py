@@ -2,7 +2,8 @@
 
 Nothing here computes; it validates inputs, builds / caches the device graph plan,
 allocates the workspace from torch's caching allocator (so stream semantics hold) and
-calls ``pdg_forward`` / ``pdg_backward_inputs`` / ``pdg_jvp_batched`` on the current CUDA stream.
+calls ``pdg_forward`` / ``pdg_backward_inputs`` / ``pdg_jvp_batched`` / ``pdg_vjp_batched`` on the current CUDA
+stream.
 """
 from __future__ import annotations
 
@@ -126,11 +127,14 @@ def _params_struct(params):
 
 
 class _EPDFunction(torch.autograd.Function):
-    """pdg_forward, pdg_backward_inputs (reverse mode) and pdg_jvp (forward mode).  Written in setup_context style so
-    that torch.func.jvp accepts it; the forward workspace reaches ctx as a second, non-differentiable output."""
+    """pdg_forward, pdg_backward_inputs (reverse mode), pdg_vjp_batched (vmapped reverse mode) and pdg_jvp (forward
+    mode).  Written in setup_context style so that torch.func.jvp accepts it; the forward workspace reaches ctx as a
+    second, non-differentiable output.  `swapped`: parameters other than the cached param_list were in the module
+    (torch.func.functional_call), so a gradient for them would never reach this Function."""
 
     @staticmethod
-    def forward(model, plan, mean_stress, pos, types, edge_attr, flags, steps, prec, need_grad, need_tan, *params):
+    def forward(model, plan, mean_stress, pos, types, edge_attr, flags, steps, prec, need_grad, need_tan, swapped,
+                *params):
         L = _lib.lib()
         dev = mean_stress.device
         n, e = plan.n_nodes, plan.n_edges
@@ -150,7 +154,7 @@ class _EPDFunction(torch.autograd.Function):
 
     @staticmethod
     def setup_context(ctx, inputs, output):
-        model, plan, mean_stress, pos, types, edge_attr, flags, steps, prec, need_grad, need_tan, *params = inputs
+        model, plan, mean_stress, pos, types, edge_attr, flags, steps, prec, need_grad, need_tan, swapped, *params = inputs
         _, ws = output
         ctx.mark_non_differentiable(ws)
         # no zero gradient is materialised for the workspace output (a memset of the whole saved state per backward);
@@ -162,6 +166,7 @@ class _EPDFunction(torch.autograd.Function):
             ctx.pdg = (model, plan, mean_stress, pos, types, edge_attr, flags | _lib.FLAG_SAVE, steps, prec, params, ws,
                        model._norm_struct())
         ctx.pdg_need_grad = need_grad
+        ctx.pdg_swapped = swapped
 
     @staticmethod
     def jvp(ctx, _model, _plan, t_ms, t_pos, _types, t_ea, *_rest):
@@ -182,6 +187,8 @@ class _EPDFunction(torch.autograd.Function):
 
     @staticmethod
     def backward(ctx, grad_out, _grad_ws):
+        if grad_out is not None and _lib.is_vmapped(grad_out):
+            return _EPDFunction._backward_batched(ctx, grad_out)
         L = _lib.lib()
         if not hasattr(L, "pdg_backward_inputs") or getattr(L.pdg_backward_inputs, "argtypes", None) is None:
             raise RuntimeError("libpdivgnn.so was built without pdg_backward_inputs")
@@ -212,10 +219,75 @@ class _EPDFunction(torch.autograd.Function):
             allreduce_flat_(flat, dp[1], getattr(model, "_pdg_peer", None))
         grads, off = [], 0
         for i, p in enumerate(params):
-            grads.append(flat[off:off + p.numel()].view(p.shape) if need[11 + i] else None)
+            grads.append(flat[off:off + p.numel()].view(p.shape) if need[12 + i] else None)
             off += p.numel()
         ctx.pdg = None
-        return (None, None, g_ms, g_pos, None, g_ea) + (None,) * 5 + tuple(grads)
+        return (None, None, g_ms, g_pos, None, g_ea) + (None,) * 6 + tuple(grads)
+
+    @staticmethod
+    def _backward_batched(ctx, grad_out):
+        """The cotangent carries a vmap level (torch.func.jacrev, torch.func.vmap over torch.func.vjp or torch.func.grad):
+        _EPDAdjoint's vmap rule runs every cotangent of the level in one pdg_vjp_batched pass.  Input gradients only;
+        under data parallelism they stay rank-local.  The forward state is kept: jacrev may call again (chunk_size)."""
+        need = ctx.needs_input_grad
+        prec = ctx.pdg[8]
+        if prec != _lib.PREC_FP32:
+            raise NotImplementedError("pdivgnn_b200: batched reverse-mode derivatives (torch.func.jacrev, vmap over vjp) "
+                                      "need precision='fp32'; the 16-bit mode's input gradients miss its 2e-2 tolerance")
+        if ctx.pdg_swapped or any(need[12:]):
+            raise NotImplementedError("pdivgnn_b200: batched reverse-mode derivatives with respect to the parameters are "
+                                      "not implemented (torch.func.jacrev or vmap over vjp of the parameters); those "
+                                      "with respect to mean_stress, pos and edge_attr are")
+        want = (need[2], need[3], need[5])
+        outs = iter(_EPDAdjoint.apply(ctx.pdg, want, grad_out) if any(want) else ())
+        g_ms, g_pos, g_ea = (next(outs) if w else None for w in want)
+        return (None, None, g_ms, g_pos, None, g_ea) + (None,) * (6 + len(ctx.pdg[9]))
+
+
+class _EPDAdjoint(torch.autograd.Function):
+    """Input gradients for K cotangents of local_stress in one pdg_vjp_batched pass.  `state` is the forward's ctx tuple,
+    `want` the (mean_stress, pos, edge_attr) flags of the gradients to form, `g` the cotangent [N, 3] or [K, N, 3].
+    Returns the wanted gradients in that order, each [K, *input shape] (or the input's shape when g is [N, 3]).  The
+    vmap rule folds the vmapped dimension into K.  There is no backward: second-order derivatives are not implemented."""
+
+    @staticmethod
+    def forward(state, want, g):
+        L = _lib.lib()
+        model, plan, mean_stress, pos, types, edge_attr, flags, steps, prec, params, ws, norm = state
+        dev = mean_stress.device
+        n, e = plan.n_nodes, plan.n_edges
+        k = g.shape[0] if g.dim() == 3 else None
+        g = _lib.require_cuda(g.to(torch.float32), "grad_local_stress", torch.float32).reshape(k or 1, n, 3)
+        with torch.cuda.device(dev):
+            outs = [torch.empty((k or 1,) + s, dtype=torch.float32, device=dev) if w else None
+                    for w, s in zip(want, _tangent_shapes(state))]
+            vws_bytes = L.pdg_vjp_batched_ws_bytes(n, e, steps, k or 1)
+            vws = torch.empty(_bucket(vws_bytes), dtype=torch.uint8, device=dev)
+            ps = _params_struct(params)
+            _lib.check(L.pdg_vjp_batched(C.byref(ps), C.byref(norm), _lib.ptr(mean_stress), _lib.ptr(pos),
+                                         _lib.ptr(types), _lib.ptr(edge_attr), _lib.ptr(plan.buf), n, e, steps, flags,
+                                         prec, _lib.ptr(ws), _lib.ptr(vws), vws_bytes, k or 1, _lib.ptr(g),
+                                         *(_lib.ptr(o) for o in outs), _lib.stream_ptr(dev)), "pdg_vjp_batched")
+        return tuple(o if k is not None else o[0] for o in outs if o is not None)
+
+    @staticmethod
+    def setup_context(ctx, inputs, output):
+        pass
+
+    @staticmethod
+    def vmap(info, in_dims, state, want, g):
+        """Moves the vmapped dimension B of the cotangent to the front and merges it with a K that an inner vmap level
+        already folded in ([B, K, N, 3] -> [B*K, N, 3]: nested vmap flattens).  One pass per at most VJP_MAX_COTANGENTS
+        cotangents."""
+        b = info.batch_size
+        g = g.unsqueeze(0).expand(b, *g.shape) if in_dims[2] is None else g.movedim(in_dims[2], 0)
+        k = g.shape[1] if g.dim() == 4 else None
+        g = g.reshape(b * (k or 1), *g.shape[-2:])
+        cap = _lib.VJP_MAX_COTANGENTS
+        parts = [_EPDAdjoint.apply(state, want, g[i:i + cap]) for i in range(0, g.shape[0], cap)]
+        outs = tuple(p[0] if len(parts) == 1 else torch.cat(p) for p in zip(*parts))
+        outs = tuple(o.reshape(b, k, *o.shape[1:]) if k is not None else o for o in outs)
+        return outs, (0,) * len(outs)
 
 
 def _tangent_shapes(state):
@@ -387,9 +459,21 @@ def epd_forward(model, mesh_graph, scale_output: bool, scale_input: bool, zero_c
             raise NotImplementedError("pdivgnn_b200: forward-mode derivatives need precision='fp32'; in the 16-bit mode "
                                       "per-row derivatives amplify the fp16 rounding beyond its 2e-2 tolerance "
                                       "(DESIGN.md section 5)")
+    # inside torch.func transforms, parameters that torch.func.functional_call swapped in are not the cached list above,
+    # so their gradient would never reach the library (jacrev over them would return zeros): a reverse-mode derivative
+    # with respect to them is refused here, and a batched backward refuses any swapped parameter (a fresh walk only
+    # under a transform)
+    swapped = False
+    if torch._C._functorch.maybe_current_level() is not None:
+        fresh = [q for _, q in model.named_parameters()]
+        swapped = any(q is not p for q, p in zip(fresh, params))
+        if swapped and torch.is_grad_enabled() and any(q is not p and q.requires_grad for q, p in zip(fresh, params)):
+            raise NotImplementedError("pdivgnn_b200: reverse-mode derivatives with respect to parameters swapped in by "
+                                      "torch.func.functional_call are not implemented (torch.func.jacrev, vjp or grad "
+                                      "of the parameters); those with respect to mean_stress, pos and edge_attr are")
     if not (need_grad or need_tan) and (getattr(model, "cuda_graphs", False) or _GRAPHS_ENV) \
             and not torch.cuda.is_current_stream_capturing():
         return _forward_graphed(model, plan, mean_stress, pos, types, edge_attr, flags, model.message_passing_steps, prec,
                                 params)
     return _EPDFunction.apply(model, plan, mean_stress, pos, types, edge_attr, flags, model.message_passing_steps, prec,
-                              need_grad, need_tan, *params)[0]
+                              need_grad, need_tan, swapped, *params)[0]

@@ -67,7 +67,8 @@ static const char* kclass_names[KC_COUNT] = {
     "pack_weights", "node_encoder", "edge_encoder", "node_pre", "edge_step", "node_update", "decoder",
     "decoder_bwd", "node_update_bwd", "edge_step_bwd", "node_pre_bwd", "encoder_bwd", "ln_finalize", "grad_reduce",
     "loss", "loss_bwd",
-    "jvp_node_encoder", "jvp_edge_encoder", "jvp_node_pre", "jvp_edge_step", "jvp_node_update", "jvp_decoder"};
+    "jvp_node_encoder", "jvp_edge_encoder", "jvp_node_pre", "jvp_edge_step", "jvp_node_update", "jvp_decoder",
+    "vjp_decoder", "vjp_node_update", "vjp_edge_step", "vjp_node_pre", "vjp_encoder", "vjp_ln_finalize"};
 }  // namespace pdg
 
 extern "C" long long pdg_launch_count(int reset) {

@@ -47,7 +47,8 @@ enum KClass {
   KC_PACK = 0, KC_NODE_ENC, KC_EDGE_ENC, KC_NODE_PRE, KC_EDGE_STEP, KC_NODE_UPD, KC_DECODER,
   KC_DEC_BWD, KC_NODE_UPD_BWD, KC_EDGE_STEP_BWD, KC_NODE_PRE_BWD, KC_ENC_BWD, KC_LN_FIN, KC_GRAD_REDUCE,
   KC_LOSS, KC_LOSS_BWD,
-  KC_JVP_NODE_ENC, KC_JVP_EDGE_ENC, KC_JVP_NODE_PRE, KC_JVP_EDGE_STEP, KC_JVP_NODE_UPD, KC_JVP_DECODER, KC_COUNT
+  KC_JVP_NODE_ENC, KC_JVP_EDGE_ENC, KC_JVP_NODE_PRE, KC_JVP_EDGE_STEP, KC_JVP_NODE_UPD, KC_JVP_DECODER,
+  KC_VJP_DECODER, KC_VJP_NODE_UPD, KC_VJP_EDGE_STEP, KC_VJP_NODE_PRE, KC_VJP_ENC, KC_VJP_LN_FIN, KC_COUNT
 };
 void timing_begin(int cls, cudaStream_t st);
 void timing_end(cudaStream_t st);
