@@ -15,6 +15,14 @@ void set_error(const char* fmt, ...) {
   vsnprintf(g_err, sizeof(g_err), fmt, ap);
   va_end(ap);
 }
+int set_smem(const void* fn, size_t bytes) {
+  cudaError_t e = cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
+  if (e != cudaSuccess) {
+    set_error("cudaFuncSetAttribute(%zu B smem): %s", bytes, cudaGetErrorString(e));
+    return -2;
+  }
+  return 0;
+}
 int num_sms() {
   static int sms[64] = {0};
   static std::mutex mu;

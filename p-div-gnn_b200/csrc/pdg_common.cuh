@@ -26,6 +26,8 @@ constexpr float LN_EPS = 1e-5f; // torch_geometric.nn.LayerNorm eps
 
 // ---- error reporting ---------------------------------------------------------------
 void set_error(const char* fmt, ...);
+// a kernel's dynamic shared-memory limit (cudaFuncAttributeMaxDynamicSharedMemorySize); -2 with the error set on failure
+int set_smem(const void* fn, size_t bytes);
 int num_sms();
 #define PDG_CUDA_CHECK(expr)                                                          \
   do {                                                                                \
@@ -129,6 +131,13 @@ struct PackOffsets {
 
 // ---- device helpers ----------------------------------------------------------------
 #ifdef __CUDACC__
+
+// tangent or cotangent k's copy of a workspace buffer (or of an output): p + off bytes, off = k * (bytes between
+// consecutive copies); nullptr stays nullptr
+template <class T>
+__device__ __forceinline__ T* copy_at(T* p, size_t off) {
+  return p == nullptr ? p : reinterpret_cast<T*>(reinterpret_cast<uintptr_t>(p) + off);
+}
 
 __device__ __forceinline__ void cp_async16(void* smem, const void* gmem) {
   unsigned s = (unsigned)__cvta_generic_to_shared(smem);

@@ -536,15 +536,6 @@ k_decoder(const float* __restrict__ base, const float* __restrict__ yprev, const
   }
 }
 
-static int set_smem(const void* fn, size_t bytes) {
-  cudaError_t e = cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
-  if (e != cudaSuccess) {
-    set_error("cudaFuncSetAttribute(%zu B smem): %s", bytes, cudaGetErrorString(e));
-    return -2;
-  }
-  return 0;
-}
-
 // All weight packs of one forward in ONE launch: blockIdx.y = job.
 //   kind 0: fp32 transpose  Wt[k][o] = W[o][col0 + k]                     (FFMA tiles, k-major B operand)
 //   kind 1: fp16 pre-swizzled operand image (the exact smem bytes of a tcgen05 K-major B tile; fp16, not bf16: a

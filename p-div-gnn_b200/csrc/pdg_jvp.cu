@@ -38,12 +38,6 @@ constexpr size_t SMEM_JEDGE = (size_t)(3 * TM * LDS + 2 * BKJ * H) * sizeof(floa
 constexpr size_t SMEM_JEDGE_TAN = 2 * sizeof(float) + 4 * sizeof(double);
 static_assert(SMEM_JEDGE + PDG_JVP_MAX_TANGENTS * SMEM_JEDGE_TAN <= 227 * 1024, "edge JVP kernel exceeds shared memory");
 
-// tangent k's copy of a tangent-workspace buffer: p + k * (bytes between consecutive tangent workspaces)
-template <class T>
-__device__ __forceinline__ T* tan_at(T* p, size_t off) {
-  return p == nullptr ? p : reinterpret_cast<T*>(reinterpret_cast<uintptr_t>(p) + off);
-}
-
 // Tangent statistics of one LayerNorm instance: mud and c = r^2 sigmad, from the tangent partials and the primal
 // statistics st (ln_stat_block of the same slot).  CTA-wide; sm: >= 2 floats.
 struct LnTan { float mud, c; };
@@ -128,8 +122,8 @@ k_node_encoder_jvp(const float* __restrict__ mean_stress, const float* __restric
   extern __shared__ __align__(16) float smem[];
   if (tan_ms != nullptr) tan_ms += blockIdx.y * ms_stride;
   if (tan_pos != nullptr) tan_pos += blockIdx.y * pos_stride;
-  yd_out = tan_at(yd_out, blockIdx.y * tws);
-  tparts = tan_at(tparts, blockIdx.y * tws);
+  yd_out = copy_at(yd_out, blockIdx.y * tws);
+  tparts = copy_at(tparts, blockIdx.y * tws);
   float* A = smem;
   float* Ws = A + TM * LDS;
   float* feat = Ws + 2 * BK * H;  // [TM][8] primal features
@@ -214,8 +208,8 @@ k_edge_encoder_jvp(const float* __restrict__ edge_attr, const int32_t* __restric
                    int64_t ea_stride, size_t tws) {
   extern __shared__ __align__(16) float smem[];
   if (tan_ea != nullptr) tan_ea += blockIdx.y * ea_stride;
-  yd_out = tan_at(yd_out, blockIdx.y * tws);
-  tparts = tan_at(tparts, blockIdx.y * tws);
+  yd_out = copy_at(yd_out, blockIdx.y * tws);
+  tparts = copy_at(tparts, blockIdx.y * tws);
   float* A = smem;
   float* Ws = A + TM * LDS;
   float* feat = Ws + 2 * BK * H;  // [TM]
@@ -273,12 +267,12 @@ k_node_pre_jvp(const float* __restrict__ yprev, const double* __restrict__ prev_
   extern __shared__ __align__(16) float smem[];
   {
     const size_t off = blockIdx.y * tws;
-    tprev_parts = tan_at(tprev_parts, off);
-    tbase = tan_at(tbase, off);
-    typrev = tan_at(typrev, off);
-    tx_out = tan_at(tx_out, off);
-    tPa = tan_at(tPa, off);
-    tPb = tan_at(tPb, off);
+    tprev_parts = copy_at(tprev_parts, off);
+    tbase = copy_at(tbase, off);
+    typrev = copy_at(typrev, off);
+    tx_out = copy_at(tx_out, off);
+    tPa = copy_at(tPa, off);
+    tPb = copy_at(tPb, off);
   }
   float* A = smem;
   float* Ws = A + TM * LDS;
@@ -433,9 +427,9 @@ __device__ __forceinline__ void load_ed(const EdgeJvpArgs& a, const LnStat& st, 
   LnTan tt;
   tt.mud = tt2[0];
   tt.c = tt2[1];
-  const float* tbase = tan_at(a.tbase, off);
-  const float* typrev = tan_at(a.typrev, off);
-  float* te_out = tan_at(a.te_out, off);
+  const float* tbase = copy_at(a.tbase, off);
+  const float* typrev = copy_at(a.typrev, off);
+  float* te_out = copy_at(a.te_out, off);
 #pragma unroll
   for (int bt = 0; bt < 4; ++bt) {
     float4 ly[4], ld[4], lx[4];
@@ -478,7 +472,7 @@ __global__ void __launch_bounds__(NT, 1) k_edge_step_jvp(EdgeJvpArgs a) {
   const bool upd = a.ty2_out != nullptr;
   const int k0 = blockIdx.y * a.C, nk = min(a.C, a.K - k0);  // this CTA's tangents: k0 .. k0 + nk - 1
   const LnStat st = ln_stat_block(a.prev_parts, a.count, smf);
-  for (int c = tid >> 5; c < nk; c += NT / 32) ln_tan_warp(tan_at(a.tprev_parts, (k0 + c) * a.tws), a.count, st, ttan + 2 * c);
+  for (int c = tid >> 5; c < nk; c += NT / 32) ln_tan_warp(copy_at(a.tprev_parts, (k0 + c) * a.tws), a.count, st, ttan + 2 * c);
   for (int i = tid; i < 4 * nk; i += NT) tsum[i] = 0.0;
   const float mu1 = ln_stat_block(a.parts1, a.count, smf).mu;  // its barriers publish ttan and tsum
   const float mu2 = upd ? ln_stat_block(a.parts2, a.count, smf).mu : 0.f;
@@ -544,8 +538,8 @@ __global__ void __launch_bounds__(NT, 1) k_edge_step_jvp(EdgeJvpArgs a) {
       acc_store(acc, T2, LDS);
       __syncthreads();  // T2 visible
       // ---- h1d -> T1 ----
-      const float* tPa = tan_at(a.tPa, off);
-      const float* tPb = tan_at(a.tPb, off);
+      const float* tPa = copy_at(a.tPa, off);
+      const float* tPb = copy_at(a.tPb, off);
       gather_hidden_tan(acc, T2, tPa, recv_s, tPb, send_s, m1);
       acc_store(acc, T1, LDS);
       acc_zero(acc);
@@ -556,7 +550,7 @@ __global__ void __launch_bounds__(NT, 1) k_edge_step_jvp(EdgeJvpArgs a) {
         acc_store(acc, T1, LDS);
         __syncthreads();
         float u0 = 0.f, u1 = 0.f;
-        tile_segsum_warp<false>(T1, recv_s, seg_row, nseg, a.rowptr, row0, nvalid, tan_at(a.taggraw, off), u0, u1);
+        tile_segsum_warp<false>(T1, recv_s, seg_row, nseg, a.rowptr, row0, nvalid, copy_at(a.taggraw, off), u0, u1);
         finish_partials(s, cc, red, tsum[4 * c], tsum[4 * c + 1]);  // its barriers also end every read of T1
       }
       // ---- edge-update tangent (skipped on the last step, as in the forward); h2d -> T1, T0 keeps y1 ----
@@ -567,7 +561,7 @@ __global__ void __launch_bounds__(NT, 1) k_edge_step_jvp(EdgeJvpArgs a) {
         gemm_rowA<BKJ>(T1, a.Wt2, H, acc, Ws);
         float s = 0.f, cc = 0.f;
         relu_mask_stats(acc, a.y2_t + (size_t)row0 * H, H, mu2, nvalid, s, cc);
-        acc_store(acc, tan_at(a.ty2_out, off) + (size_t)row0 * H, H);
+        acc_store(acc, copy_at(a.ty2_out, off) + (size_t)row0 * H, H);
         finish_partials(s, cc, red, tsum[4 * c + 2], tsum[4 * c + 3]);
       }
       __syncthreads();
@@ -576,11 +570,11 @@ __global__ void __launch_bounds__(NT, 1) k_edge_step_jvp(EdgeJvpArgs a) {
   if (tid == 0) {
     for (int c = 0; c < nk; ++c) {
       const size_t off = (size_t)(k0 + c) * a.tws;
-      double* p1 = tan_at(a.tparts1, off);
+      double* p1 = copy_at(a.tparts1, off);
       p1[2 * blockIdx.x] = tsum[4 * c];
       p1[2 * blockIdx.x + 1] = tsum[4 * c + 1];
       if (a.tparts2 != nullptr) {
-        double* p2 = tan_at(a.tparts2, off);
+        double* p2 = copy_at(a.tparts2, off);
         p2[2 * blockIdx.x] = tsum[4 * c + 2];
         p2[2 * blockIdx.x + 1] = tsum[4 * c + 3];
       }
@@ -602,11 +596,11 @@ k_node_update_jvp(const float* __restrict__ aggraw, const float* __restrict__ ta
   extern __shared__ __align__(16) float smem[];
   {
     const size_t off = blockIdx.y * tws;
-    taggraw = tan_at(taggraw, off);
-    tparts1 = tan_at(tparts1, off);
-    tx_t = tan_at(tx_t, off);
-    ty3_out = tan_at(ty3_out, off);
-    tparts3 = tan_at(tparts3, off);
+    taggraw = copy_at(taggraw, off);
+    tparts1 = copy_at(tparts1, off);
+    tx_t = copy_at(tx_t, off);
+    ty3_out = copy_at(ty3_out, off);
+    tparts3 = copy_at(tparts3, off);
   }
   float* A0 = smem;
   float* A1 = A0 + TM * LDS;
@@ -683,9 +677,9 @@ k_decoder_jvp(const float* __restrict__ yprev, const double* __restrict__ prev_p
   extern __shared__ __align__(16) float smem[];
   {
     const size_t off = blockIdx.y * tws;
-    tprev_parts = tan_at(tprev_parts, off);
-    tbase = tan_at(tbase, off);
-    typrev = tan_at(typrev, off);
+    tprev_parts = copy_at(tprev_parts, off);
+    tbase = copy_at(tbase, off);
+    typrev = copy_at(typrev, off);
     tout += (size_t)blockIdx.y * N * PDG_OUT;  // [K][N][3]
   }
   float* A = smem;
@@ -729,15 +723,6 @@ k_decoder_jvp(const float* __restrict__ yprev, const double* __restrict__ prev_p
     }
     __syncthreads();
   }
-}
-
-static int set_smem_j(const void* fn, size_t bytes) {
-  cudaError_t e = cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
-  if (e != cudaSuccess) {
-    set_error("cudaFuncSetAttribute(%zu B smem): %s", bytes, cudaGetErrorString(e));
-    return -2;
-  }
-  return 0;
 }
 
 }  // namespace pdg
@@ -795,12 +780,12 @@ extern "C" int pdg_jvp_batched(const pdg_params_t* params, const pdg_norm_t* nor
   groups = (K + C - 1) / C;  // no empty group
   const size_t smem_edge = SMEM_JEDGE + (size_t)C * SMEM_JEDGE_TAN;
   const double cnt_n = (double)N * H, cnt_e = (double)E * H;
-  if (set_smem_j((const void*)k_node_encoder_jvp, SMEM_JENC)) return -2;
-  if (set_smem_j((const void*)k_edge_encoder_jvp, SMEM_JENC)) return -2;
-  if (set_smem_j((const void*)k_node_pre_jvp, SMEM_J1A)) return -2;
-  if (set_smem_j((const void*)k_edge_step_jvp, smem_edge)) return -2;
-  if (set_smem_j((const void*)k_node_update_jvp, SMEM_J2A)) return -2;
-  if (set_smem_j((const void*)k_decoder_jvp, SMEM_J1A)) return -2;
+  if (set_smem((const void*)k_node_encoder_jvp, SMEM_JENC)) return -2;
+  if (set_smem((const void*)k_edge_encoder_jvp, SMEM_JENC)) return -2;
+  if (set_smem((const void*)k_node_pre_jvp, SMEM_J1A)) return -2;
+  if (set_smem((const void*)k_edge_step_jvp, smem_edge)) return -2;
+  if (set_smem((const void*)k_node_update_jvp, SMEM_J2A)) return -2;
+  if (set_smem((const void*)k_decoder_jvp, SMEM_J1A)) return -2;
 
   // tangent partials of all K tangents (one strided memset): slots of CTAs that do not exist must read as zero
   PDG_CUDA_CHECK(cudaMemset2DAsync(J.parts, tws, 0, (size_t)(2 + 3 * T) * MAXP * 2 * sizeof(double), K, st));
