@@ -120,6 +120,23 @@ int pdg_forward(const pdg_params_t* params, const pdg_norm_t* norm, const float*
                 int64_t n_edges, int steps, int flags, int precision, void* ws, size_t ws_bytes,
                 float* local_stress, void* stream);
 
+/* Batched forward: n_instances (1..PDG_FWD_MAX_INSTANCES) instances K of one graph in one pass.  All instances share
+ * the plan, nodes_types, the parameters and the statistics; instance k has its own inputs, its own graph-LayerNorm
+ * statistics and its own output.  Instance k's input x starts at x + k * x_stride (elements; each instance contiguous in
+ * the layout of pdg_forward); stride 0 gives every k the same input.  local_stress [K][N][3].  ws:
+ * pdg_forward_batched_ws_bytes (K forward workspaces of the fp32 mode, one after another); 0 for K or steps out of
+ * range.  Row k has the bits of pdg_forward on instance k's inputs with the same flags; with PDG_FLAG_ZERO_CHECK an
+ * instance whose mean_stress is all zeros gives zeros whatever the others hold.  Launches the kernels and memsets of
+ * one pdg_forward for any K.  Returns -1 for K outside 1..PDG_FWD_MAX_INSTANCES, precision != PDG_PREC_FP32,
+ * PDG_FLAG_SAVE (no derivative follows a batched forward), steps outside 1..62, a negative stride, a workspace that is
+ * too small and an empty graph.  Replaces torch.func.vmap over the inputs of models.py:288-326. */
+#define PDG_FWD_MAX_INSTANCES 64
+size_t pdg_forward_batched_ws_bytes(int64_t n_nodes, int64_t n_edges, int steps, int flags, int n_instances);
+int pdg_forward_batched(const pdg_params_t* params, const pdg_norm_t* norm, const float* mean_stress, int64_t ms_stride,
+                        const float* pos, int64_t pos_stride, const int64_t* nodes_types, const float* edge_attr,
+                        int64_t ea_stride, const void* plan, int64_t n_nodes, int64_t n_edges, int steps, int flags,
+                        int precision, void* ws, size_t ws_bytes, int n_instances, float* local_stress, void* stream);
+
 /* test/debug: byte offset + element count of a saved tensor in a PDG_FLAG_SAVE workspace.
  * what: 0 x_t, 1 e_t, 2 y2_t, 3 Pa_t, 4 Pb_t, 5 aggraw_t, 6 hq_t, 7 y3_t, 8 y_nenc,
  * 9 y_eenc, 10 hd (fp32), 11 LayerNorm partials of slot t (doubles). Edge tensors are in

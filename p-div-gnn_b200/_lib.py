@@ -18,6 +18,7 @@ FLAG_SCALE_INPUT, FLAG_SCALE_OUTPUT, FLAG_SAVE, FLAG_ZERO_CHECK = 1, 2, 4, 8
 PREC_FP32, PREC_BF16 = 0, 1
 JVP_MAX_TANGENTS = 64  # PDG_JVP_MAX_TANGENTS: tangents of one pdg_jvp_batched call
 VJP_MAX_COTANGENTS = 64  # PDG_VJP_MAX_COTANGENTS: cotangents of one pdg_vjp_batched call
+FWD_MAX_INSTANCES = 64  # PDG_FWD_MAX_INSTANCES: instances of one pdg_forward_batched call
 
 
 class PdgParams(C.Structure):
@@ -56,6 +57,9 @@ _SIGS = {
     "pdg_forward_ws_bytes": (_sz, [_i64, _i64, _i32, _i32]),
     "pdg_forward": (_i32, [C.POINTER(PdgParams), C.POINTER(PdgNorm), _vp, _vp, _vp, _vp, _vp, _i64, _i64, _i32, _i32,
                            _i32, _vp, _sz, _vp, _vp]),
+    "pdg_forward_batched_ws_bytes": (_sz, [_i64, _i64, _i32, _i32, _i32]),
+    "pdg_forward_batched": (_i32, [C.POINTER(PdgParams), C.POINTER(PdgNorm), _vp, _i64, _vp, _i64, _vp, _vp, _i64, _vp,
+                                   _i64, _i64, _i32, _i32, _i32, _vp, _sz, _i32, _vp, _vp]),
     "pdg_ws_offset": (_i32, [_i64, _i64, _i32, _i32, _i32, _i32, C.POINTER(_sz), C.POINTER(_sz)]),
     "pdg_backward_ws_bytes": (_sz, [_i64, _i64, _i32]),
     "pdg_backward": (_i32, [C.POINTER(PdgParams), C.POINTER(PdgNorm), _vp, _vp, _vp, _vp, _vp, _i64, _i64, _i32, _i32,

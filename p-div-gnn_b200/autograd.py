@@ -2,8 +2,8 @@
 
 Nothing here computes; it validates inputs, builds / caches the device graph plan,
 allocates the workspace from torch's caching allocator (so stream semantics hold) and
-calls ``pdg_forward`` / ``pdg_backward_inputs`` / ``pdg_jvp_batched`` / ``pdg_vjp_batched`` on the current CUDA
-stream.
+calls ``pdg_forward`` / ``pdg_forward_batched`` / ``pdg_backward_inputs`` / ``pdg_jvp_batched`` / ``pdg_vjp_batched``
+on the current CUDA stream.
 """
 from __future__ import annotations
 
@@ -179,11 +179,30 @@ class _EPDFunction(torch.autograd.Function):
         return t_out, None
 
     @staticmethod
-    def vmap(info, in_dims, *args):
+    def vmap(info, in_dims, model, plan, mean_stress, pos, types, edge_attr, flags, steps, prec, need_grad, need_tan,
+             swapped, *params):
         """torch reaches this rule only when a model input or parameter is batched at this vmap level: with unbatched
-        primals it skips the level, and batched tangents go to _EPDTangent.vmap."""
-        raise NotImplementedError("pdivgnn_b200: vmap over the model's inputs or parameters is not implemented; batched "
-                                  "tangents are (torch.func.jacfwd, torch.func.vmap over torch.func.jvp)")
+        primals it skips the level, and batched tangents go to _EPDTangent.vmap.  Batched mean_stress, pos and
+        edge_attr (one graph under many loads or shapes) run as instances of pdg_forward_batched: the vmapped dimension
+        moves to the front, unbatched inputs are shared (stride 0).  Inference only, fp32 only."""
+        if need_grad or need_tan:
+            raise NotImplementedError(
+                "pdivgnn_b200: vmap over mean_stress, pos or edge_attr runs the forward only (under torch.no_grad(), or "
+                "with a model whose parameters and inputs do not require grad); derivatives through it are not "
+                "implemented.  Derivatives at one input point are: batched tangents (torch.func.jacfwd, vmap over "
+                "torch.func.jvp) and batched cotangents (torch.func.jacrev, vmap over torch.func.vjp)")
+        if prec != _lib.PREC_FP32:
+            raise NotImplementedError("pdivgnn_b200: vmap over the model's inputs needs precision='fp32'; in the 16-bit "
+                                      "mode call the model once per input")
+        if any(d is not None for d in in_dims[12:]):
+            raise NotImplementedError(_BATCHED_PARAMS)
+        if in_dims[4] is not None:
+            raise NotImplementedError("pdivgnn_b200: vmap over nodes_types is not implemented; the instances of one "
+                                      "vmapped forward share the graph and its node types, and differ in mean_stress, "
+                                      "pos and edge_attr")
+        xs = [x if d is None else x.movedim(d, 0) for x, d in zip((mean_stress, pos, edge_attr), (in_dims[2], in_dims[3], in_dims[5]))]
+        out, ws = _EPDInstances.apply((model, plan, types, flags, steps, params), *xs)
+        return (out, ws), (0, None)
 
     @staticmethod
     def backward(ctx, grad_out, _grad_ws):
@@ -293,6 +312,73 @@ class _EPDAdjoint(torch.autograd.Function):
 def _tangent_shapes(state):
     plan = state[1]
     return ((plan.n_nodes, 3), (plan.n_nodes, 2), (plan.n_edges,))
+
+
+_BATCHED_PARAMS = ("pdivgnn_b200: vmap over the model's parameters (model ensembles through torch.func.functional_call) "
+                   "is not implemented; vmap over mean_stress, pos and edge_attr is")
+
+
+class _EPDInstances(torch.autograd.Function):
+    """local_stress of K instances of one graph: pdg_forward_batched, one pass per at most FWD_MAX_INSTANCES instances.
+    `state` is (model, plan, nodes_types, flags, steps, params).  An input is of its per-graph shape (the same for every
+    instance) or [K, *shape], at least one of them the latter; returns local_stress [K, N, 3] and the workspace.  The
+    vmap rule folds the vmapped dimension into K.  Inference only: there is no backward."""
+
+    @staticmethod
+    def forward(state, mean_stress, pos, edge_attr):
+        L = _lib.lib()
+        model, plan, types, flags, steps, params = state
+        dev = types.device
+        n, e = plan.n_nodes, plan.n_edges
+        xs, shapes = (mean_stress, pos, edge_attr), _tangent_shapes(state)
+        k = next(x.shape[0] for x, s in zip(xs, shapes) if x.dim() == len(s) + 1)
+        args = []
+        for x, s, name in zip(xs, shapes, ("mean_stress", "pos", "edge_attr")):
+            stride = 0
+            if x.dim() == len(s) + 1 and x.stride(0) != 0:
+                x, stride = x.contiguous(), x[0].numel()
+            elif x.dim() == len(s) + 1:
+                x = x[0]  # one input expanded over K: passed once, with stride 0
+            args.append((_lib.require_cuda(x, name, torch.float32), stride))
+        cap = _lib.FWD_MAX_INSTANCES
+        with torch.cuda.device(dev):
+            ws_bytes = L.pdg_forward_batched_ws_bytes(n, e, steps, flags, min(k, cap))
+            ws = torch.empty(_bucket(ws_bytes), dtype=torch.uint8, device=dev)  # reused by every pass (stream order)
+            out = torch.empty((k, n, 3), dtype=torch.float32, device=dev)
+            ps, norm = _params_struct(params), model._norm_struct()
+            for i in range(0, k, cap):
+                kk = min(cap, k - i)
+                xp = [_lib.ptr(x[i:i + kk] if st else x) for x, st in args]
+                _lib.check(L.pdg_forward_batched(C.byref(ps), C.byref(norm), xp[0], args[0][1], xp[1], args[1][1],
+                                                 _lib.ptr(types), xp[2], args[2][1], _lib.ptr(plan.buf), n, e, steps,
+                                                 flags, _lib.PREC_FP32, _lib.ptr(ws), ws_bytes, kk, _lib.ptr(out[i:i + kk]),
+                                                 _lib.stream_ptr(dev)), "pdg_forward_batched")
+        return out, ws
+
+    @staticmethod
+    def setup_context(ctx, inputs, output):
+        ctx.mark_non_differentiable(*output)
+
+    @staticmethod
+    def vmap(info, in_dims, state, *xs):
+        """Moves the vmapped dimension B of every batched input to the front and merges it with the K that an inner
+        vmap level folded in ([B, K, ...] -> [B*K, ...]: nested vmap flattens).  Unbatched inputs stay shared."""
+        shapes = _tangent_shapes(state)
+        b = info.batch_size
+        xs = [x if d is None else x.movedim(d, 0) for x, d in zip(xs, in_dims[1:])]
+        k = next(x.shape[1 if d is not None else 0] for x, d, s in zip(xs, in_dims[1:], shapes)
+                 if x.dim() == len(s) + 1 + (d is not None))
+        flat = []
+        for x, d, s in zip(xs, in_dims[1:], shapes):
+            if d is not None or x.dim() == len(s) + 1:
+                if d is None:
+                    x = x.unsqueeze(0)
+                elif x.dim() == len(s) + 1:
+                    x = x.unsqueeze(1)
+                x = x.expand(b, k, *s).reshape(b * k, *s)
+            flat.append(x)
+        out, ws = _EPDInstances.apply(state, *flat)
+        return (out.reshape(b, k, *out.shape[1:]), ws), (0, None)
 
 
 class _EPDTangent(torch.autograd.Function):
@@ -464,14 +550,19 @@ def epd_forward(model, mesh_graph, scale_output: bool, scale_input: bool, zero_c
     # with respect to them is refused here, and a batched backward refuses any swapped parameter (a fresh walk only
     # under a transform)
     swapped = False
-    if torch._C._functorch.maybe_current_level() is not None:
+    transformed = torch._C._functorch.maybe_current_level() is not None
+    if transformed:
         fresh = [q for _, q in model.named_parameters()]
         swapped = any(q is not p for q, p in zip(fresh, params))
+        if swapped and any(_lib.is_vmapped(q) for q in fresh):
+            raise NotImplementedError(_BATCHED_PARAMS)
         if swapped and torch.is_grad_enabled() and any(q is not p and q.requires_grad for q, p in zip(fresh, params)):
             raise NotImplementedError("pdivgnn_b200: reverse-mode derivatives with respect to parameters swapped in by "
                                       "torch.func.functional_call are not implemented (torch.func.jacrev, vjp or grad "
                                       "of the parameters); those with respect to mean_stress, pos and edge_attr are")
-    if not (need_grad or need_tan) and (getattr(model, "cuda_graphs", False) or _GRAPHS_ENV) \
+    # the CUDA-graph replay reads raw pointers: not under a torch.func transform (a vmapped input has no storage of its
+    # own; its forward runs as pdg_forward_batched instances)
+    if not (need_grad or need_tan) and (getattr(model, "cuda_graphs", False) or _GRAPHS_ENV) and not transformed \
             and not torch.cuda.is_current_stream_capturing():
         return _forward_graphed(model, plan, mean_stress, pos, types, edge_attr, flags, model.message_passing_steps, prec,
                                 params)

@@ -45,16 +45,29 @@ __device__ __forceinline__ void bias_relu_stats(float (&acc)[8][8], const float 
   }
 }
 
+// Instances (pdg_forward_batched): every fp32 forward kernel is a template on INST.  With INST, instance k = blockIdx.y
+// over the x-grid of one pdg_forward; its workspace pointers move by k * iws bytes (one forward workspace per instance)
+// and its inputs by k * (element stride).  Without INST (pdg_forward) the offsets and their arguments are not read.
+
 // ------------------------------------------------------------------------------------
 // node encoder: format_node_features (models.py:140-152) + node_encoder MLP (:260-266)
 // writes RAW relu output + LN partials (slot 0)
 // ------------------------------------------------------------------------------------
+template <bool INST>
 __global__ void __launch_bounds__(NT, 1)
 k_node_encoder(const float* __restrict__ mean_stress, const float* __restrict__ pos, const int64_t* __restrict__ types,
                pdg_norm_t nrm, int scale_in, const float* __restrict__ W0, const float* __restrict__ b0,
                const float* __restrict__ Wt2, const float* __restrict__ b2, float* __restrict__ y_out,
-               double* __restrict__ parts, int* __restrict__ nzflag, int N, int n_tiles) {
+               double* __restrict__ parts, int* __restrict__ nzflag, int N, int n_tiles, int64_t ms_stride,
+               int64_t pos_stride, size_t iws) {
   extern __shared__ __align__(16) float smem[];
+  if constexpr (INST) {
+    mean_stress += blockIdx.y * ms_stride;
+    pos += blockIdx.y * pos_stride;
+    y_out = copy_at(y_out, blockIdx.y * iws);
+    parts = copy_at(parts, blockIdx.y * iws);
+    nzflag = copy_at(nzflag, blockIdx.y * iws);
+  }
   float* A = smem;
   float* Ws = A + TM * LDS;
   float* feat = Ws + 2 * BK * H;       // [TM][8]
@@ -127,12 +140,18 @@ k_node_encoder(const float* __restrict__ mean_stress, const float* __restrict__ 
 // edge encoder: format_edge_features (models.py:154-162, :303-307) + edge_encoder MLP
 // (:268-274), edges taken in receiver-sorted order through perm.  RAW output + slot 1.
 // ------------------------------------------------------------------------------------
+template <bool INST>
 __global__ void __launch_bounds__(NT, 1)
 k_edge_encoder(const float* __restrict__ edge_attr, const int32_t* __restrict__ perm, pdg_norm_t nrm, int scale_in,
                const float* __restrict__ W0, const float* __restrict__ b0, const float* __restrict__ Wt2,
                const float* __restrict__ b2, float* __restrict__ y_out, double* __restrict__ parts, int E,
-               int n_tiles) {
+               int n_tiles, int64_t ea_stride, size_t iws) {
   extern __shared__ __align__(16) float smem[];
+  if constexpr (INST) {
+    edge_attr += blockIdx.y * ea_stride;
+    y_out = copy_at(y_out, blockIdx.y * iws);
+    parts = copy_at(parts, blockIdx.y * iws);
+  }
   float* A = smem;
   float* Ws = A + TM * LDS;
   float* feat = Ws + 2 * BK * H;  // [TM]
@@ -182,12 +201,22 @@ k_edge_encoder(const float* __restrict__ edge_attr, const int32_t* __restrict__ 
 // then the node-level halves of edge_net layer 1:  Pa = x_t Wa^T, Pb = x_t Wb^T  with
 // edge_net.0.weight = [Wa | Wb | We]  (x_i | x_j | edge_attr column blocks, :233-238).
 // ------------------------------------------------------------------------------------
+template <bool INST>
 __global__ void __launch_bounds__(NT, 1)
 k_node_pre(const float* __restrict__ base, const float* __restrict__ yprev, const double* __restrict__ prev_parts,
            double prev_count, const float* __restrict__ lnw, const float* __restrict__ lnb, float* __restrict__ x_out,
            const float* __restrict__ WtA, const float* __restrict__ WtB, float* __restrict__ Pa, float* __restrict__ Pb,
-           int n_tiles) {
+           int n_tiles, size_t iws) {
   extern __shared__ __align__(16) float smem[];
+  if constexpr (INST) {
+    const size_t off = blockIdx.y * iws;
+    base = copy_at(base, off);
+    yprev = copy_at(yprev, off);
+    prev_parts = copy_at(prev_parts, off);
+    x_out = copy_at(x_out, off);
+    Pa = copy_at(Pa, off);
+    Pb = copy_at(Pb, off);
+  }
   float* A = smem;
   float* Ws = A + TM * LDS;
   float* smf = Ws + 2 * BK * H;
@@ -276,8 +305,22 @@ __device__ __forceinline__ void gather_hidden(float (&acc)[8][8], const float* _
   }
 }
 
-__global__ void __launch_bounds__(NT, 1) k_edge_step(EdgeStepArgs a) {
+template <bool INST>
+__global__ void __launch_bounds__(NT, 1) k_edge_step(EdgeStepArgs a, size_t iws) {
   extern __shared__ __align__(16) float smem[];
+  if constexpr (INST) {
+    const size_t off = blockIdx.y * iws;
+    a.base = copy_at(a.base, off);
+    a.yprev = copy_at(a.yprev, off);
+    a.prev_parts = copy_at(a.prev_parts, off);
+    a.e_out = copy_at(a.e_out, off);
+    a.Pa = copy_at(a.Pa, off);
+    a.Pb = copy_at(a.Pb, off);
+    a.y2_out = copy_at(a.y2_out, off);
+    a.aggraw = copy_at(a.aggraw, off);
+    a.parts1 = copy_at(a.parts1, off);
+    a.parts2 = copy_at(a.parts2, off);
+  }
   float* A = smem;
   float* Gs = A + TM * LDS;
   float* Ws = Gs + TM * LDS;
@@ -392,13 +435,24 @@ __global__ void __launch_bounds__(NT, 1) k_edge_step(EdgeStepArgs a) {
 //   agg = w_e/(sigma1+eps) * (aggraw - deg*mu1) + deg*b_e      (LN1 pushed through the sum)
 //   y3  = relu(relu([agg, x_t] V1^T + c1) V2^T + c2)           RAW + partials (slot LN3)
 // ------------------------------------------------------------------------------------
+template <bool INST>
 __global__ void __launch_bounds__(NT, 1)
 k_node_update(const float* __restrict__ aggraw, const int32_t* __restrict__ rowptr, const double* __restrict__ parts1,
               double count1, const float* __restrict__ lnw_e, const float* __restrict__ lnb_e,
               const float* __restrict__ x_t, const float* __restrict__ WtA, const float* __restrict__ WtX,
               const float* __restrict__ c1, const float* __restrict__ Wt2, const float* __restrict__ c2,
-              float* __restrict__ hq_out, float* __restrict__ y3_out, double* __restrict__ parts3, int N, int n_tiles) {
+              float* __restrict__ hq_out, float* __restrict__ y3_out, double* __restrict__ parts3, int N, int n_tiles,
+              size_t iws) {
   extern __shared__ __align__(16) float smem[];
+  if constexpr (INST) {
+    const size_t off = blockIdx.y * iws;
+    aggraw = copy_at(aggraw, off);
+    parts1 = copy_at(parts1, off);
+    x_t = copy_at(x_t, off);
+    hq_out = copy_at(hq_out, off);
+    y3_out = copy_at(y3_out, off);
+    parts3 = copy_at(parts3, off);
+  }
   float* A0 = smem;
   float* A1 = A0 + TM * LDS;
   float* Ws = A1 + TM * LDS;
@@ -472,13 +526,24 @@ k_node_update(const float* __restrict__ aggraw, const int32_t* __restrict__ rowp
 // ------------------------------------------------------------------------------------
 // decoder: x_T = x_{T-1} + LN(y3_{T-1}); node_decoder (models.py:282-286, :316-321)
 // ------------------------------------------------------------------------------------
+template <bool INST>
 __global__ void __launch_bounds__(NT, 1)
 k_decoder(const float* __restrict__ base, const float* __restrict__ yprev, const double* __restrict__ prev_parts,
           double prev_count, const float* __restrict__ lnw, const float* __restrict__ lnb, float* __restrict__ x_out,
           const float* __restrict__ WtD, const float* __restrict__ d1, const float* __restrict__ D2,
           const float* __restrict__ d2, float* __restrict__ hd_out, float out_scale, float out_shift,
-          float* __restrict__ out, const int* __restrict__ nzflag, int N, int n_tiles) {
+          float* __restrict__ out, const int* __restrict__ nzflag, int N, int n_tiles, size_t iws) {
   extern __shared__ __align__(16) float smem[];
+  if constexpr (INST) {
+    const size_t off = blockIdx.y * iws;
+    base = copy_at(base, off);
+    yprev = copy_at(yprev, off);
+    prev_parts = copy_at(prev_parts, off);
+    x_out = copy_at(x_out, off);
+    hd_out = copy_at(hd_out, off);
+    nzflag = copy_at(nzflag, off);
+    out += (size_t)blockIdx.y * N * PDG_OUT;  // local_stress [K][N][3]
+  }
   float* A = smem;
   float* Ws = A + TM * LDS;
   float* smf = Ws + 2 * BK * H;
@@ -594,6 +659,128 @@ int pack_weights(const pdg_params_t* P, float* pack, uint8_t* img, bool images, 
   return 0;
 }
 
+// Zeroes `bytes` at p in each of K instance workspaces, iws bytes apart: one memset for any K (a plain one for K = 1).
+static cudaError_t memset_instances(void* p, size_t iws, size_t bytes, int K, cudaStream_t st) {
+  return K == 1 ? cudaMemsetAsync(p, 0, bytes, st) : cudaMemset2DAsync(p, iws, 0, bytes, K, st);
+}
+
+// The fp32 (FFMA) forward of K instances of one graph.  Instance k's workspace is W moved by k * W.total bytes, its
+// inputs start k * (element stride) after the given pointers, its output at local_stress + k * N * 3.  The weights are
+// packed once, into instance 0's workspace, and every instance reads them there.  pdg_forward is K = 1 with INST off.
+template <bool INST>
+int forward_ffma(const pdg_params_t* params, const pdg_norm_t* norm, const float* mean_stress, int64_t ms_stride,
+                 const float* pos, int64_t pos_stride, const int64_t* nodes_types, const float* edge_attr,
+                 int64_t ea_stride, const void* plan, const FwdWs& W, int flags, int K, float* local_stress,
+                 cudaStream_t st) {
+  const size_t iws = W.total;
+  const bool save = W.save;
+  const int N = (int)W.N, E = (int)W.E, T = W.T;
+  int32_t *perm, *recv, *send, *rowptr;
+  pdg_plan_views(const_cast<void*>(plan), W.N, W.E, &perm, &recv, &send, &rowptr, nullptr, nullptr);
+  const int nt_n = (int)(W.N_pad / TM), nt_e = (int)(W.E_pad / TM);
+  int sms = num_sms();
+  if (sms > MAXP) sms = MAXP;  // LayerNorm partials are kept per CTA in slots of MAXP entries (as in pdg_backward)
+  const int grid_n = balanced_grid(nt_n, sms), grid_e = balanced_grid(nt_e, sms);
+  const dim3 gn(grid_n, K), ge(grid_e, K);
+  const double cnt_n = (double)N * H, cnt_e = (double)E * H;
+  const size_t smem_enc = SMEM_1A + TM * 8 * sizeof(float);
+  if (set_smem((const void*)k_node_encoder<INST>, smem_enc)) return -2;
+  if (set_smem((const void*)k_edge_encoder<INST>, smem_enc)) return -2;
+  if (set_smem((const void*)k_node_pre<INST>, SMEM_1A)) return -2;
+  if (set_smem((const void*)k_edge_step<INST>, SMEM_EDGE)) return -2;
+  if (set_smem((const void*)k_node_update<INST>, SMEM_2A)) return -2;
+  if (set_smem((const void*)k_decoder<INST>, SMEM_1A)) return -2;
+
+  // LayerNorm partials + the non-zero-load flag (contiguous) in one memset
+  PDG_CUDA_CHECK(memset_instances(W.parts, iws, (size_t)((char*)W.nzflag - (char*)W.parts) + 256, K, st));
+  int* nzflag = (flags & PDG_FLAG_ZERO_CHECK) ? W.nzflag : nullptr;
+  {
+    ScopedTimer tm_(KC_PACK, st);
+    if (pack_weights(params, W.pack, W.img, false, st)) return -2;
+  }
+  const float* const* P = params->p;
+  const float* pk = W.pack;
+  const int scale_in = (flags & PDG_FLAG_SCALE_INPUT) ? 1 : 0;
+
+  {
+    ScopedTimer tm_(KC_NODE_ENC, st);
+    PDG_CUDA_CHECK(launch_pdl(k_node_encoder<INST>, gn, dim3(NT), smem_enc, st, mean_stress, pos, nodes_types, *norm, scale_in,
+                              P[NE_W0], P[NE_B0], pk + PackOffsets::NE_W2T, P[NE_B2], W.y_nenc, W.parts_slot(0), nzflag, N,
+                              nt_n, ms_stride, pos_stride, iws));
+  }
+  PDG_LAUNCH_CHECK();
+  {
+    ScopedTimer tm_(KC_EDGE_ENC, st);
+    k_edge_encoder<INST><<<ge, NT, smem_enc, st>>>(edge_attr, perm, *norm, scale_in, P[EE_W0], P[EE_B0],
+                                                   pk + PackOffsets::EE_W2T, P[EE_B2], W.y_eenc, W.parts_slot(1), E, nt_e,
+                                                   ea_stride, iws);
+  }
+  PDG_LAUNCH_CHECK();
+  for (int t = 0; t < T; ++t) {
+    const bool first = t == 0, last = t == T - 1;
+    // K1
+    {
+      ScopedTimer tm_(KC_NODE_PRE, st);
+      k_node_pre<INST><<<gn, NT, SMEM_1A, st>>>(first ? nullptr : W.x_[t - 1], first ? W.y_nenc : W.y3_[t - 1],
+                                                W.parts_slot(first ? 0 : slot_ln3(t - 1)), cnt_n,
+                                                first ? P[NE_LNW] : P[PN_LNW], first ? P[NE_LNB] : P[PN_LNB], W.x_[t],
+                                                pk + PackOffsets::PE_WAT, pk + PackOffsets::PE_WBT, W.Pa_[t], W.Pb_[t], nt_n,
+                                                iws);
+    }
+    PDG_LAUNCH_CHECK();
+    // K2
+    PDG_CUDA_CHECK(memset_instances(W.aggraw_[t], iws, (size_t)W.N_pad * H * sizeof(float), K, st));
+    EdgeStepArgs a;
+    a.base = first ? nullptr : W.e_[t - 1];
+    a.yprev = first ? W.y_eenc : W.y2_[t - 1];
+    a.prev_parts = W.parts_slot(first ? 1 : slot_ln2(t - 1));
+    a.prev_count = cnt_e;
+    a.prev_w = first ? P[EE_LNW] : P[PE_LNW];
+    a.prev_b = first ? P[EE_LNB] : P[PE_LNB];
+    a.e_out = (save || !last) ? W.e_[t] : nullptr;
+    a.e_img = nullptr;
+    a.Pa = W.Pa_[t];
+    a.Pb = W.Pb_[t];
+    a.recv = recv;
+    a.send = send;
+    a.rowptr = rowptr;
+    a.WtE = pk + PackOffsets::PE_WET;
+    a.b1 = P[PE_B0];
+    a.Wt2 = pk + PackOffsets::PE_W2T;
+    a.b2 = P[PE_B2];
+    a.y2_out = last ? nullptr : W.y2_[t];
+    a.aggraw = W.aggraw_[t];
+    a.parts1 = W.parts_slot(slot_ln1(t));
+    a.parts2 = last ? nullptr : W.parts_slot(slot_ln2(t));
+    a.E = E;
+    a.n_tiles = nt_e;
+    {
+      ScopedTimer tm_(KC_EDGE_STEP, st);
+      k_edge_step<INST><<<ge, NT, SMEM_EDGE, st>>>(a, iws);
+    }
+    PDG_LAUNCH_CHECK();
+    // K3
+    {
+      ScopedTimer tm_(KC_NODE_UPD, st);
+      k_node_update<INST><<<gn, NT, SMEM_2A, st>>>(W.aggraw_[t], rowptr, W.parts_slot(slot_ln1(t)), cnt_e, P[PE_LNW],
+                                                   P[PE_LNB], W.x_[t], pk + PackOffsets::PN_WAT, pk + PackOffsets::PN_WXT,
+                                                   P[PN_B0], pk + PackOffsets::PN_W2T, P[PN_B2], save ? W.hq_[t] : nullptr,
+                                                   W.y3_[t], W.parts_slot(slot_ln3(t)), N, nt_n, iws);
+    }
+    PDG_LAUNCH_CHECK();
+  }
+  const bool scale_out = (flags & PDG_FLAG_SCALE_OUTPUT) != 0;
+  {
+    ScopedTimer tm_(KC_DECODER, st);
+    PDG_CUDA_CHECK(launch_pdl(k_decoder<INST>, gn, dim3(NT), SMEM_1A, st, W.x_[T - 1], W.y3_[T - 1], W.parts_slot(slot_ln3(T - 1)),
+                              cnt_n, P[PN_LNW], P[PN_LNB], save ? W.x_[T] : nullptr, pk + PackOffsets::ND_W0T, P[ND_B0], P[ND_W2],
+                              P[ND_B2], save ? W.hd : nullptr, scale_out ? norm->std_local_stress : 1.f,
+                              scale_out ? norm->mean_local_stress : 0.f, local_stress, nzflag, N, nt_n, iws));
+  }
+  PDG_LAUNCH_CHECK();
+  return 0;
+}
+
 }  // namespace pdg
 
 using namespace pdg;
@@ -617,6 +804,9 @@ extern "C" int pdg_forward(const pdg_params_t* params, const pdg_norm_t* norm, c
   const bool save = (flags & PDG_FLAG_SAVE) != 0;
   FwdWs W(n_nodes, n_edges, steps, save, ws, tcm);
   if (ws_bytes < W.total) { set_error("pdg_forward: workspace %zu < %zu", ws_bytes, W.total); return -1; }
+  if (!tcm) return forward_ffma<false>(params, norm, mean_stress, 0, pos, 0, nodes_types, edge_attr, 0, plan, W, flags, 1,
+                                       local_stress, st);
+  // 16-bit mode: tcgen05 tile kernels (pdg_tc_*.cu)
   const int N = (int)n_nodes, E = (int)n_edges, T = steps;
   int32_t *perm, *recv, *send, *rowptr;
   pdg_plan_views(const_cast<void*>(plan), n_nodes, n_edges, &perm, &recv, &send, &rowptr, nullptr, nullptr);
@@ -625,13 +815,6 @@ extern "C" int pdg_forward(const pdg_params_t* params, const pdg_norm_t* norm, c
   if (sms > MAXP) sms = MAXP;  // LayerNorm partials are kept per CTA in slots of MAXP entries (as in pdg_backward)
   const int grid_n = balanced_grid(nt_n, sms), grid_e = balanced_grid(nt_e, sms);
   const double cnt_n = (double)N * H, cnt_e = (double)E * H;
-  const size_t smem_enc = SMEM_1A + TM * 8 * sizeof(float);
-  if (set_smem((const void*)k_node_encoder, smem_enc)) return -2;
-  if (set_smem((const void*)k_edge_encoder, smem_enc)) return -2;
-  if (set_smem((const void*)k_node_pre, SMEM_1A)) return -2;
-  if (set_smem((const void*)k_edge_step, SMEM_EDGE)) return -2;
-  if (set_smem((const void*)k_node_update, SMEM_2A)) return -2;
-  if (set_smem((const void*)k_decoder, SMEM_1A)) return -2;
 
   // LayerNorm partials + the non-zero-load flag (contiguous) in one memset
   PDG_CUDA_CHECK(cudaMemsetAsync(W.parts, 0, (size_t)((char*)W.nzflag - (char*)W.parts) + 256, st));
@@ -641,29 +824,18 @@ extern "C" int pdg_forward(const pdg_params_t* params, const pdg_norm_t* norm, c
     if (pack_weights(params, W.pack, W.img, tcm, st)) return -2;
   }
   const float* const* P = params->p;
-  const float* pk = W.pack;
   const int scale_in = (flags & PDG_FLAG_SCALE_INPUT) ? 1 : 0;
 
   {
     ScopedTimer tm_(KC_NODE_ENC, st);
-    if (tcm) {
-      if (launch_node_encoder_tc(mean_stress, pos, nodes_types, norm, scale_in, P[NE_W0], P[NE_B0], P[NE_B2], W.y_nenc,
-                                 W.parts_slot(0), nzflag, N, nt_n, grid_n, W.img, st)) return -2;
-    } else {
-      PDG_CUDA_CHECK(launch_pdl(k_node_encoder, dim3(grid_n), dim3(NT), smem_enc, st, mean_stress, pos, nodes_types, *norm, scale_in,
-                                P[NE_W0], P[NE_B0], pk + PackOffsets::NE_W2T, P[NE_B2], W.y_nenc, W.parts_slot(0), nzflag, N, nt_n));
-    }
+    if (launch_node_encoder_tc(mean_stress, pos, nodes_types, norm, scale_in, P[NE_W0], P[NE_B0], P[NE_B2], W.y_nenc,
+                               W.parts_slot(0), nzflag, N, nt_n, grid_n, W.img, st)) return -2;
   }
   PDG_LAUNCH_CHECK();
   {
     ScopedTimer tm_(KC_EDGE_ENC, st);
-    if (tcm) {
-      if (launch_edge_encoder_tc(edge_attr, perm, norm, scale_in, P[EE_W0], P[EE_B0], P[EE_B2], W.y_eenc, W.parts_slot(1), E,
-                                 nt_e, W.img, st)) return -2;
-    } else {
-      k_edge_encoder<<<grid_e, NT, smem_enc, st>>>(edge_attr, perm, *norm, scale_in, P[EE_W0], P[EE_B0],
-                                                   pk + PackOffsets::EE_W2T, P[EE_B2], W.y_eenc, W.parts_slot(1), E, nt_e);
-    }
+    if (launch_edge_encoder_tc(edge_attr, perm, norm, scale_in, P[EE_W0], P[EE_B0], P[EE_B2], W.y_eenc, W.parts_slot(1), E,
+                               nt_e, W.img, st)) return -2;
   }
   PDG_LAUNCH_CHECK();
   for (int t = 0; t < T; ++t) {
@@ -671,26 +843,18 @@ extern "C" int pdg_forward(const pdg_params_t* params, const pdg_norm_t* norm, c
     // K1
     {
       ScopedTimer tm_(KC_NODE_PRE, st);
-      if (tcm) {
-        NodePreArgs np;
-        np.base = first ? nullptr : W.x_[t - 1]; np.yprev = first ? W.y_nenc : W.y3_[t - 1];
-        np.prev_parts = W.parts_slot(first ? 0 : slot_ln3(t - 1)); np.prev_count = cnt_n;
-        np.lnw = first ? P[NE_LNW] : P[PN_LNW]; np.lnb = first ? P[NE_LNB] : P[PN_LNB];
-        np.x_out = W.x_[t]; np.Pa = W.Pa_[t]; np.Pb = W.Pb_[t]; np.n_tiles = nt_n;
-        np.aggraw_zero = W.aggraw_[t];  // zeroed here instead of a memset between the kernels (keeps the PDL chain)
-        np.b1 = P[PE_B0];
-        np.x_img = W.ximg(t);
-        if (launch_node_pre_tc(np, W.img, nt_n, st)) return -2;
-      } else {
-        k_node_pre<<<grid_n, NT, SMEM_1A, st>>>(first ? nullptr : W.x_[t - 1], first ? W.y_nenc : W.y3_[t - 1],
-                                                W.parts_slot(first ? 0 : slot_ln3(t - 1)), cnt_n,
-                                                first ? P[NE_LNW] : P[PN_LNW], first ? P[NE_LNB] : P[PN_LNB], W.x_[t],
-                                                pk + PackOffsets::PE_WAT, pk + PackOffsets::PE_WBT, W.Pa_[t], W.Pb_[t], nt_n);
-      }
+      NodePreArgs np;
+      np.base = first ? nullptr : W.x_[t - 1]; np.yprev = first ? W.y_nenc : W.y3_[t - 1];
+      np.prev_parts = W.parts_slot(first ? 0 : slot_ln3(t - 1)); np.prev_count = cnt_n;
+      np.lnw = first ? P[NE_LNW] : P[PN_LNW]; np.lnb = first ? P[NE_LNB] : P[PN_LNB];
+      np.x_out = W.x_[t]; np.Pa = W.Pa_[t]; np.Pb = W.Pb_[t]; np.n_tiles = nt_n;
+      np.aggraw_zero = W.aggraw_[t];  // zeroed here instead of a memset between the kernels (keeps the PDL chain)
+      np.b1 = P[PE_B0];
+      np.x_img = W.ximg(t);
+      if (launch_node_pre_tc(np, W.img, nt_n, st)) return -2;
     }
     PDG_LAUNCH_CHECK();
     // K2
-    if (!tcm) PDG_CUDA_CHECK(cudaMemsetAsync(W.aggraw_[t], 0, (size_t)W.N_pad * H * sizeof(float), st));
     EdgeStepArgs a;
     a.base = first ? nullptr : W.e_[t - 1];
     a.yprev = first ? W.y_eenc : W.y2_[t - 1];
@@ -698,16 +862,16 @@ extern "C" int pdg_forward(const pdg_params_t* params, const pdg_norm_t* norm, c
     a.prev_count = cnt_e;
     a.prev_w = first ? P[EE_LNW] : P[PE_LNW];
     a.prev_b = first ? P[EE_LNB] : P[PE_LNB];
-    a.e_out = ((save && !tcm) || !last) ? W.e_[t] : nullptr;  // tcgen05 path: the backward reads the bf16 image instead
-    a.e_img = tcm && save ? W.eimg_[t] : nullptr;
+    a.e_out = !last ? W.e_[t] : nullptr;  // the backward reads the fp16 image instead
+    a.e_img = save ? W.eimg_[t] : nullptr;
     a.Pa = W.Pa_[t];
     a.Pb = W.Pb_[t];
     a.recv = recv;
     a.send = send;
     a.rowptr = rowptr;
-    a.WtE = pk + PackOffsets::PE_WET;
+    a.WtE = W.pack + PackOffsets::PE_WET;
     a.b1 = P[PE_B0];
-    a.Wt2 = pk + PackOffsets::PE_W2T;
+    a.Wt2 = W.pack + PackOffsets::PE_W2T;
     a.b2 = P[PE_B2];
     a.y2_out = last ? nullptr : W.y2_[t];
     a.aggraw = W.aggraw_[t];
@@ -717,50 +881,74 @@ extern "C" int pdg_forward(const pdg_params_t* params, const pdg_norm_t* norm, c
     a.n_tiles = nt_e;
     {
       ScopedTimer tm_(KC_EDGE_STEP, st);
-      if (tcm) {
-        if (launch_edge_step_tc(a, W.img, grid_e, st)) return -2;
-      } else {
-        k_edge_step<<<grid_e, NT, SMEM_EDGE, st>>>(a);
-      }
+      if (launch_edge_step_tc(a, W.img, grid_e, st)) return -2;
     }
     PDG_LAUNCH_CHECK();
     // K3
     {
       ScopedTimer tm_(KC_NODE_UPD, st);
-      if (tcm) {
-        NodeUpdArgs nu;
-        nu.aggraw = W.aggraw_[t]; nu.rowptr = rowptr; nu.parts1 = W.parts_slot(slot_ln1(t)); nu.count1 = cnt_e;
-        nu.lnw_e = P[PE_LNW]; nu.lnb_e = P[PE_LNB]; nu.x_t = W.x_[t]; nu.c1 = P[PN_B0]; nu.c2 = P[PN_B2];
-        nu.hq_out = save ? W.hq_[t] : nullptr; nu.y3_out = W.y3_[t]; nu.parts3 = W.parts_slot(slot_ln3(t));
-        nu.N = N; nu.n_tiles = nt_n;
-        nu.x_img = W.ximg(t); nu.hq_img = save ? W.hqimg(t) : nullptr; nu.agg_img = save ? W.aggimg(t) : nullptr;
-        if (launch_node_update_tc(nu, W.img, grid_n, st)) return -2;
-      } else {
-        k_node_update<<<grid_n, NT, SMEM_2A, st>>>(W.aggraw_[t], rowptr, W.parts_slot(slot_ln1(t)), cnt_e, P[PE_LNW],
-                                                   P[PE_LNB], W.x_[t], pk + PackOffsets::PN_WAT, pk + PackOffsets::PN_WXT,
-                                                   P[PN_B0], pk + PackOffsets::PN_W2T, P[PN_B2], save ? W.hq_[t] : nullptr,
-                                                   W.y3_[t], W.parts_slot(slot_ln3(t)), N, nt_n);
-      }
+      NodeUpdArgs nu;
+      nu.aggraw = W.aggraw_[t]; nu.rowptr = rowptr; nu.parts1 = W.parts_slot(slot_ln1(t)); nu.count1 = cnt_e;
+      nu.lnw_e = P[PE_LNW]; nu.lnb_e = P[PE_LNB]; nu.x_t = W.x_[t]; nu.c1 = P[PN_B0]; nu.c2 = P[PN_B2];
+      nu.hq_out = save ? W.hq_[t] : nullptr; nu.y3_out = W.y3_[t]; nu.parts3 = W.parts_slot(slot_ln3(t));
+      nu.N = N; nu.n_tiles = nt_n;
+      nu.x_img = W.ximg(t); nu.hq_img = save ? W.hqimg(t) : nullptr; nu.agg_img = save ? W.aggimg(t) : nullptr;
+      if (launch_node_update_tc(nu, W.img, grid_n, st)) return -2;
     }
     PDG_LAUNCH_CHECK();
   }
   const bool scale_out = (flags & PDG_FLAG_SCALE_OUTPUT) != 0;
   {
     ScopedTimer tm_(KC_DECODER, st);
-    if (tcm) {
-      if (launch_decoder_tc(W.x_[T - 1], W.y3_[T - 1], W.parts_slot(slot_ln3(T - 1)), cnt_n, P[PN_LNW], P[PN_LNB],
-                            save ? W.x_[T] : nullptr, P[ND_B0], P[ND_W2], P[ND_B2], save ? W.hd : nullptr,
-                            scale_out ? norm->std_local_stress : 1.f, scale_out ? norm->mean_local_stress : 0.f, local_stress,
-                            nzflag, N, nt_n, grid_n, W.img, st)) return -2;
-    } else {
-      PDG_CUDA_CHECK(launch_pdl(k_decoder, dim3(grid_n), dim3(NT), SMEM_1A, st, W.x_[T - 1], W.y3_[T - 1], W.parts_slot(slot_ln3(T - 1)),
-                                cnt_n, P[PN_LNW], P[PN_LNB], save ? W.x_[T] : nullptr, pk + PackOffsets::ND_W0T, P[ND_B0], P[ND_W2],
-                                P[ND_B2], save ? W.hd : nullptr, scale_out ? norm->std_local_stress : 1.f,
-                                scale_out ? norm->mean_local_stress : 0.f, local_stress, nzflag, N, nt_n));
-    }
+    if (launch_decoder_tc(W.x_[T - 1], W.y3_[T - 1], W.parts_slot(slot_ln3(T - 1)), cnt_n, P[PN_LNW], P[PN_LNB],
+                          save ? W.x_[T] : nullptr, P[ND_B0], P[ND_W2], P[ND_B2], save ? W.hd : nullptr,
+                          scale_out ? norm->std_local_stress : 1.f, scale_out ? norm->mean_local_stress : 0.f, local_stress,
+                          nzflag, N, nt_n, grid_n, W.img, st)) return -2;
   }
   PDG_LAUNCH_CHECK();
   return 0;
+}
+
+// K instances of one graph: the workspace holds K fp32 forward workspaces without saved state, one after another
+// (each total is a multiple of 256 bytes, so every instance stays aligned).
+extern "C" size_t pdg_forward_batched_ws_bytes(int64_t n_nodes, int64_t n_edges, int steps, int flags, int n_instances) {
+  if (n_instances < 1 || n_instances > PDG_FWD_MAX_INSTANCES || steps < 1 || steps > 62) return 0;
+  return (size_t)n_instances * FwdWs(n_nodes, n_edges, steps, (flags & PDG_FLAG_SAVE) != 0, nullptr, false).total;
+}
+
+extern "C" int pdg_forward_batched(const pdg_params_t* params, const pdg_norm_t* norm, const float* mean_stress,
+                                   int64_t ms_stride, const float* pos, int64_t pos_stride, const int64_t* nodes_types,
+                                   const float* edge_attr, int64_t ea_stride, const void* plan, int64_t n_nodes,
+                                   int64_t n_edges, int steps, int flags, int precision, void* ws, size_t ws_bytes,
+                                   int n_instances, float* local_stress, void* stream_) {
+  const int K = n_instances;
+  if (K < 1 || K > PDG_FWD_MAX_INSTANCES) {
+    set_error("pdg_forward_batched: n_instances=%d outside 1..%d", K, PDG_FWD_MAX_INSTANCES);
+    return -1;
+  }
+  if (precision != PDG_PREC_FP32) {
+    set_error("pdg_forward_batched: only the fp32 mode (PDG_PREC_FP32) runs instances; the 16-bit mode's kernels are "
+              "persistent, one CTA per SM");
+    return -1;
+  }
+  if (flags & PDG_FLAG_SAVE) {
+    set_error("pdg_forward_batched: PDG_FLAG_SAVE is not supported (the batched forward keeps no state for a backward)");
+    return -1;
+  }
+  if (steps < 1 || steps > 62) { set_error("pdg_forward_batched: steps=%d unsupported", steps); return -1; }
+  if (ms_stride < 0 || pos_stride < 0 || ea_stride < 0) {
+    set_error("pdg_forward_batched: negative input stride (mean_stress %lld, pos %lld, edge_attr %lld)",
+              (long long)ms_stride, (long long)pos_stride, (long long)ea_stride);
+    return -1;
+  }
+  if (n_nodes <= 0 || n_edges <= 0) { set_error("pdg_forward_batched: empty graph"); return -1; }
+  const FwdWs W(n_nodes, n_edges, steps, false, ws, false);
+  if (ws_bytes < (size_t)K * W.total) {
+    set_error("pdg_forward_batched: workspace %zu < %zu", ws_bytes, (size_t)K * W.total);
+    return -1;
+  }
+  return forward_ffma<true>(params, norm, mean_stress, ms_stride, pos, pos_stride, nodes_types, edge_attr, ea_stride,
+                            plan, W, flags, K, local_stress, (cudaStream_t)stream_);
 }
 
 // Test/debug helper: byte offset and element count of a saved tensor inside a forward
