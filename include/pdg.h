@@ -219,13 +219,15 @@ int pdg_vjp_batched(const pdg_params_t* params, const pdg_norm_t* norm, const fl
  * data_utils.standardize (:46-51).
  *   pred [N,3] standardised prediction; local_stress [N,3] raw ground truth
  *   (standardised inside with norm->mean/std_local_stress); graph_ptr [B+1] int64;
- *   labels [N] int64 (NodeType); op_div given as a plan (below) over batch rows with
+ *   labels [N] int64 (NodeType; rows labelled 1 or -1 get a zero divergence, every other
+ *   label is kept); op_div given as a plan (below) over batch rows with
  *   graph-LOCAL columns in [0, 2*N_i) exactly as PyG collation leaves them (SURVEY 2.3d).
  *   out[0] = sum_i NMSE_i / B ; out[1] = penalty * sum_i div_i / B   (device floats) */
 /* op_div plan: CSR (by batch row) + CSC (by stacked-stress row 2*n0_i + j) of the
  * row-stacked operator, from the coalesced COO triplets torch holds
  * (datasets.py:191-213 + SURVEY 2.3d).  coo_row/coo_col int64 [nnz], values stay in the
- * caller's buffer and are indexed by the plan. */
+ * caller's buffer and are indexed by the plan.  nnz = 0 is an empty operator: a divergence
+ * of exactly 0 (op_val may then be NULL). */
 size_t pdg_opdiv_plan_bytes(int64_t n_nodes, int64_t nnz);
 size_t pdg_opdiv_tmp_bytes(int64_t n_nodes, int64_t nnz);
 int pdg_opdiv_plan_build(const int64_t* coo_row, const int64_t* coo_col, int64_t nnz, const int64_t* graph_ptr,

@@ -455,6 +455,72 @@ def compute_divergence_spmm(local_stress, row, col, val, labels):
     return torch.sum(torch.mean(torch.square(div), dim=0))
 
 
+def opdiv_entries(op_div_matrix, ptr):
+    """The entries of a row-stacked batch operator that ``compute_divergence`` keeps, with the stacked-stress value
+    each one multiplies.  The batch operator is coalesced first (fp32 sums of duplicates, as torch and the device
+    path do); entry k of graph i multiplies S[col_k] of that graph, S[j] = (sxx, sxy)[j] for j < N_i and
+    (sxy, syy)[j - N_i] below (gnn_train.py:68-70); columns outside [0, 2 N_i) are sliced away (:73-76).
+    Returns (row, node, first, val): batch row, batch node of S[col], True where S[col] = (sxx, sxy), fp32 value."""
+    m = op_div_matrix.coalesce()
+    row, col = m.indices()[0], m.indices()[1]
+    val = m.values()
+    ptr = ptr.to(row.device)
+    g = torch.searchsorted(ptr, row, right=True) - 1
+    n0, ni = ptr[g], ptr[g + 1] - ptr[g]
+    keep = (col >= 0) & (col < 2 * ni)
+    row, col, val, n0, ni = row[keep], col[keep], val[keep], n0[keep], ni[keep]
+    first = col < ni
+    node = n0 + torch.where(first, col, col - ni)
+    return row, node, first, val
+
+
+def loss_fp64(pred, local_stress, mean_ls, std_ls, ptr, op_div_matrix=None, labels=None, divergence=True,
+              penalty=1.0, upstream=(1.0, 1.0)):
+    """Vectorised fp64 restatement of ``train_loss``'s loss assembly (gnn_train.py:162-202) and of its gradient, for
+    any batch: segment sums instead of the per-graph loop and the dense operator blocks.
+
+    The ground truth is standardised in fp32, ``(local_stress - mean) / std`` rounded as IEEE fp32 like the reference
+    and the device kernel; everything after that is fp64 from the same fp32 ``pred``, ground truth and operator values.
+    ``upstream`` = (g_nmse, g_div) weights the two outputs in ``grad`` = d(g_nmse*nmse + g_div*div)/d pred.
+    Returns a namespace: gt (fp32), nmse_graph [B], div_node [N,2] (masked), div_graph [B] (before penalty),
+    nmse, div (= penalty * mean div_graph, 0 without divergence), total, grad [N,3]."""
+    dev = pred.device
+    f64 = torch.float64
+    ls = local_stress.to(torch.float32)
+    # full-size operands: a scalar divisor may be turned into a multiplication by its reciprocal
+    gt = (ls - torch.full_like(ls, float(mean_ls))) / torch.full_like(ls, float(std_ls))
+    ptr = ptr.to(dev)
+    b, n = ptr.numel() - 1, pred.shape[0]
+    ni = (ptr[1:] - ptr[:-1]).to(f64)
+    gid = torch.repeat_interleave(torch.arange(b, device=dev), ptr[1:] - ptr[:-1])
+    seg = lambda x: torch.zeros(b, *x.shape[1:], dtype=f64, device=dev).index_add_(0, gid, x)  # noqa: E731
+    p, t = pred.to(f64), gt.to(f64)
+    mean = seg(t) / ni[:, None]
+    norm = seg((t - mean[gid]).square())
+    d = p - t
+    nmse_graph = (seg(d.square()) / norm).mean(dim=1)
+    g_nmse, g_div = (float(v) for v in upstream)
+    grad = g_nmse * 2.0 * d / norm[gid] / (3.0 * b)
+    div_node = torch.zeros(n, 2, dtype=f64, device=dev)
+    div_graph = torch.zeros(b, dtype=f64, device=dev)
+    if divergence:
+        row, node, first, val = opdiv_entries(op_div_matrix, ptr)
+        v = val.to(f64)[:, None]
+        s = torch.where(first[:, None], p[node][:, [0, 2]], p[node][:, [2, 1]])
+        div_node.index_add_(0, row, v * s)
+        lab = labels.reshape(-1).to(dev)
+        div_node *= ((lab != 1) & (lab != -1)).to(f64)[:, None]
+        div_graph = seg(div_node.square()).sum(dim=1) / ni
+        # d div_graph_i / d S[col] = 2 / N_i * sum over rows of v * div[row]
+        ds = v * div_node[row] * (g_div * penalty * 2.0 / (ni[gid[row]] * b))[:, None]
+        grad.index_add_(0, node, torch.where(first[:, None], torch.stack([ds[:, 0], 0 * ds[:, 0], ds[:, 1]], 1),
+                                             torch.stack([0 * ds[:, 0], ds[:, 1], ds[:, 0]], 1)))
+    nmse = nmse_graph.sum() / b
+    div = penalty * div_graph.sum() / b if divergence else torch.zeros((), dtype=f64, device=dev)
+    return SimpleNamespace(gt=gt, nmse_graph=nmse_graph, div_node=div_node, div_graph=div_graph, nmse=nmse, div=div,
+                           total=nmse + div, grad=grad)
+
+
 def op_div_row_block(op, start: int, end: int):
     """What PyG ``Batch.get_example`` returns for the row-stacked sparse attribute
     (SURVEY 2.3d): rows [start,end) narrowed, column count unchanged."""

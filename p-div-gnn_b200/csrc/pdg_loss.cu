@@ -69,7 +69,7 @@ __global__ void k_gather32(const int32_t* __restrict__ src, const int32_t* __res
 }
 
 // ---- forward: one CTA per graph --------------------------------------------------------
-// ws_graph[i] = {nmse_i, div_i, 1/norm_0, 1/norm_1, 1/norm_2, N_i}; gdiv [N][2] masked divergence
+// ws_graph[i] = {nmse_i, div_i, 1/norm_0, 1/norm_1, 1/norm_2} (stride 8); gdiv [N][2] masked divergence
 constexpr int LOSS_NT = 256;
 __device__ __forceinline__ double block_sum_d(double v, double* red) {
   v = warp_sum(v);
@@ -121,7 +121,8 @@ k_loss_graph(const float* __restrict__ pred, const float* __restrict__ ls, float
     double d2[2] = {0, 0};
     for (int n = n0 + tid; n < n1; n += LOSS_NT) {
       float d0 = 0.f, d1 = 0.f;
-      if (labels[n] == 0) {
+      // the reference zeroes the rows labelled 1 or -1 (gnn_train.py:88-89) and keeps every other label
+      if (labels[n] != 1 && labels[n] != -1) {
         for (int k = rowptr[n]; k < rowptr[n + 1]; ++k) {
           const int j = col[k];
           if (j < 0) continue;  // column outside [0, 2 N_i): sliced away by the reference
@@ -148,7 +149,6 @@ k_loss_graph(const float* __restrict__ pred, const float* __restrict__ ls, float
     w[2] = inv_norm[0];
     w[3] = inv_norm[1];
     w[4] = inv_norm[2];
-    w[5] = (float)ni;
   }
 }
 
@@ -189,7 +189,7 @@ __global__ void k_loss_backward(const float* __restrict__ pred, const float* __r
   }
   if (use_div) {
     const int n0 = (int)gptr[lo];
-    const int ni = (int)w[5];
+    const int ni = (int)gptr[lo + 1] - n0;  // exact: a float holds N_i only up to 2^24
     const int ml = n - n0;
     float a0 = 0, a1 = 0, b0 = 0, b1 = 0;  // dS[ml][0], dS[ml][1], dS[ni+ml][0], dS[ni+ml][1]
     const int s1 = 2 * n0 + ml, s2 = 2 * n0 + ni + ml;
@@ -235,7 +235,7 @@ extern "C" int pdg_opdiv_plan_build(const int64_t* coo_row, const int64_t* coo_c
                                     const int64_t* graph_ptr, int64_t n_graphs, int64_t n_nodes, void* plan, void* tmp,
                                     size_t tmp_bytes, void* stream_) {
   cudaStream_t st = (cudaStream_t)stream_;
-  if (nnz <= 0 || nnz >= 0x7fffffff || n_nodes * 2 >= 0x7fffffff) { set_error("pdg_opdiv_plan_build: sizes out of range"); return -1; }
+  if (nnz < 0 || nnz >= 0x7fffffff || n_nodes * 2 >= 0x7fffffff) { set_error("pdg_opdiv_plan_build: sizes out of range"); return -1; }
   if (tmp_bytes < pdg_opdiv_tmp_bytes(n_nodes, nnz)) { set_error("pdg_opdiv_plan_build: tmp too small"); return -1; }
   OpPlanLayout L(n_nodes, nnz);
   char* pb = (char*)plan;
@@ -253,19 +253,25 @@ extern "C" int pdg_opdiv_plan_build(const int64_t* coo_row, const int64_t* coo_c
   int32_t* iota = (int32_t*)t; t += round_up(nnz * 4, 256);
   int32_t* skey_sorted = (int32_t*)t;
   const int TB = 256, gb = (int)((nnz + TB - 1) / TB);
-  k_op_keys<<<gb, TB, 0, st>>>(coo_row, coo_col, nnz, graph_ptr, (int)n_graphs, n_nodes, row32, col32, skey, iota);
-  PDG_LAUNCH_CHECK();
+  // nnz == 0 (an empty operator): no keys to make or sort; both pointer arrays come out all 0
+  if (nnz > 0) {
+    k_op_keys<<<gb, TB, 0, st>>>(coo_row, coo_col, nnz, graph_ptr, (int)n_graphs, n_nodes, row32, col32, skey, iota);
+    PDG_LAUNCH_CHECK();
+  }
   // CSR: coalesced COO is already row-sorted (torch .coalesce())
   k_lower_bound32<<<(int)((n_nodes + 1 + TB - 1) / TB), TB, 0, st>>>(row32, nnz, n_nodes, rowptr);
   PDG_LAUNCH_CHECK();
   int bits = 1;
   while ((1ll << bits) <= 2 * n_nodes && bits < 31) ++bits;
-  PDG_CUDA_CHECK(cub::DeviceRadixSort::SortPairs(sort_tmp, const_cast<size_t&>(sb), skey, skey_sorted, iota, tidx,
-                                                 (int)nnz, 0, bits, st));
+  if (nnz > 0)
+    PDG_CUDA_CHECK(cub::DeviceRadixSort::SortPairs(sort_tmp, const_cast<size_t&>(sb), skey, skey_sorted, iota, tidx,
+                                                   (int)nnz, 0, bits, st));
   k_lower_bound32<<<(int)((2 * n_nodes + 1 + TB - 1) / TB), TB, 0, st>>>(skey_sorted, nnz, 2 * n_nodes, tptr);
   PDG_LAUNCH_CHECK();
-  k_gather32<<<gb, TB, 0, st>>>(row32, tidx, nnz, trow);
-  PDG_LAUNCH_CHECK();
+  if (nnz > 0) {
+    k_gather32<<<gb, TB, 0, st>>>(row32, tidx, nnz, trow);
+    PDG_LAUNCH_CHECK();
+  }
   return 0;
 }
 
@@ -279,7 +285,7 @@ extern "C" int pdg_loss(const float* pred, const float* local_stress, const pdg_
                         void* stream_) {
   cudaStream_t st = (cudaStream_t)stream_;
   if (n_graphs <= 0 || n_nodes <= 0) { set_error("pdg_loss: empty batch"); return -1; }
-  if (use_divergence && (opdiv_plan == nullptr || op_val == nullptr || labels == nullptr)) {
+  if (use_divergence && (opdiv_plan == nullptr || (op_val == nullptr && nnz > 0) || labels == nullptr)) {
     set_error("pdg_loss: divergence requested without operator/labels");
     return -1;
   }
