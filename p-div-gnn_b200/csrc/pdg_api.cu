@@ -15,10 +15,10 @@ void set_error(const char* fmt, ...) {
   vsnprintf(g_err, sizeof(g_err), fmt, ap);
   va_end(ap);
 }
-int set_smem(const void* fn, size_t bytes) {
+int set_smem(const void* fn, size_t bytes, const char* name) {
   cudaError_t e = cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
   if (e != cudaSuccess) {
-    set_error("cudaFuncSetAttribute(%zu B smem): %s", bytes, cudaGetErrorString(e));
+    set_error("%s smem attribute (%zu B): %s", name, bytes, cudaGetErrorString(e));
     return -2;
   }
   return 0;

@@ -393,13 +393,13 @@ extern "C" int pdg_backward_inputs(const pdg_params_t* params, const pdg_norm_t*
   {
     ScopedTimer tm_(KC_DEC_BWD, st);
     const int* nzf = (flags & PDG_FLAG_ZERO_CHECK) ? W.nzflag : nullptr;
+    const DecArgs d = fwd_dec_args(W, P);  // what the forward's decoder read and saved
     if (tcm) {
-      if (launch_decoder_bwd_tc(grad_local_stress, gscale, gs, W.hd, W.x_[T], W.y3_[T - 1], W.parts_slot(slot_ln3(T - 1)), cnt_n,
-                                P[ND_W2], B.gx, B.cta_grads, B.cs3, nzf, N, nt_n, grid_n, W.img, st)) return -2;
+      if (launch_decoder_bwd_tc(grad_local_stress, gscale, gs, d.hd_out, d.x_out, d.yprev, d.prev_parts, d.prev_count, d.D2, B.gx,
+                                B.cta_grads, B.cs3, nzf, N, nt_n, grid_n, W.img, st)) return -2;
     } else {
-      PDG_CUDA_CHECK(launch_pdl(k_decoder_bwd, dim3(grid_n), dim3(NT), SMEM_B3T, st, grad_local_stress, gscale, W.hd, W.x_[T],
-                                W.y3_[T - 1], W.parts_slot(slot_ln3(T - 1)), cnt_n, P[ND_W0], P[ND_W2], B.gx, B.cta_grads, B.cs3,
-                                nzf, N, nt_n));
+      PDG_CUDA_CHECK(launch_pdl(k_decoder_bwd, dim3(grid_n), dim3(NT), SMEM_B3T, st, grad_local_stress, gscale, d.hd_out, d.x_out,
+                                d.yprev, d.prev_parts, d.prev_count, P[ND_W0], d.D2, B.gx, B.cta_grads, B.cs3, nzf, N, nt_n));
     }
   }
   PDG_LAUNCH_CHECK();

@@ -58,32 +58,29 @@ struct BwdStepArgs {
 inline BwdStepArgs bwd_step_args(const FwdWs& W, const float* const* P, const DataGradBufs& D, const int32_t* recv,
                                  const int32_t* send, const int32_t* rowptr, const int32_t* sptr, const int32_t* slist,
                                  int t) {
-  const bool last = t == W.T - 1, first = t == 0;
-  const int N = (int)W.N, E = (int)W.E, nt_n = (int)(W.N_pad / TM), nt_e = (int)(W.E_pad / TM);
-  const double cnt_n = (double)N * H, cnt_e = (double)E * H;
+  const bool last = t == W.T - 1;
+  const FwdStepArgs f = fwd_step_args(W, P, recv, send, rowptr, t);  // what forward step t read and wrote
   auto scal = [&](int slot) { return D.scal + slot * 4; };
   BwdStepArgs s = {};
   NodeUpdBwdArgs& u = s.u;
-  u.gx = D.gx; u.y3 = W.y3_[t]; u.hq = W.hq_[t]; u.aggraw = W.aggraw_[t]; u.x_t = W.x_[t]; u.rowptr = rowptr;
-  u.scal3 = scal(slot_ln3(t)); u.lnw_n = P[PN_LNW]; u.parts1 = W.parts_slot(slot_ln1(t)); u.count1 = cnt_e;
+  u.gx = D.gx; u.y3 = f.u.y3_out; u.hq = f.u.hq_out; u.aggraw = f.u.aggraw; u.x_t = f.u.x_t; u.rowptr = rowptr;
+  u.scal3 = scal(slot_ln3(t)); u.lnw_n = P[PN_LNW]; u.parts1 = f.u.parts1; u.count1 = f.u.count1;
   u.lnw_e = P[PE_LNW]; u.lnb_e = P[PE_LNB]; u.V1 = P[PN_W0]; u.V2 = P[PN_W2]; u.gagg = D.gagg;
-  u.cs1 = D.cs1; u.N = N; u.n_tiles = nt_n;
+  u.cs1 = D.cs1; u.N = f.u.N; u.n_tiles = f.u.n_tiles;
   EdgeBwdArgs& e = s.e;
-  e.e_t = W.e_[t]; e.Pa = W.Pa_[t]; e.Pb = W.Pb_[t]; e.gagg = D.gagg; e.ge = D.ge;
-  e.y2_t = last ? nullptr : W.y2_[t];
-  e.yprev = first ? W.y_eenc : W.y2_[t - 1];
-  e.parts_prev = W.parts_slot(first ? 1 : slot_ln2(t - 1)); e.count_prev = cnt_e;
+  e.e_t = f.e.e_out; e.Pa = f.e.Pa; e.Pb = f.e.Pb; e.gagg = D.gagg; e.ge = D.ge;
+  e.y2_t = f.e.y2_out; e.yprev = f.e.yprev; e.parts_prev = f.e.prev_parts; e.count_prev = f.e.prev_count;
   e.recv = recv; e.send = send; e.rowptr = rowptr;
-  e.WtE = W.pack + PackOffsets::PE_WET; e.b1 = P[PE_B0]; e.Wt2 = W.pack + PackOffsets::PE_W2T; e.b2 = P[PE_B2];
+  e.WtE = f.e.WtE; e.b1 = f.e.b1; e.Wt2 = f.e.Wt2; e.b2 = f.e.b2;
   e.W0 = P[PE_W0]; e.W2 = P[PE_W2]; e.lnw = P[PE_LNW];
   e.scal1 = scal(slot_ln1(t)); e.scal2 = last ? nullptr : scal(slot_ln2(t));
   e.DHM = D.DHM; e.DHN = D.DHN; e.RA = D.RA; e.RB = D.RB; e.cs2 = D.cs2;
-  e.E = E; e.n_tiles = nt_e; e.last = last ? 1 : 0;
+  e.E = f.e.E; e.n_tiles = f.e.n_tiles; e.last = last ? 1 : 0;
   NodePreBwdArgs& n = s.n;
   n.gx = D.gx; n.RA = D.RA; n.RB = last ? nullptr : D.RB; n.DHM = D.DHM; n.DHN = last ? nullptr : D.DHN;
-  n.sptr = sptr; n.slist = slist; n.x_t = W.x_[t]; n.yprev = first ? W.y_nenc : W.y3_[t - 1];
-  n.parts_prev = W.parts_slot(first ? 0 : slot_ln3(t - 1)); n.count_prev = cnt_n; n.W0 = P[PE_W0];
-  n.cs3 = D.cs3; n.N = N; n.n_tiles = nt_n;
+  n.sptr = sptr; n.slist = slist; n.x_t = f.np.x_out; n.yprev = f.np.yprev;
+  n.parts_prev = f.np.prev_parts; n.count_prev = f.np.prev_count; n.W0 = P[PE_W0];
+  n.cs3 = D.cs3; n.N = f.u.N; n.n_tiles = f.np.n_tiles;
   return s;
 }
 
@@ -615,20 +612,10 @@ __device__ __forceinline__ void encoder_bwd_body(const float* __restrict__ g_in,
       float f[8] = {0, 0, 0, 0, 0, 0, 0, 0};
       if (row < R) {
         if (NODE) {
-          float m0 = mean_stress[row * 3 + 0], m1 = mean_stress[row * 3 + 1], m2 = mean_stress[row * 3 + 2];
-          float p0 = pos[row * 2 + 0], p1 = pos[row * 2 + 1];
-          if (scale_in) {
-            m0 = (m0 - nrm.mean_mean_stress) / nrm.std_mean_stress;
-            m1 = (m1 - nrm.mean_mean_stress) / nrm.std_mean_stress;
-            m2 = (m2 - nrm.mean_mean_stress) / nrm.std_mean_stress;
-            p0 = (p0 - nrm.mean_pos) / nrm.std_pos;
-            p1 = (p1 - nrm.mean_pos) / nrm.std_pos;
-          }
-          f[0] = m0; f[1] = m1; f[2] = m2; f[3] = p0; f[4] = p1; f[5] = (float)types[row];
+          bool nz;
+          node_features(mean_stress, pos, types, nrm, scale_in, row, f, nz);
         } else {
-          float v = edge_attr[perm[row]];
-          if (scale_in) v = (v - nrm.mean_edge_weight) / nrm.std_edge_weight;
-          f[0] = v;
+          f[0] = edge_feature(edge_attr[perm[row]], nrm, scale_in);
         }
       }
 #pragma unroll

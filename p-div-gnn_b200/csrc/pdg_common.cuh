@@ -27,7 +27,7 @@ constexpr float LN_EPS = 1e-5f; // torch_geometric.nn.LayerNorm eps
 // ---- error reporting ---------------------------------------------------------------
 void set_error(const char* fmt, ...);
 // a kernel's dynamic shared-memory limit (cudaFuncAttributeMaxDynamicSharedMemorySize); -2 with the error set on failure
-int set_smem(const void* fn, size_t bytes);
+int set_smem(const void* fn, size_t bytes, const char* name = "kernel");
 int num_sms();
 #define PDG_CUDA_CHECK(expr)                                                          \
   do {                                                                                \
@@ -89,6 +89,22 @@ inline cudaError_t launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, s
   cfg.attrs = at;
   cfg.numAttrs = 1;
   return cudaLaunchKernelEx(&cfg, kernel, KArgs(args)...);
+}
+// Sets the kernel's shared-memory limit to `smem` and launches it, with launch_pdl when `pdl`; names it in set_error on
+// failure.  0, or -2.
+template <typename... KArgs, typename... Args>
+inline int launch_named(const char* name, bool pdl, void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem,
+                        cudaStream_t st, Args&&... args) {
+  if (set_smem((const void*)kernel, smem, name)) return -2;
+  cudaError_t e;
+  if (pdl) {
+    e = launch_pdl(kernel, grid, block, smem, st, args...);
+  } else {
+    kernel<<<grid, block, smem, st>>>(KArgs(args)...);
+    e = cudaGetLastError();
+  }
+  if (e != cudaSuccess) { set_error("%s launch: %s", name, cudaGetErrorString(e)); return -2; }
+  return 0;
 }
 #endif
 
@@ -279,6 +295,9 @@ __device__ __forceinline__ void tile_segsum_warp(const float* T, const int* recv
 }
 
 // ---- 128x128 register-tiled FFMA GEMM engine -----------------------------------------
+// dynamic shared memory of a kernel with one (1A) or two (2A) fp32 [128][LDS] tiles and the engine's weight chunks
+constexpr size_t SMEM_1A = (size_t)(TM * LDS + 2 * BK * H) * sizeof(float) + 1024 + 256;
+constexpr size_t SMEM_2A = (size_t)(2 * TM * LDS + 2 * BK * H) * sizeof(float) + 1024 + 256;
 // One micro-tile row update  acc[0..7] += a * {b0, b1}  as FOUR packed FFMA2 (fma.rn.f32x2, sm_100: two IEEE fp32 FMAs per
 // instruction, scalar-broadcast first operand -- SASS `FFMA2 Rd, Ra.F32, Rb.F32x2.HI_LO, Rc.F32x2.HI_LO`).  The 3-register
 // FFMA issues every other cycle per scheduler on Blackwell, so the scalar form tops out at half the fp32 peak; the packed
@@ -402,6 +421,57 @@ __device__ __forceinline__ void load_cols(float (&v)[8], const float* __restrict
   const float4 w = *reinterpret_cast<const float4*>(vec + 64 + tx * 4);
   v[0] = u.x; v[1] = u.y; v[2] = u.z; v[3] = u.w;
   v[4] = w.x; v[5] = w.y; v[6] = w.z; v[7] = w.w;
+}
+
+// ---- model arithmetic shared by the forward, its tangent and its backward --------------------------------
+// Each exists once so that the tangent and backward kernels recompute exactly the forward's values (ReLU masks).
+// the six standardised node features of one row (models.py:140-152) into f[0..5]; nz = any raw mean-stress entry is
+// non-zero (torch.any(mean_stress), models.py:294: raw values, NaN counts)
+__device__ __forceinline__ void node_features(const float* __restrict__ mean_stress, const float* __restrict__ pos,
+                                              const int64_t* __restrict__ types, const pdg_norm_t& nrm, int scale_in, int row,
+                                              float* f, bool& nz) {
+  float m0 = mean_stress[row * 3 + 0], m1 = mean_stress[row * 3 + 1], m2 = mean_stress[row * 3 + 2];
+  float p0 = pos[row * 2 + 0], p1 = pos[row * 2 + 1];
+  nz = m0 != 0.f || m1 != 0.f || m2 != 0.f;
+  if (scale_in) {
+    m0 = (m0 - nrm.mean_mean_stress) / nrm.std_mean_stress;
+    m1 = (m1 - nrm.mean_mean_stress) / nrm.std_mean_stress;
+    m2 = (m2 - nrm.mean_mean_stress) / nrm.std_mean_stress;
+    p0 = (p0 - nrm.mean_pos) / nrm.std_pos;
+    p1 = (p1 - nrm.mean_pos) / nrm.std_pos;
+  }
+  f[0] = m0; f[1] = m1; f[2] = m2; f[3] = p0; f[4] = p1; f[5] = (float)types[row];
+}
+// the standardised edge weight (models.py:154-162)
+__device__ __forceinline__ float edge_feature(float w, const pdg_norm_t& nrm, int scale_in) {
+  if (scale_in) w = (w - nrm.mean_edge_weight) / nrm.std_edge_weight;
+  return w;
+}
+// edge-MLP hidden layer of a 128-edge tile: acc = relu(G + P1[idx1[row]] + P2[idx2[row]])  (Gs: smem [128][LDS])
+__device__ __forceinline__ void gather_hidden(float (&acc)[8][8], const float* __restrict__ Gs, const float* __restrict__ P1,
+                                              const int* __restrict__ idx1, const float* __restrict__ P2,
+                                              const int* __restrict__ idx2) {
+  const int ty = threadIdx.x >> 4, tx = threadIdx.x & 15;
+#pragma unroll
+  for (int i = 0; i < 8; ++i) {
+    const int r = ty * 8 + i;
+    const float* p1 = P1 + (size_t)idx1[r] * H + tx * 4;
+    const float* p2 = P2 + (size_t)idx2[r] * H + tx * 4;
+    const float4 a0 = __ldg(reinterpret_cast<const float4*>(p1));
+    const float4 a1 = __ldg(reinterpret_cast<const float4*>(p1 + 64));
+    const float4 c0 = __ldg(reinterpret_cast<const float4*>(p2));
+    const float4 c1 = __ldg(reinterpret_cast<const float4*>(p2 + 64));
+    const float4 g0 = *reinterpret_cast<const float4*>(Gs + r * LDS + tx * 4);
+    const float4 g1 = *reinterpret_cast<const float4*>(Gs + r * LDS + 64 + tx * 4);
+    acc[i][0] = fmaxf(g0.x + a0.x + c0.x, 0.f);
+    acc[i][1] = fmaxf(g0.y + a0.y + c0.y, 0.f);
+    acc[i][2] = fmaxf(g0.z + a0.z + c0.z, 0.f);
+    acc[i][3] = fmaxf(g0.w + a0.w + c0.w, 0.f);
+    acc[i][4] = fmaxf(g1.x + a1.x + c1.x, 0.f);
+    acc[i][5] = fmaxf(g1.y + a1.y + c1.y, 0.f);
+    acc[i][6] = fmaxf(g1.z + a1.z + c1.z, 0.f);
+    acc[i][7] = fmaxf(g1.w + a1.w + c1.w, 0.f);
+  }
 }
 #endif  // __CUDACC__
 

@@ -26,8 +26,7 @@ struct SmemTile {
   float* A;
   float* Ws;
 };
-constexpr size_t SMEM_1A = (size_t)(TM * LDS + 2 * BK * H) * sizeof(float) + 1024 + 256;
-constexpr size_t SMEM_2A = (size_t)(2 * TM * LDS + 2 * BK * H) * sizeof(float) + 1024 + 256;
+constexpr size_t SMEM_ENC = SMEM_1A + TM * 8 * sizeof(float);
 
 // relu(acc + bias) in place; accumulate sum / sumsq over rows < nvalid
 __device__ __forceinline__ void bias_relu_stats(float (&acc)[8][8], const float (&bias)[8], int nvalid, float& s,
@@ -92,19 +91,7 @@ k_node_encoder(const float* __restrict__ mean_stress, const float* __restrict__ 
       const int row = row0 + tid;
       float f[6] = {0, 0, 0, 0, 0, 0};
       bool nz = false;
-      if (row < N) {
-        float m0 = mean_stress[row * 3 + 0], m1 = mean_stress[row * 3 + 1], m2 = mean_stress[row * 3 + 2];
-        float p0 = pos[row * 2 + 0], p1 = pos[row * 2 + 1];
-        nz = m0 != 0.f || m1 != 0.f || m2 != 0.f;  // torch.any(mean_stress), models.py:294 (raw values; NaN counts)
-        if (scale_in) {
-          m0 = (m0 - nrm.mean_mean_stress) / nrm.std_mean_stress;
-          m1 = (m1 - nrm.mean_mean_stress) / nrm.std_mean_stress;
-          m2 = (m2 - nrm.mean_mean_stress) / nrm.std_mean_stress;
-          p0 = (p0 - nrm.mean_pos) / nrm.std_pos;
-          p1 = (p1 - nrm.mean_pos) / nrm.std_pos;
-        }
-        f[0] = m0; f[1] = m1; f[2] = m2; f[3] = p0; f[4] = p1; f[5] = (float)types[row];
-      }
+      if (row < N) node_features(mean_stress, pos, types, nrm, scale_in, row, f, nz);
 #pragma unroll
       for (int j = 0; j < 6; ++j) feat[tid * 8 + j] = f[j];
       if (nzflag != nullptr && __any_sync(0xffffffffu, nz) && (tid & 31) == 0) atomicOr(nzflag, 1);  // warps 0-3, whole
@@ -134,6 +121,14 @@ k_node_encoder(const float* __restrict__ mean_stress, const float* __restrict__ 
     if (tid == 0) { tot_s += ds; tot_ss += dss; }
   }
   if (tid == 0) { parts[2 * blockIdx.x] = tot_s; parts[2 * blockIdx.x + 1] = tot_ss; }
+}
+template <bool INST>
+static int launch_node_encoder(const FwdWs& W, const float* const* P, const float* mean_stress, int64_t ms_stride,
+                               const float* pos, int64_t pos_stride, const int64_t* types, const pdg_norm_t* nrm, int scale_in,
+                               int* nzflag, dim3 grid, cudaStream_t st) {
+  return launch_named("k_node_encoder", true, k_node_encoder<INST>, grid, dim3(NT), SMEM_ENC, st, mean_stress, pos, types, *nrm,
+                      scale_in, P[NE_W0], P[NE_B0], W.pack + PackOffsets::NE_W2T, P[NE_B2], W.y_nenc, W.parts_slot(0), nzflag,
+                      (int)W.N, (int)(W.N_pad / TM), ms_stride, pos_stride, W.total);
 }
 
 // ------------------------------------------------------------------------------------
@@ -168,10 +163,7 @@ k_edge_encoder(const float* __restrict__ edge_attr, const int32_t* __restrict__ 
     const int nvalid = min(TM, E - row0);
     if (tid < TM) {
       float a = 0.f;
-      if (row0 + tid < E) {
-        a = edge_attr[perm[row0 + tid]];
-        if (scale_in) a = (a - nrm.mean_edge_weight) / nrm.std_edge_weight;
-      }
+      if (row0 + tid < E) a = edge_feature(edge_attr[perm[row0 + tid]], nrm, scale_in);
       feat[tid] = a;
     }
     __syncthreads();
@@ -194,6 +186,13 @@ k_edge_encoder(const float* __restrict__ edge_attr, const int32_t* __restrict__ 
     if (tid == 0) { tot_s += ds; tot_ss += dss; }
   }
   if (tid == 0) { parts[2 * blockIdx.x] = tot_s; parts[2 * blockIdx.x + 1] = tot_ss; }
+}
+template <bool INST>
+static int launch_edge_encoder(const FwdWs& W, const float* const* P, const float* edge_attr, int64_t ea_stride,
+                               const int32_t* perm, const pdg_norm_t* nrm, int scale_in, dim3 grid, cudaStream_t st) {
+  return launch_named("k_edge_encoder", false, k_edge_encoder<INST>, grid, dim3(NT), SMEM_ENC, st, edge_attr, perm, *nrm, scale_in,
+                      P[EE_W0], P[EE_B0], W.pack + PackOffsets::EE_W2T, P[EE_B2], W.y_eenc, W.parts_slot(1), (int)W.E,
+                      (int)(W.E_pad / TM), ea_stride, W.total);
 }
 
 // ------------------------------------------------------------------------------------
@@ -266,6 +265,12 @@ k_node_pre(const float* __restrict__ base, const float* __restrict__ yprev, cons
     }
   }
 }
+template <bool INST>
+static int launch_node_pre(const NodePreArgs& a, const float* pack, dim3 grid, size_t iws, cudaStream_t st) {
+  return launch_named("k_node_pre", false, k_node_pre<INST>, grid, dim3(NT), SMEM_1A, st, a.base, a.yprev, a.prev_parts,
+                      a.prev_count, a.lnw, a.lnb, a.x_out, pack + PackOffsets::PE_WAT, pack + PackOffsets::PE_WBT, a.Pa, a.Pb,
+                      a.n_tiles, iws);
+}
 
 // ------------------------------------------------------------------------------------
 // K2 edge_step: one Processor step on a tile of 128 receiver-sorted edges
@@ -277,33 +282,6 @@ k_node_pre(const float* __restrict__ base, const float* __restrict__ yprev, cons
 // LN partials of y1 -> slot LN1(t), of y2 -> slot LN2(t).
 // ------------------------------------------------------------------------------------
 constexpr size_t SMEM_EDGE = (size_t)(2 * TM * LDS + 2 * BK * H) * sizeof(float) + 2 * TM * sizeof(int) + 16 * sizeof(double) + 64 + 256;
-
-__device__ __forceinline__ void gather_hidden(float (&acc)[8][8], const float* __restrict__ Gs, const float* __restrict__ P1,
-                                              const int* __restrict__ idx1, const float* __restrict__ P2,
-                                              const int* __restrict__ idx2) {
-  // acc = relu(G + P1[idx1[row]] + P2[idx2[row]])
-  const int ty = threadIdx.x >> 4, tx = threadIdx.x & 15;
-#pragma unroll
-  for (int i = 0; i < 8; ++i) {
-    const int r = ty * 8 + i;
-    const float* p1 = P1 + (size_t)idx1[r] * H + tx * 4;
-    const float* p2 = P2 + (size_t)idx2[r] * H + tx * 4;
-    const float4 a0 = __ldg(reinterpret_cast<const float4*>(p1));
-    const float4 a1 = __ldg(reinterpret_cast<const float4*>(p1 + 64));
-    const float4 c0 = __ldg(reinterpret_cast<const float4*>(p2));
-    const float4 c1 = __ldg(reinterpret_cast<const float4*>(p2 + 64));
-    const float4 g0 = *reinterpret_cast<const float4*>(Gs + r * LDS + tx * 4);
-    const float4 g1 = *reinterpret_cast<const float4*>(Gs + r * LDS + 64 + tx * 4);
-    acc[i][0] = fmaxf(g0.x + a0.x + c0.x, 0.f);
-    acc[i][1] = fmaxf(g0.y + a0.y + c0.y, 0.f);
-    acc[i][2] = fmaxf(g0.z + a0.z + c0.z, 0.f);
-    acc[i][3] = fmaxf(g0.w + a0.w + c0.w, 0.f);
-    acc[i][4] = fmaxf(g1.x + a1.x + c1.x, 0.f);
-    acc[i][5] = fmaxf(g1.y + a1.y + c1.y, 0.f);
-    acc[i][6] = fmaxf(g1.z + a1.z + c1.z, 0.f);
-    acc[i][7] = fmaxf(g1.w + a1.w + c1.w, 0.f);
-  }
-}
 
 template <bool INST>
 __global__ void __launch_bounds__(NT, 1) k_edge_step(EdgeStepArgs a, size_t iws) {
@@ -429,6 +407,10 @@ __global__ void __launch_bounds__(NT, 1) k_edge_step(EdgeStepArgs a, size_t iws)
     }
   }
 }
+template <bool INST>
+static int launch_edge_step(const EdgeStepArgs& a, dim3 grid, size_t iws, cudaStream_t st) {
+  return launch_named("k_edge_step", false, k_edge_step<INST>, grid, dim3(NT), SMEM_EDGE, st, a, iws);
+}
 
 // ------------------------------------------------------------------------------------
 // K3 node_update: update() of models.py:240-243
@@ -522,6 +504,12 @@ k_node_update(const float* __restrict__ aggraw, const int32_t* __restrict__ rowp
   }
   if (tid == 0) { parts3[2 * blockIdx.x] = tot_s; parts3[2 * blockIdx.x + 1] = tot_ss; }
 }
+template <bool INST>
+static int launch_node_update(const NodeUpdArgs& a, const float* pack, dim3 grid, size_t iws, cudaStream_t st) {
+  return launch_named("k_node_update", false, k_node_update<INST>, grid, dim3(NT), SMEM_2A, st, a.aggraw, a.rowptr, a.parts1,
+                      a.count1, a.lnw_e, a.lnb_e, a.x_t, pack + PackOffsets::PN_WAT, pack + PackOffsets::PN_WXT, a.c1,
+                      pack + PackOffsets::PN_W2T, a.c2, a.hq_out, a.y3_out, a.parts3, a.N, a.n_tiles, iws);
+}
 
 // ------------------------------------------------------------------------------------
 // decoder: x_T = x_{T-1} + LN(y3_{T-1}); node_decoder (models.py:282-286, :316-321)
@@ -600,6 +588,12 @@ k_decoder(const float* __restrict__ base, const float* __restrict__ yprev, const
     __syncthreads();
   }
 }
+template <bool INST>
+static int launch_decoder(const DecArgs& d, const float* pack, dim3 grid, size_t iws, cudaStream_t st) {
+  return launch_named("k_decoder", true, k_decoder<INST>, grid, dim3(NT), SMEM_1A, st, d.base, d.yprev, d.prev_parts, d.prev_count,
+                      d.lnw, d.lnb, d.x_out, pack + PackOffsets::ND_W0T, d.d1, d.D2, d.d2, d.hd_out, d.out_scale, d.out_shift,
+                      d.out, d.nzflag, d.N, d.n_tiles, iws);
+}
 
 // All weight packs of one forward in ONE launch: blockIdx.y = job.
 //   kind 0: fp32 transpose  Wt[k][o] = W[o][col0 + k]                     (FFMA tiles, k-major B operand)
@@ -664,16 +658,15 @@ static cudaError_t memset_instances(void* p, size_t iws, size_t bytes, int K, cu
   return K == 1 ? cudaMemsetAsync(p, 0, bytes, st) : cudaMemset2DAsync(p, iws, 0, bytes, K, st);
 }
 
-// The fp32 (FFMA) forward of K instances of one graph.  Instance k's workspace is W moved by k * W.total bytes, its
-// inputs start k * (element stride) after the given pointers, its output at local_stress + k * N * 3.  The weights are
+// The forward of K instances of one graph.  fp32 (FFMA tiles): instance k's workspace is W moved by k * W.total bytes, its
+// inputs start k * (element stride) after the given pointers, its output at local_stress + k * N * 3; the weights are
 // packed once, into instance 0's workspace, and every instance reads them there.  pdg_forward is K = 1 with INST off.
+// tcm: the 16-bit mode's tensor-core kernels (pdg_tc_*.cu), K = 1.
 template <bool INST>
-int forward_ffma(const pdg_params_t* params, const pdg_norm_t* norm, const float* mean_stress, int64_t ms_stride,
-                 const float* pos, int64_t pos_stride, const int64_t* nodes_types, const float* edge_attr,
-                 int64_t ea_stride, const void* plan, const FwdWs& W, int flags, int K, float* local_stress,
-                 cudaStream_t st) {
+int forward_run(const pdg_params_t* params, const pdg_norm_t* norm, const float* mean_stress, int64_t ms_stride,
+                const float* pos, int64_t pos_stride, const int64_t* nodes_types, const float* edge_attr, int64_t ea_stride,
+                const void* plan, const FwdWs& W, int flags, int K, bool tcm, float* local_stress, cudaStream_t st) {
   const size_t iws = W.total;
-  const bool save = W.save;
   const int N = (int)W.N, E = (int)W.E, T = W.T;
   int32_t *perm, *recv, *send, *rowptr;
   pdg_plan_views(const_cast<void*>(plan), W.N, W.E, &perm, &recv, &send, &rowptr, nullptr, nullptr);
@@ -682,100 +675,71 @@ int forward_ffma(const pdg_params_t* params, const pdg_norm_t* norm, const float
   if (sms > MAXP) sms = MAXP;  // LayerNorm partials are kept per CTA in slots of MAXP entries (as in pdg_backward)
   const int grid_n = balanced_grid(nt_n, sms), grid_e = balanced_grid(nt_e, sms);
   const dim3 gn(grid_n, K), ge(grid_e, K);
-  const double cnt_n = (double)N * H, cnt_e = (double)E * H;
-  const size_t smem_enc = SMEM_1A + TM * 8 * sizeof(float);
-  if (set_smem((const void*)k_node_encoder<INST>, smem_enc)) return -2;
-  if (set_smem((const void*)k_edge_encoder<INST>, smem_enc)) return -2;
-  if (set_smem((const void*)k_node_pre<INST>, SMEM_1A)) return -2;
-  if (set_smem((const void*)k_edge_step<INST>, SMEM_EDGE)) return -2;
-  if (set_smem((const void*)k_node_update<INST>, SMEM_2A)) return -2;
-  if (set_smem((const void*)k_decoder<INST>, SMEM_1A)) return -2;
 
   // LayerNorm partials + the non-zero-load flag (contiguous) in one memset
   PDG_CUDA_CHECK(memset_instances(W.parts, iws, (size_t)((char*)W.nzflag - (char*)W.parts) + 256, K, st));
   int* nzflag = (flags & PDG_FLAG_ZERO_CHECK) ? W.nzflag : nullptr;
   {
     ScopedTimer tm_(KC_PACK, st);
-    if (pack_weights(params, W.pack, W.img, false, st)) return -2;
+    if (pack_weights(params, W.pack, W.img, tcm, st)) return -2;
   }
   const float* const* P = params->p;
-  const float* pk = W.pack;
   const int scale_in = (flags & PDG_FLAG_SCALE_INPUT) ? 1 : 0;
 
   {
     ScopedTimer tm_(KC_NODE_ENC, st);
-    PDG_CUDA_CHECK(launch_pdl(k_node_encoder<INST>, gn, dim3(NT), smem_enc, st, mean_stress, pos, nodes_types, *norm, scale_in,
-                              P[NE_W0], P[NE_B0], pk + PackOffsets::NE_W2T, P[NE_B2], W.y_nenc, W.parts_slot(0), nzflag, N,
-                              nt_n, ms_stride, pos_stride, iws));
+    if (tcm ? launch_node_encoder_tc(mean_stress, pos, nodes_types, norm, scale_in, P[NE_W0], P[NE_B0], P[NE_B2], W.y_nenc,
+                                     W.parts_slot(0), nzflag, N, nt_n, grid_n, W.img, st)
+            : launch_node_encoder<INST>(W, P, mean_stress, ms_stride, pos, pos_stride, nodes_types, norm, scale_in, nzflag, gn, st))
+      return -2;
   }
   PDG_LAUNCH_CHECK();
   {
     ScopedTimer tm_(KC_EDGE_ENC, st);
-    k_edge_encoder<INST><<<ge, NT, smem_enc, st>>>(edge_attr, perm, *norm, scale_in, P[EE_W0], P[EE_B0],
-                                                   pk + PackOffsets::EE_W2T, P[EE_B2], W.y_eenc, W.parts_slot(1), E, nt_e,
-                                                   ea_stride, iws);
+    if (tcm ? launch_edge_encoder_tc(edge_attr, perm, norm, scale_in, P[EE_W0], P[EE_B0], P[EE_B2], W.y_eenc, W.parts_slot(1), E,
+                                     nt_e, W.img, st)
+            : launch_edge_encoder<INST>(W, P, edge_attr, ea_stride, perm, norm, scale_in, ge, st))
+      return -2;
   }
   PDG_LAUNCH_CHECK();
   for (int t = 0; t < T; ++t) {
-    const bool first = t == 0, last = t == T - 1;
-    // K1
+    FwdStepArgs s = fwd_step_args(W, P, recv, send, rowptr, t);
+    if (tcm) {
+      s.np.aggraw_zero = W.aggraw_[t];  // zeroed by node_pre instead of a memset between the kernels (keeps the PDL chain)
+      s.np.b1 = P[PE_B0];
+      s.e.e_out = t < T - 1 ? W.e_[t] : nullptr;  // with `save` too: the backward reads the fp16 image instead
+      s.np.x_img = W.ximg(t);
+      s.u.x_img = s.np.x_img;
+      s.e.e_img = W.eimg_[t];  // the images for the backward are null without `save`
+      s.u.hq_img = W.hqimg(t);
+      s.u.agg_img = W.aggimg(t);
+    }
     {
       ScopedTimer tm_(KC_NODE_PRE, st);
-      k_node_pre<INST><<<gn, NT, SMEM_1A, st>>>(first ? nullptr : W.x_[t - 1], first ? W.y_nenc : W.y3_[t - 1],
-                                                W.parts_slot(first ? 0 : slot_ln3(t - 1)), cnt_n,
-                                                first ? P[NE_LNW] : P[PN_LNW], first ? P[NE_LNB] : P[PN_LNB], W.x_[t],
-                                                pk + PackOffsets::PE_WAT, pk + PackOffsets::PE_WBT, W.Pa_[t], W.Pb_[t], nt_n,
-                                                iws);
+      if (tcm ? launch_node_pre_tc(s.np, W.img, nt_n, st) : launch_node_pre<INST>(s.np, W.pack, gn, iws, st)) return -2;
     }
     PDG_LAUNCH_CHECK();
-    // K2
-    PDG_CUDA_CHECK(memset_instances(W.aggraw_[t], iws, (size_t)W.N_pad * H * sizeof(float), K, st));
-    EdgeStepArgs a;
-    a.base = first ? nullptr : W.e_[t - 1];
-    a.yprev = first ? W.y_eenc : W.y2_[t - 1];
-    a.prev_parts = W.parts_slot(first ? 1 : slot_ln2(t - 1));
-    a.prev_count = cnt_e;
-    a.prev_w = first ? P[EE_LNW] : P[PE_LNW];
-    a.prev_b = first ? P[EE_LNB] : P[PE_LNB];
-    a.e_out = (save || !last) ? W.e_[t] : nullptr;
-    a.e_img = nullptr;
-    a.Pa = W.Pa_[t];
-    a.Pb = W.Pb_[t];
-    a.recv = recv;
-    a.send = send;
-    a.rowptr = rowptr;
-    a.WtE = pk + PackOffsets::PE_WET;
-    a.b1 = P[PE_B0];
-    a.Wt2 = pk + PackOffsets::PE_W2T;
-    a.b2 = P[PE_B2];
-    a.y2_out = last ? nullptr : W.y2_[t];
-    a.aggraw = W.aggraw_[t];
-    a.parts1 = W.parts_slot(slot_ln1(t));
-    a.parts2 = last ? nullptr : W.parts_slot(slot_ln2(t));
-    a.E = E;
-    a.n_tiles = nt_e;
+    if (!tcm) PDG_CUDA_CHECK(memset_instances(W.aggraw_[t], iws, (size_t)W.N_pad * H * sizeof(float), K, st));
     {
       ScopedTimer tm_(KC_EDGE_STEP, st);
-      k_edge_step<INST><<<ge, NT, SMEM_EDGE, st>>>(a, iws);
+      if (tcm ? launch_edge_step_tc(s.e, W.img, grid_e, st) : launch_edge_step<INST>(s.e, ge, iws, st)) return -2;
     }
     PDG_LAUNCH_CHECK();
-    // K3
     {
       ScopedTimer tm_(KC_NODE_UPD, st);
-      k_node_update<INST><<<gn, NT, SMEM_2A, st>>>(W.aggraw_[t], rowptr, W.parts_slot(slot_ln1(t)), cnt_e, P[PE_LNW],
-                                                   P[PE_LNB], W.x_[t], pk + PackOffsets::PN_WAT, pk + PackOffsets::PN_WXT,
-                                                   P[PN_B0], pk + PackOffsets::PN_W2T, P[PN_B2], save ? W.hq_[t] : nullptr,
-                                                   W.y3_[t], W.parts_slot(slot_ln3(t)), N, nt_n, iws);
+      if (tcm ? launch_node_update_tc(s.u, W.img, grid_n, st) : launch_node_update<INST>(s.u, W.pack, gn, iws, st)) return -2;
     }
     PDG_LAUNCH_CHECK();
   }
+  DecArgs d = fwd_dec_args(W, P);
   const bool scale_out = (flags & PDG_FLAG_SCALE_OUTPUT) != 0;
+  d.out_scale = scale_out ? norm->std_local_stress : 1.f;
+  d.out_shift = scale_out ? norm->mean_local_stress : 0.f;
+  d.out = local_stress;
+  d.nzflag = nzflag;
   {
     ScopedTimer tm_(KC_DECODER, st);
-    PDG_CUDA_CHECK(launch_pdl(k_decoder<INST>, gn, dim3(NT), SMEM_1A, st, W.x_[T - 1], W.y3_[T - 1], W.parts_slot(slot_ln3(T - 1)),
-                              cnt_n, P[PN_LNW], P[PN_LNB], save ? W.x_[T] : nullptr, pk + PackOffsets::ND_W0T, P[ND_B0], P[ND_W2],
-                              P[ND_B2], save ? W.hd : nullptr, scale_out ? norm->std_local_stress : 1.f,
-                              scale_out ? norm->mean_local_stress : 0.f, local_stress, nzflag, N, nt_n, iws));
+    if (tcm ? launch_decoder_tc(d, W.img, grid_n, st) : launch_decoder<INST>(d, W.pack, gn, iws, st)) return -2;
   }
   PDG_LAUNCH_CHECK();
   return 0;
@@ -804,109 +768,7 @@ extern "C" int pdg_forward(const pdg_params_t* params, const pdg_norm_t* norm, c
   const bool save = (flags & PDG_FLAG_SAVE) != 0;
   FwdWs W(n_nodes, n_edges, steps, save, ws, tcm);
   if (ws_bytes < W.total) { set_error("pdg_forward: workspace %zu < %zu", ws_bytes, W.total); return -1; }
-  if (!tcm) return forward_ffma<false>(params, norm, mean_stress, 0, pos, 0, nodes_types, edge_attr, 0, plan, W, flags, 1,
-                                       local_stress, st);
-  // 16-bit mode: tcgen05 tile kernels (pdg_tc_*.cu)
-  const int N = (int)n_nodes, E = (int)n_edges, T = steps;
-  int32_t *perm, *recv, *send, *rowptr;
-  pdg_plan_views(const_cast<void*>(plan), n_nodes, n_edges, &perm, &recv, &send, &rowptr, nullptr, nullptr);
-  const int nt_n = (int)(W.N_pad / TM), nt_e = (int)(W.E_pad / TM);
-  int sms = num_sms();
-  if (sms > MAXP) sms = MAXP;  // LayerNorm partials are kept per CTA in slots of MAXP entries (as in pdg_backward)
-  const int grid_n = balanced_grid(nt_n, sms), grid_e = balanced_grid(nt_e, sms);
-  const double cnt_n = (double)N * H, cnt_e = (double)E * H;
-
-  // LayerNorm partials + the non-zero-load flag (contiguous) in one memset
-  PDG_CUDA_CHECK(cudaMemsetAsync(W.parts, 0, (size_t)((char*)W.nzflag - (char*)W.parts) + 256, st));
-  int* nzflag = (flags & PDG_FLAG_ZERO_CHECK) ? W.nzflag : nullptr;
-  {
-    ScopedTimer tm_(KC_PACK, st);
-    if (pack_weights(params, W.pack, W.img, tcm, st)) return -2;
-  }
-  const float* const* P = params->p;
-  const int scale_in = (flags & PDG_FLAG_SCALE_INPUT) ? 1 : 0;
-
-  {
-    ScopedTimer tm_(KC_NODE_ENC, st);
-    if (launch_node_encoder_tc(mean_stress, pos, nodes_types, norm, scale_in, P[NE_W0], P[NE_B0], P[NE_B2], W.y_nenc,
-                               W.parts_slot(0), nzflag, N, nt_n, grid_n, W.img, st)) return -2;
-  }
-  PDG_LAUNCH_CHECK();
-  {
-    ScopedTimer tm_(KC_EDGE_ENC, st);
-    if (launch_edge_encoder_tc(edge_attr, perm, norm, scale_in, P[EE_W0], P[EE_B0], P[EE_B2], W.y_eenc, W.parts_slot(1), E,
-                               nt_e, W.img, st)) return -2;
-  }
-  PDG_LAUNCH_CHECK();
-  for (int t = 0; t < T; ++t) {
-    const bool first = t == 0, last = t == T - 1;
-    // K1
-    {
-      ScopedTimer tm_(KC_NODE_PRE, st);
-      NodePreArgs np;
-      np.base = first ? nullptr : W.x_[t - 1]; np.yprev = first ? W.y_nenc : W.y3_[t - 1];
-      np.prev_parts = W.parts_slot(first ? 0 : slot_ln3(t - 1)); np.prev_count = cnt_n;
-      np.lnw = first ? P[NE_LNW] : P[PN_LNW]; np.lnb = first ? P[NE_LNB] : P[PN_LNB];
-      np.x_out = W.x_[t]; np.Pa = W.Pa_[t]; np.Pb = W.Pb_[t]; np.n_tiles = nt_n;
-      np.aggraw_zero = W.aggraw_[t];  // zeroed here instead of a memset between the kernels (keeps the PDL chain)
-      np.b1 = P[PE_B0];
-      np.x_img = W.ximg(t);
-      if (launch_node_pre_tc(np, W.img, nt_n, st)) return -2;
-    }
-    PDG_LAUNCH_CHECK();
-    // K2
-    EdgeStepArgs a;
-    a.base = first ? nullptr : W.e_[t - 1];
-    a.yprev = first ? W.y_eenc : W.y2_[t - 1];
-    a.prev_parts = W.parts_slot(first ? 1 : slot_ln2(t - 1));
-    a.prev_count = cnt_e;
-    a.prev_w = first ? P[EE_LNW] : P[PE_LNW];
-    a.prev_b = first ? P[EE_LNB] : P[PE_LNB];
-    a.e_out = !last ? W.e_[t] : nullptr;  // the backward reads the fp16 image instead
-    a.e_img = save ? W.eimg_[t] : nullptr;
-    a.Pa = W.Pa_[t];
-    a.Pb = W.Pb_[t];
-    a.recv = recv;
-    a.send = send;
-    a.rowptr = rowptr;
-    a.WtE = W.pack + PackOffsets::PE_WET;
-    a.b1 = P[PE_B0];
-    a.Wt2 = W.pack + PackOffsets::PE_W2T;
-    a.b2 = P[PE_B2];
-    a.y2_out = last ? nullptr : W.y2_[t];
-    a.aggraw = W.aggraw_[t];
-    a.parts1 = W.parts_slot(slot_ln1(t));
-    a.parts2 = last ? nullptr : W.parts_slot(slot_ln2(t));
-    a.E = E;
-    a.n_tiles = nt_e;
-    {
-      ScopedTimer tm_(KC_EDGE_STEP, st);
-      if (launch_edge_step_tc(a, W.img, grid_e, st)) return -2;
-    }
-    PDG_LAUNCH_CHECK();
-    // K3
-    {
-      ScopedTimer tm_(KC_NODE_UPD, st);
-      NodeUpdArgs nu;
-      nu.aggraw = W.aggraw_[t]; nu.rowptr = rowptr; nu.parts1 = W.parts_slot(slot_ln1(t)); nu.count1 = cnt_e;
-      nu.lnw_e = P[PE_LNW]; nu.lnb_e = P[PE_LNB]; nu.x_t = W.x_[t]; nu.c1 = P[PN_B0]; nu.c2 = P[PN_B2];
-      nu.hq_out = save ? W.hq_[t] : nullptr; nu.y3_out = W.y3_[t]; nu.parts3 = W.parts_slot(slot_ln3(t));
-      nu.N = N; nu.n_tiles = nt_n;
-      nu.x_img = W.ximg(t); nu.hq_img = save ? W.hqimg(t) : nullptr; nu.agg_img = save ? W.aggimg(t) : nullptr;
-      if (launch_node_update_tc(nu, W.img, grid_n, st)) return -2;
-    }
-    PDG_LAUNCH_CHECK();
-  }
-  const bool scale_out = (flags & PDG_FLAG_SCALE_OUTPUT) != 0;
-  {
-    ScopedTimer tm_(KC_DECODER, st);
-    if (launch_decoder_tc(W.x_[T - 1], W.y3_[T - 1], W.parts_slot(slot_ln3(T - 1)), cnt_n, P[PN_LNW], P[PN_LNB],
-                          save ? W.x_[T] : nullptr, P[ND_B0], P[ND_W2], P[ND_B2], save ? W.hd : nullptr,
-                          scale_out ? norm->std_local_stress : 1.f, scale_out ? norm->mean_local_stress : 0.f, local_stress,
-                          nzflag, N, nt_n, grid_n, W.img, st)) return -2;
-  }
-  PDG_LAUNCH_CHECK();
-  return 0;
+  return forward_run<false>(params, norm, mean_stress, 0, pos, 0, nodes_types, edge_attr, 0, plan, W, flags, 1, tcm, local_stress, st);
 }
 
 // K instances of one graph: the workspace holds K fp32 forward workspaces without saved state, one after another
@@ -947,8 +809,8 @@ extern "C" int pdg_forward_batched(const pdg_params_t* params, const pdg_norm_t*
     set_error("pdg_forward_batched: workspace %zu < %zu", ws_bytes, (size_t)K * W.total);
     return -1;
   }
-  return forward_ffma<true>(params, norm, mean_stress, ms_stride, pos, pos_stride, nodes_types, edge_attr, ea_stride,
-                            plan, W, flags, K, local_stress, (cudaStream_t)stream_);
+  return forward_run<true>(params, norm, mean_stress, ms_stride, pos, pos_stride, nodes_types, edge_attr, ea_stride, plan, W,
+                           flags, K, false, local_stress, (cudaStream_t)stream_);
 }
 
 // Test/debug helper: byte offset and element count of a saved tensor inside a forward

@@ -29,9 +29,7 @@
 namespace pdg {
 
 constexpr int BKJ = 16;  // weight k-chunk of the edge kernel (three tiles + two chunks fit in 227 KB, as k_edge_step_bwd)
-constexpr size_t SMEM_J1A = (size_t)(TM * LDS + 2 * BK * H) * sizeof(float) + 1024 + 256;
-constexpr size_t SMEM_J2A = (size_t)(2 * TM * LDS + 2 * BK * H) * sizeof(float) + 1024 + 256;
-constexpr size_t SMEM_JENC = SMEM_J1A + TM * 16 * sizeof(float);
+constexpr size_t SMEM_JENC = SMEM_1A + TM * 16 * sizeof(float);
 constexpr size_t SMEM_JEDGE = (size_t)(3 * TM * LDS + 2 * BKJ * H) * sizeof(float) + 2 * TM * sizeof(int) + 16 * sizeof(double) +
                               8 * sizeof(float) + 4 * sizeof(unsigned) + TM + 1 + 256;
 // per tangent of an edge-kernel group: the LayerNorm tangent statistics {mud, c} and the fp64 partials {t1s, t1c, t2s, t2c}
@@ -148,17 +146,8 @@ k_node_encoder_jvp(const float* __restrict__ mean_stress, const float* __restric
       const int row = row0 + tid;
       float f[6] = {0, 0, 0, 0, 0, 0}, fd[6] = {0, 0, 0, 0, 0, 0};
       if (row < N) {
-        // primal features exactly as k_node_encoder forms them (the first-layer mask must be the forward's)
-        float m0 = mean_stress[row * 3 + 0], m1 = mean_stress[row * 3 + 1], m2 = mean_stress[row * 3 + 2];
-        float p0 = pos[row * 2 + 0], p1 = pos[row * 2 + 1];
-        if (scale_in) {
-          m0 = (m0 - nrm.mean_mean_stress) / nrm.std_mean_stress;
-          m1 = (m1 - nrm.mean_mean_stress) / nrm.std_mean_stress;
-          m2 = (m2 - nrm.mean_mean_stress) / nrm.std_mean_stress;
-          p0 = (p0 - nrm.mean_pos) / nrm.std_pos;
-          p1 = (p1 - nrm.mean_pos) / nrm.std_pos;
-        }
-        f[0] = m0; f[1] = m1; f[2] = m2; f[3] = p0; f[4] = p1; f[5] = (float)types[row];
+        bool nz;
+        node_features(mean_stress, pos, types, nrm, scale_in, row, f, nz);  // the forward's features: its first-layer mask
         if (tan_ms != nullptr)
 #pragma unroll
           for (int j = 0; j < 3; ++j) fd[j] = scale_in ? tan_ms[row * 3 + j] / nrm.std_mean_stress : tan_ms[row * 3 + j];
@@ -229,8 +218,7 @@ k_edge_encoder_jvp(const float* __restrict__ edge_attr, const int32_t* __restric
       float a = 0.f, ad = 0.f;
       if (row0 + tid < E) {
         const int src = perm[row0 + tid];
-        a = edge_attr[src];
-        if (scale_in) a = (a - nrm.mean_edge_weight) / nrm.std_edge_weight;
+        a = edge_feature(edge_attr[src], nrm, scale_in);
         if (tan_ea != nullptr) ad = scale_in ? tan_ea[src] / nrm.std_edge_weight : tan_ea[src];
       }
       feat[tid] = a;
@@ -361,32 +349,6 @@ struct EdgeJvpArgs {
   int K, C;    // tangents of the pass; tangents per CTA group (blockIdx.y = group)
 };
 
-// acc = relu(G + P1[idx1[row]] + P2[idx2[row]])  (the arithmetic of k_edge_step's gather_hidden, so the masks are its)
-__device__ __forceinline__ void gather_hidden_j(float (&acc)[8][8], const float* __restrict__ Gs, const float* __restrict__ P1,
-                                                const int* __restrict__ idx1, const float* __restrict__ P2,
-                                                const int* __restrict__ idx2) {
-  const int ty = threadIdx.x >> 4, tx = threadIdx.x & 15;
-#pragma unroll
-  for (int i = 0; i < 8; ++i) {
-    const int r = ty * 8 + i;
-    const float* p1 = P1 + (size_t)idx1[r] * H + tx * 4;
-    const float* p2 = P2 + (size_t)idx2[r] * H + tx * 4;
-    const float4 a0 = __ldg(reinterpret_cast<const float4*>(p1));
-    const float4 a1 = __ldg(reinterpret_cast<const float4*>(p1 + 64));
-    const float4 c0 = __ldg(reinterpret_cast<const float4*>(p2));
-    const float4 c1 = __ldg(reinterpret_cast<const float4*>(p2 + 64));
-    const float4 g0 = *reinterpret_cast<const float4*>(Gs + r * LDS + tx * 4);
-    const float4 g1 = *reinterpret_cast<const float4*>(Gs + r * LDS + 64 + tx * 4);
-    acc[i][0] = fmaxf(g0.x + a0.x + c0.x, 0.f);
-    acc[i][1] = fmaxf(g0.y + a0.y + c0.y, 0.f);
-    acc[i][2] = fmaxf(g0.z + a0.z + c0.z, 0.f);
-    acc[i][3] = fmaxf(g0.w + a0.w + c0.w, 0.f);
-    acc[i][4] = fmaxf(g1.x + a1.x + c1.x, 0.f);
-    acc[i][5] = fmaxf(g1.y + a1.y + c1.y, 0.f);
-    acc[i][6] = fmaxf(g1.z + a1.z + c1.z, 0.f);
-    acc[i][7] = fmaxf(g1.w + a1.w + c1.w, 0.f);
-  }
-}
 // acc = m (Gd + P1d[idx1[row]] + P2d[idx2[row]]), bit i*8+j of m = mask of micro-tile element (i, j)
 __device__ __forceinline__ void gather_hidden_tan(float (&acc)[8][8], const float* __restrict__ Gd, const float* __restrict__ P1,
                                                   const int* __restrict__ idx1, const float* __restrict__ P2,
@@ -511,10 +473,10 @@ __global__ void __launch_bounds__(NT, 1) k_edge_step_jvp(EdgeJvpArgs a) {
     __syncthreads();  // T1 visible
     unsigned long long m2 = 0;
     if (upd) {
-      gather_hidden_j(acc, T1, a.Pa, send_s, a.Pb, recv_s);
+      gather_hidden(acc, T1, a.Pa, send_s, a.Pb, recv_s);  // the forward's: its masks
       m2 = pos_bits(acc);
     }
-    gather_hidden_j(acc, T1, a.Pa, recv_s, a.Pb, send_s);
+    gather_hidden(acc, T1, a.Pa, recv_s, a.Pb, send_s);
     const unsigned long long m1 = pos_bits(acc);
     acc_store(acc, T0, LDS);
     acc_zero(acc);
@@ -780,12 +742,6 @@ extern "C" int pdg_jvp_batched(const pdg_params_t* params, const pdg_norm_t* nor
   groups = (K + C - 1) / C;  // no empty group
   const size_t smem_edge = SMEM_JEDGE + (size_t)C * SMEM_JEDGE_TAN;
   const double cnt_n = (double)N * H, cnt_e = (double)E * H;
-  if (set_smem((const void*)k_node_encoder_jvp, SMEM_JENC)) return -2;
-  if (set_smem((const void*)k_edge_encoder_jvp, SMEM_JENC)) return -2;
-  if (set_smem((const void*)k_node_pre_jvp, SMEM_J1A)) return -2;
-  if (set_smem((const void*)k_edge_step_jvp, smem_edge)) return -2;
-  if (set_smem((const void*)k_node_update_jvp, SMEM_J2A)) return -2;
-  if (set_smem((const void*)k_decoder_jvp, SMEM_J1A)) return -2;
 
   // tangent partials of all K tangents (one strided memset): slots of CTAs that do not exist must read as zero
   PDG_CUDA_CHECK(cudaMemset2DAsync(J.parts, tws, 0, (size_t)(2 + 3 * T) * MAXP * 2 * sizeof(double), K, st));
@@ -796,59 +752,57 @@ extern "C" int pdg_jvp_batched(const pdg_params_t* params, const pdg_norm_t* nor
   const dim3 gn(grid_n, K), ge(grid_e, K);
   {
     ScopedTimer tm_(KC_JVP_NODE_ENC, st);
-    k_node_encoder_jvp<<<gn, NT, SMEM_JENC, st>>>(mean_stress, pos, nodes_types, *norm, scale_in, tan_mean_stress, tan_pos,
-                                                  P[NE_W0], P[NE_B0], pk + PackOffsets::NE_W2T, F.y_nenc, F.parts_slot(0),
-                                                  cnt_n, J.y_nenc, J.parts_slot(0), N, nt_n, ms_stride, pos_stride, tws);
+    if (launch_named("k_node_encoder_jvp", false, k_node_encoder_jvp, gn, dim3(NT), SMEM_JENC, st, mean_stress, pos, nodes_types,
+                     *norm, scale_in, tan_mean_stress, tan_pos, P[NE_W0], P[NE_B0], pk + PackOffsets::NE_W2T, F.y_nenc,
+                     F.parts_slot(0), cnt_n, J.y_nenc, J.parts_slot(0), N, nt_n, ms_stride, pos_stride, tws)) return -2;
   }
   PDG_LAUNCH_CHECK();
   {
     ScopedTimer tm_(KC_JVP_EDGE_ENC, st);
-    k_edge_encoder_jvp<<<ge, NT, SMEM_JENC, st>>>(edge_attr, perm, *norm, scale_in, tan_edge_attr, P[EE_W0], P[EE_B0],
-                                                  pk + PackOffsets::EE_W2T, F.y_eenc, F.parts_slot(1), cnt_e, J.y_eenc,
-                                                  J.parts_slot(1), E, nt_e, ea_stride, tws);
+    if (launch_named("k_edge_encoder_jvp", false, k_edge_encoder_jvp, ge, dim3(NT), SMEM_JENC, st, edge_attr, perm, *norm, scale_in,
+                     tan_edge_attr, P[EE_W0], P[EE_B0], pk + PackOffsets::EE_W2T, F.y_eenc, F.parts_slot(1), cnt_e, J.y_eenc,
+                     J.parts_slot(1), E, nt_e, ea_stride, tws)) return -2;
   }
   PDG_LAUNCH_CHECK();
+  // step t of the forward on F gives the primal state, on J the tangent state
   for (int t = 0; t < T; ++t) {
-    const bool first = t == 0, last = t == T - 1;
+    const FwdStepArgs f = fwd_step_args(F, P, recv, send, rowptr, t), j = fwd_step_args(J, P, recv, send, rowptr, t);
     {
       ScopedTimer tm_(KC_JVP_NODE_PRE, st);
-      const int ps = first ? 0 : slot_ln3(t - 1);
-      k_node_pre_jvp<<<gn, NT, SMEM_J1A, st>>>(first ? F.y_nenc : F.y3_[t - 1], F.parts_slot(ps), J.parts_slot(ps), cnt_n,
-                                               first ? P[NE_LNW] : P[PN_LNW], first ? nullptr : J.x_[t - 1],
-                                               first ? J.y_nenc : J.y3_[t - 1], J.x_[t], pk + PackOffsets::PE_WAT,
-                                               pk + PackOffsets::PE_WBT, J.Pa_[t], J.Pb_[t], nt_n, tws);
+      if (launch_named("k_node_pre_jvp", false, k_node_pre_jvp, gn, dim3(NT), SMEM_1A, st, f.np.yprev, f.np.prev_parts,
+                       j.np.prev_parts, f.np.prev_count, f.np.lnw, j.np.base, j.np.yprev, j.np.x_out, pk + PackOffsets::PE_WAT,
+                       pk + PackOffsets::PE_WBT, j.np.Pa, j.np.Pb, nt_n, tws)) return -2;
     }
     PDG_LAUNCH_CHECK();
     PDG_CUDA_CHECK(cudaMemset2DAsync(J.aggraw_[t], tws, 0, (size_t)J.N_pad * H * sizeof(float), K, st));
     EdgeJvpArgs a;
-    const int ps = first ? 1 : slot_ln2(t - 1);
-    a.yprev = first ? F.y_eenc : F.y2_[t - 1];
-    a.prev_parts = F.parts_slot(ps);
-    a.prev_w = first ? P[EE_LNW] : P[PE_LNW];
-    a.e_t = F.e_[t];
-    a.Pa = F.Pa_[t];
-    a.Pb = F.Pb_[t];
-    a.y2_t = last ? nullptr : F.y2_[t];
-    a.parts1 = F.parts_slot(slot_ln1(t));
-    a.parts2 = last ? nullptr : F.parts_slot(slot_ln2(t));
-    a.tprev_parts = J.parts_slot(ps);
-    a.tbase = first ? nullptr : J.e_[t - 1];
-    a.typrev = first ? J.y_eenc : J.y2_[t - 1];
-    a.te_out = last ? nullptr : J.e_[t];  // ed_t is read again only by the next step
-    a.tPa = J.Pa_[t];
-    a.tPb = J.Pb_[t];
-    a.ty2_out = last ? nullptr : J.y2_[t];
-    a.taggraw = J.aggraw_[t];
-    a.tparts1 = J.parts_slot(slot_ln1(t));
-    a.tparts2 = last ? nullptr : J.parts_slot(slot_ln2(t));
+    a.yprev = f.e.yprev;
+    a.prev_parts = f.e.prev_parts;
+    a.prev_w = f.e.prev_w;
+    a.e_t = f.e.e_out;
+    a.Pa = f.e.Pa;
+    a.Pb = f.e.Pb;
+    a.y2_t = f.e.y2_out;
+    a.parts1 = f.e.parts1;
+    a.parts2 = f.e.parts2;
+    a.tprev_parts = j.e.prev_parts;
+    a.tbase = j.e.base;
+    a.typrev = j.e.yprev;
+    a.te_out = j.e.e_out;  // ed_t is read again only by the next step
+    a.tPa = j.e.Pa;
+    a.tPb = j.e.Pb;
+    a.ty2_out = j.e.y2_out;
+    a.taggraw = j.e.aggraw;
+    a.tparts1 = j.e.parts1;
+    a.tparts2 = j.e.parts2;
     a.recv = recv;
     a.send = send;
     a.rowptr = rowptr;
-    a.WtE = pk + PackOffsets::PE_WET;
-    a.b1 = P[PE_B0];
-    a.Wt2 = pk + PackOffsets::PE_W2T;
-    a.b2 = P[PE_B2];
-    a.count = cnt_e;
+    a.WtE = f.e.WtE;
+    a.b1 = f.e.b1;
+    a.Wt2 = f.e.Wt2;
+    a.b2 = f.e.b2;
+    a.count = f.e.prev_count;
     a.E = E;
     a.n_tiles = nt_e;
     a.tws = tws;
@@ -856,25 +810,25 @@ extern "C" int pdg_jvp_batched(const pdg_params_t* params, const pdg_norm_t* nor
     a.C = C;
     {
       ScopedTimer tm_(KC_JVP_EDGE_STEP, st);
-      k_edge_step_jvp<<<dim3(grid_e, groups), NT, smem_edge, st>>>(a);
+      if (launch_named("k_edge_step_jvp", false, k_edge_step_jvp, dim3(grid_e, groups), dim3(NT), smem_edge, st, a)) return -2;
     }
     PDG_LAUNCH_CHECK();
     {
       ScopedTimer tm_(KC_JVP_NODE_UPD, st);
-      k_node_update_jvp<<<gn, NT, SMEM_J2A, st>>>(F.aggraw_[t], J.aggraw_[t], rowptr, F.parts_slot(slot_ln1(t)),
-                                                  J.parts_slot(slot_ln1(t)), cnt_e, P[PE_LNW], J.x_[t],
-                                                  pk + PackOffsets::PN_WAT, pk + PackOffsets::PN_WXT, F.hq_[t],
-                                                  pk + PackOffsets::PN_W2T, F.y3_[t], F.parts_slot(slot_ln3(t)), cnt_n,
-                                                  J.y3_[t], J.parts_slot(slot_ln3(t)), N, nt_n, tws);
+      if (launch_named("k_node_update_jvp", false, k_node_update_jvp, gn, dim3(NT), SMEM_2A, st, f.u.aggraw, j.u.aggraw, rowptr,
+                       f.u.parts1, j.u.parts1, f.u.count1, f.u.lnw_e, j.u.x_t, pk + PackOffsets::PN_WAT,
+                       pk + PackOffsets::PN_WXT, f.u.hq_out, pk + PackOffsets::PN_W2T, f.u.y3_out, f.u.parts3, cnt_n, j.u.y3_out,
+                       j.u.parts3, N, nt_n, tws)) return -2;
     }
     PDG_LAUNCH_CHECK();
   }
+  const DecArgs fd = fwd_dec_args(F, P), jd = fwd_dec_args(J, P);
   const bool scale_out = (flags & PDG_FLAG_SCALE_OUTPUT) != 0;
   {
     ScopedTimer tm_(KC_JVP_DECODER, st);
-    k_decoder_jvp<<<gn, NT, SMEM_J1A, st>>>(F.y3_[T - 1], F.parts_slot(slot_ln3(T - 1)), J.parts_slot(slot_ln3(T - 1)), cnt_n,
-                                            P[PN_LNW], J.x_[T - 1], J.y3_[T - 1], pk + PackOffsets::ND_W0T, F.hd, P[ND_W2],
-                                            scale_out ? norm->std_local_stress : 1.f, tan_local_stress, nzflag, N, nt_n, tws);
+    if (launch_named("k_decoder_jvp", false, k_decoder_jvp, gn, dim3(NT), SMEM_1A, st, fd.yprev, fd.prev_parts, jd.prev_parts,
+                     fd.prev_count, fd.lnw, jd.base, jd.yprev, pk + PackOffsets::ND_W0T, fd.hd_out, fd.D2,
+                     scale_out ? norm->std_local_stress : 1.f, tan_local_stress, nzflag, N, nt_n, tws)) return -2;
   }
   PDG_LAUNCH_CHECK();
   return 0;

@@ -601,12 +601,8 @@ extern "C" int pdg_phase_read3(unsigned long long* out32) {
 #endif
 
 int launch_edge_step_bwd_tc3(const EdgeBwdArgs& a, const uint8_t* img, int grid, cudaStream_t st) {
-  cudaError_t e = cudaFuncSetAttribute((const void*)k_edge_step_bwd_tc3, cudaFuncAttributeMaxDynamicSharedMemorySize, TC_SMEM_EDGE_BWD3);
-  if (e != cudaSuccess) { set_error("k_edge_step_bwd_tc3 smem attribute: %s", cudaGetErrorString(e)); return -2; }
-  e = launch_pdl(k_edge_step_bwd_tc3, dim3(grid), dim3(NT_B3), TC_SMEM_EDGE_BWD3, st, a, img + (size_t)IMG_PE_WE * tc::TILE_BF16_BYTES,
-                 img + (size_t)IMG_PE_W2 * tc::TILE_BF16_BYTES);
-  if (e != cudaSuccess) { set_error("k_edge_step_bwd_tc3 launch: %s", cudaGetErrorString(e)); return -2; }
-  return 0;
+  return launch_named("k_edge_step_bwd_tc3", true, k_edge_step_bwd_tc3, dim3(grid), dim3(NT_B3), TC_SMEM_EDGE_BWD3, st, a,
+                      weight_img(img, IMG_PE_WE), weight_img(img, IMG_PE_W2));
 }
 
 }  // namespace pdg

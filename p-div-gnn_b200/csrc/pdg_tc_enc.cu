@@ -271,30 +271,20 @@ k_edge_encoder_bwd_tc(EdgeEncBwdArgs a, const uint8_t* __restrict__ imgW2) {
 int launch_edge_encoder_tc(const float* edge_attr, const int32_t* perm, const pdg_norm_t* nrm, int scale_in, const float* W0,
                            const float* b0, const float* b2, float* y_out, double* parts, int E, int n_tiles,
                            const uint8_t* img, cudaStream_t st) {
-  cudaError_t e = cudaFuncSetAttribute((const void*)k_edge_encoder_tc, cudaFuncAttributeMaxDynamicSharedMemorySize, TC_SMEM_EDGE_ENC);
-  if (e != cudaSuccess) { set_error("k_edge_encoder_tc smem attribute: %s", cudaGetErrorString(e)); return -2; }
   EdgeEncArgs a{edge_attr, perm, nrm->mean_edge_weight, nrm->std_edge_weight, scale_in, W0, b0, b2, y_out, parts, E, n_tiles};
   const int cap = 2 * num_sms() < MAXP ? 2 * num_sms() : MAXP;
-  e = launch_pdl(k_edge_encoder_tc, dim3(n_tiles < cap ? n_tiles : cap), dim3(NT), TC_SMEM_EDGE_ENC, st, a,
-                 img + (size_t)IMG_EE_W2 * tc::TILE_BF16_BYTES);
-  if (e != cudaSuccess) { set_error("k_edge_encoder_tc launch: %s", cudaGetErrorString(e)); return -2; }
-  return 0;
+  return launch_named("k_edge_encoder_tc", true, k_edge_encoder_tc, dim3(n_tiles < cap ? n_tiles : cap), dim3(NT), TC_SMEM_EDGE_ENC, st,
+                      a, weight_img(img, IMG_EE_W2));
 }
 int launch_edge_encoder_bwd_tc(const float* g_in, const float* y_raw, const float* scal, const float* lnw, const float* edge_attr,
                                const int32_t* perm, const pdg_norm_t* nrm, int scale_in, const float* W0, const float* b0,
                                float* cta_grads, const float* gs, float* grad_edge_attr, int E, int n_tiles, int grid,
                                const uint8_t* img, cudaStream_t st) {
   const bool ig = grad_edge_attr != nullptr;
-  const void* fn = ig ? (const void*)k_edge_encoder_bwd_tc<true> : (const void*)k_edge_encoder_bwd_tc<false>;
-  const int smem = ig ? TC_SMEM_EDGE_ENC_BWD_IG : TC_SMEM_EDGE_ENC_BWD;
-  cudaError_t e = cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
-  if (e != cudaSuccess) { set_error("k_edge_encoder_bwd_tc smem attribute: %s", cudaGetErrorString(e)); return -2; }
   EdgeEncBwdArgs a{g_in, y_raw, scal, lnw, edge_attr, perm, nrm->mean_edge_weight, nrm->std_edge_weight, scale_in, W0, b0, cta_grads,
                    gs, grad_edge_attr, E, n_tiles};
-  e = launch_pdl(ig ? k_edge_encoder_bwd_tc<true> : k_edge_encoder_bwd_tc<false>, dim3(grid), dim3(NT), smem, st, a,
-                 img + (size_t)IMG_EE_W2 * tc::TILE_BF16_BYTES);
-  if (e != cudaSuccess) { set_error("k_edge_encoder_bwd_tc launch: %s", cudaGetErrorString(e)); return -2; }
-  return 0;
+  return launch_named("k_edge_encoder_bwd_tc", true, ig ? k_edge_encoder_bwd_tc<true> : k_edge_encoder_bwd_tc<false>, dim3(grid),
+                      dim3(NT), ig ? TC_SMEM_EDGE_ENC_BWD_IG : TC_SMEM_EDGE_ENC_BWD, st, a, weight_img(img, IMG_EE_W2));
 }
 
 }  // namespace pdg

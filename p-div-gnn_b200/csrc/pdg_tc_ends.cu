@@ -36,22 +36,6 @@ __device__ __forceinline__ void chunk8_flush(const float (&v)[8], float* scr, fl
     dst[threadIdx.x] = add ? dst[threadIdx.x] + s : s;
   }
 }
-// the six standardised node features of one row (models.py:140-152); nz = any raw mean-stress entry non-zero
-__device__ __forceinline__ void node_features(const float* __restrict__ mean_stress, const float* __restrict__ pos,
-                                              const int64_t* __restrict__ types, const pdg_norm_t& nrm, int scale_in, int row,
-                                              float (&f)[6], bool& nz) {
-  float m0 = mean_stress[row * 3 + 0], m1 = mean_stress[row * 3 + 1], m2 = mean_stress[row * 3 + 2];
-  float p0 = pos[row * 2 + 0], p1 = pos[row * 2 + 1];
-  nz = m0 != 0.f || m1 != 0.f || m2 != 0.f;
-  if (scale_in) {
-    m0 = (m0 - nrm.mean_mean_stress) / nrm.std_mean_stress;
-    m1 = (m1 - nrm.mean_mean_stress) / nrm.std_mean_stress;
-    m2 = (m2 - nrm.mean_mean_stress) / nrm.std_mean_stress;
-    p0 = (p0 - nrm.mean_pos) / nrm.std_pos;
-    p1 = (p1 - nrm.mean_pos) / nrm.std_pos;
-  }
-  f[0] = m0; f[1] = m1; f[2] = m2; f[3] = p0; f[4] = p1; f[5] = (float)types[row];
-}
 
 // ------------------------------------------------------------------------------------------------
 struct NodeEncArgs {
@@ -374,23 +358,6 @@ k_node_encoder_bwd_tc(NodeEncBwdArgs a, const uint8_t* __restrict__ imgW2) {
 }
 
 // ------------------------------------------------------------------------------------------------
-struct DecArgs {
-  const float* base;
-  const float* yprev;
-  const double* prev_parts;
-  double prev_count;
-  const float* lnw;
-  const float* lnb;
-  float* x_out;   // nullable
-  const float* d1;
-  const float* D2;  // [3][128]
-  const float* d2;  // [3]
-  float* hd_out;  // nullable, fp32 [N_pad][128]
-  float out_scale, out_shift;
-  float* out;     // [N][3]
-  const int* nzflag;
-  int N, n_tiles;
-};
 constexpr int TC_SMEM_DEC = 2 * tc::TILE_BF16_BYTES + 4 * H * 4 + 2 * TM * 4 * 4 + 512 + 2048;
 
 __global__ void __launch_bounds__(NT, 1)
@@ -645,24 +612,12 @@ k_decoder_bwd_tc(DecBwdArgs a, const uint8_t* __restrict__ imgD1) {
 }
 
 // ------------------------------------------------------------------------------------------------
-static int ends_launch(cudaError_t e, const char* name) {
-  if (e != cudaSuccess) { set_error("%s launch: %s", name, cudaGetErrorString(e)); return -2; }
-  return 0;
-}
-static int ends_attr(const void* fn, int bytes, const char* name) {
-  cudaError_t e = cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes);
-  if (e != cudaSuccess) { set_error("%s smem attribute: %s", name, cudaGetErrorString(e)); return -2; }
-  return 0;
-}
-static const uint8_t* ends_img(const uint8_t* img, int which) { return img + (size_t)which * tc::TILE_BF16_BYTES; }
-
 int launch_node_encoder_tc(const float* mean_stress, const float* pos, const int64_t* types, const pdg_norm_t* nrm, int scale_in,
                            const float* W0, const float* b0, const float* b2, float* y_out, double* parts, int* nzflag, int N,
                            int n_tiles, int grid, const uint8_t* img, cudaStream_t st) {
-  if (ends_attr((const void*)k_node_encoder_tc, TC_SMEM_NODE_ENC, "k_node_encoder_tc")) return -2;
   NodeEncArgs a{mean_stress, pos, types, *nrm, scale_in, W0, b0, b2, y_out, parts, nzflag, N, n_tiles};
-  return ends_launch(launch_pdl(k_node_encoder_tc, dim3(grid), dim3(NT), TC_SMEM_NODE_ENC, st, a, ends_img(img, IMG_NE_W2)),
-                     "k_node_encoder_tc");
+  return launch_named("k_node_encoder_tc", true, k_node_encoder_tc, dim3(grid), dim3(NT), TC_SMEM_NODE_ENC, st, a,
+                      weight_img(img, IMG_NE_W2));
 }
 int launch_node_encoder_bwd_tc(const float* g_in, const float* y_raw, const float* scal, const float* lnw, const float* mean_stress,
                                const float* pos, const int64_t* types, const pdg_norm_t* nrm, int scale_in, const float* W0,
@@ -670,30 +625,19 @@ int launch_node_encoder_bwd_tc(const float* g_in, const float* y_raw, const floa
                                int n_tiles, int grid, const uint8_t* img, cudaStream_t st) {
   NodeEncBwdArgs a{g_in, y_raw, scal, lnw, mean_stress, pos, types, *nrm, scale_in, W0, b0, cta_grads, gs, grad_mean_stress, grad_pos,
                    N, n_tiles};
-  if (grad_mean_stress != nullptr || grad_pos != nullptr) {
-    if (ends_attr((const void*)k_node_encoder_bwd_tc<true>, TC_SMEM_NODE_ENC_BWD_IG, "k_node_encoder_bwd_tc")) return -2;
-    return ends_launch(launch_pdl(k_node_encoder_bwd_tc<true>, dim3(grid), dim3(NT), TC_SMEM_NODE_ENC_BWD_IG, st, a,
-                                  ends_img(img, IMG_NE_W2)), "k_node_encoder_bwd_tc");
-  }
-  if (ends_attr((const void*)k_node_encoder_bwd_tc<false>, TC_SMEM_NODE_ENC_BWD, "k_node_encoder_bwd_tc")) return -2;
-  return ends_launch(launch_pdl(k_node_encoder_bwd_tc<false>, dim3(grid), dim3(NT), TC_SMEM_NODE_ENC_BWD, st, a, ends_img(img, IMG_NE_W2)),
-                     "k_node_encoder_bwd_tc");
+  const bool ig = grad_mean_stress != nullptr || grad_pos != nullptr;
+  return launch_named("k_node_encoder_bwd_tc", true, ig ? k_node_encoder_bwd_tc<true> : k_node_encoder_bwd_tc<false>, dim3(grid),
+                      dim3(NT), ig ? TC_SMEM_NODE_ENC_BWD_IG : TC_SMEM_NODE_ENC_BWD, st, a, weight_img(img, IMG_NE_W2));
 }
-int launch_decoder_tc(const float* base, const float* yprev, const double* prev_parts, double prev_count, const float* lnw,
-                      const float* lnb, float* x_out, const float* d1, const float* D2, const float* d2, float* hd_out,
-                      float out_scale, float out_shift, float* out, const int* nzflag, int N, int n_tiles, int grid,
-                      const uint8_t* img, cudaStream_t st) {
-  if (ends_attr((const void*)k_decoder_tc, TC_SMEM_DEC, "k_decoder_tc")) return -2;
-  DecArgs a{base, yprev, prev_parts, prev_count, lnw, lnb, x_out, d1, D2, d2, hd_out, out_scale, out_shift, out, nzflag, N, n_tiles};
-  return ends_launch(launch_pdl(k_decoder_tc, dim3(grid), dim3(NT), TC_SMEM_DEC, st, a, ends_img(img, IMG_ND_W0)), "k_decoder_tc");
+int launch_decoder_tc(const DecArgs& a, const uint8_t* img, int grid, cudaStream_t st) {
+  return launch_named("k_decoder_tc", true, k_decoder_tc, dim3(grid), dim3(NT), TC_SMEM_DEC, st, a, weight_img(img, IMG_ND_W0));
 }
 int launch_decoder_bwd_tc(const float* g_out, float gscale, const float* gs, const float* hd, const float* x_T, const float* y3_last,
                           const double* parts_prev, double count_prev, const float* D2, float* gx, float* cta_grads, float* cs3,
                           const int* nzflag, int N, int n_tiles, int grid, const uint8_t* img, cudaStream_t st) {
-  if (ends_attr((const void*)k_decoder_bwd_tc, TC_SMEM_DEC_BWD, "k_decoder_bwd_tc")) return -2;
   DecBwdArgs a{g_out, gscale, gs, hd, x_T, y3_last, parts_prev, count_prev, D2, gx, cta_grads, cs3, nzflag, N, n_tiles};
-  return ends_launch(launch_pdl(k_decoder_bwd_tc, dim3(grid), dim3(NT), TC_SMEM_DEC_BWD, st, a, ends_img(img, IMG_ND_W0)),
-                     "k_decoder_bwd_tc");
+  return launch_named("k_decoder_bwd_tc", true, k_decoder_bwd_tc, dim3(grid), dim3(NT), TC_SMEM_DEC_BWD, st, a,
+                      weight_img(img, IMG_ND_W0));
 }
 
 }  // namespace pdg

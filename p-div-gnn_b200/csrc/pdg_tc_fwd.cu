@@ -403,12 +403,8 @@ extern "C" int pdg_phase_read_fwd(unsigned long long* out32) {
 #endif
 
 int launch_edge_step_tc(const EdgeStepArgs& a, const uint8_t* img, int grid, cudaStream_t st) {
-  cudaError_t e = cudaFuncSetAttribute((const void*)k_edge_step_tc, cudaFuncAttributeMaxDynamicSharedMemorySize, TC_SMEM_EDGE);
-  if (e != cudaSuccess) { set_error("k_edge_step_tc smem attribute: %s", cudaGetErrorString(e)); return -2; }
-  e = launch_pdl(k_edge_step_tc, dim3(grid), dim3(NT_FWD), TC_SMEM_EDGE, st, a, img + (size_t)IMG_PE_WE * tc::TILE_BF16_BYTES,
-                 img + (size_t)IMG_PE_W2 * tc::TILE_BF16_BYTES);
-  if (e != cudaSuccess) { set_error("k_edge_step_tc launch: %s", cudaGetErrorString(e)); return -2; }
-  return 0;
+  return launch_named("k_edge_step_tc", true, k_edge_step_tc, dim3(grid), dim3(NT_FWD), TC_SMEM_EDGE, st, a,
+                      weight_img(img, IMG_PE_WE), weight_img(img, IMG_PE_W2));
 }
 
 }  // namespace pdg

@@ -824,37 +824,22 @@ extern "C" int pdg_phase_read_node(unsigned long long* out64) {
 #endif
 
 // ------------------------------------------------------------------------------------------------
-static int set_attr(const void* fn, int bytes, const char* name) {
-  cudaError_t e = cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes);
-  if (e != cudaSuccess) { set_error("%s smem attribute: %s", name, cudaGetErrorString(e)); return -2; }
-  return 0;
-}
-static const uint8_t* im(const uint8_t* img, int which) { return img + (size_t)which * tc::TILE_BF16_BYTES; }
-static int launch_check(cudaError_t e, const char* name) {
-  if (e != cudaSuccess) { set_error("%s launch: %s", name, cudaGetErrorString(e)); return -2; }
-  return 0;
-}
-
 int launch_node_pre_tc(const NodePreArgs& a, const uint8_t* img, int n_tiles, cudaStream_t st) {
-  if (set_attr((const void*)k_node_pre_tc, TC_SMEM_NODE_PRE, "k_node_pre_tc")) return -2;
   const int cap = 2 * num_sms();
-  return launch_check(launch_pdl(k_node_pre_tc, dim3(n_tiles < cap ? n_tiles : cap), dim3(NT), TC_SMEM_NODE_PRE, st, a, im(img, IMG_PE_WA),
-                                 im(img, IMG_PE_WB)), "k_node_pre_tc");
+  return launch_named("k_node_pre_tc", true, k_node_pre_tc, dim3(n_tiles < cap ? n_tiles : cap), dim3(NT), TC_SMEM_NODE_PRE, st, a,
+                      weight_img(img, IMG_PE_WA), weight_img(img, IMG_PE_WB));
 }
 int launch_node_update_tc(const NodeUpdArgs& a, const uint8_t* img, int grid, cudaStream_t st) {
-  if (set_attr((const void*)k_node_update_tc, TC_SMEM_NODE_UPD, "k_node_update_tc")) return -2;
-  return launch_check(launch_pdl(k_node_update_tc, dim3(grid), dim3(NT), TC_SMEM_NODE_UPD, st, a, im(img, IMG_PN_WA), im(img, IMG_PN_WX),
-                                 im(img, IMG_PN_W2)), "k_node_update_tc");
+  return launch_named("k_node_update_tc", true, k_node_update_tc, dim3(grid), dim3(NT), TC_SMEM_NODE_UPD, st, a,
+                      weight_img(img, IMG_PN_WA), weight_img(img, IMG_PN_WX), weight_img(img, IMG_PN_W2));
 }
 int launch_node_update_bwd_tc(const NodeUpdBwdArgs& a, const uint8_t* img, int grid, cudaStream_t st) {
-  if (set_attr((const void*)k_node_update_bwd_tc, TC_SMEM_NODE_UPD_BWD, "k_node_update_bwd_tc")) return -2;
-  return launch_check(launch_pdl(k_node_update_bwd_tc, dim3(grid), dim3(NT), TC_SMEM_NODE_UPD_BWD, st, a, im(img, IMG_PN_WA),
-                                 im(img, IMG_PN_WX), im(img, IMG_PN_W2)), "k_node_update_bwd_tc");
+  return launch_named("k_node_update_bwd_tc", true, k_node_update_bwd_tc, dim3(grid), dim3(NT), TC_SMEM_NODE_UPD_BWD, st, a,
+                      weight_img(img, IMG_PN_WA), weight_img(img, IMG_PN_WX), weight_img(img, IMG_PN_W2));
 }
 int launch_node_pre_bwd_tc(const NodePreBwdArgs& a, const uint8_t* img, int grid, cudaStream_t st) {
-  if (set_attr((const void*)k_node_pre_bwd_tc, TC_SMEM_NODE_PRE_BWD, "k_node_pre_bwd_tc")) return -2;
-  return launch_check(launch_pdl(k_node_pre_bwd_tc, dim3(grid), dim3(NT), TC_SMEM_NODE_PRE_BWD, st, a, im(img, IMG_PE_WA),
-                                 im(img, IMG_PE_WB)), "k_node_pre_bwd_tc");
+  return launch_named("k_node_pre_bwd_tc", true, k_node_pre_bwd_tc, dim3(grid), dim3(NT), TC_SMEM_NODE_PRE_BWD, st, a,
+                      weight_img(img, IMG_PE_WA), weight_img(img, IMG_PE_WB));
 }
 
 }  // namespace pdg

@@ -357,8 +357,9 @@ extern "C" int pdg_vjp_batched(const pdg_params_t* params, const pdg_norm_t* nor
     ScopedTimer tm_(KC_VJP_DECODER, st);
     const int* nzf = (flags & PDG_FLAG_ZERO_CHECK) ? W.nzflag : nullptr;
     const float gscale = (flags & PDG_FLAG_SCALE_OUTPUT) ? norm->std_local_stress : 1.f;
-    k_decoder_vjp<<<gn, NT, SMEM_V2T, st>>>(grad_local_stress, gscale, W.hd, W.y3_[T - 1], W.parts_slot(slot_ln3(T - 1)), cnt_n,
-                                            P[ND_W0], P[ND_W2], V.gx, V.cs3, nzf, N, nt_n, cws);
+    const DecArgs d = fwd_dec_args(W, P);  // what the forward's decoder read and saved
+    k_decoder_vjp<<<gn, NT, SMEM_V2T, st>>>(grad_local_stress, gscale, d.hd_out, d.yprev, d.prev_parts, d.prev_count, P[ND_W0],
+                                            d.D2, V.gx, V.cs3, nzf, N, nt_n, cws);
   }
   PDG_LAUNCH_CHECK();
   // receiver-side segment sums RA / RB (adjacent) of every cotangent start from zero: one strided memset

@@ -13,6 +13,8 @@ static inline int slot_ln3(int t) { return 4 + 3 * t; }
 
 // fp16 operand images kept in the forward workspace (tcgen05 path)
 enum ImgIdx { IMG_PE_WE = 0, IMG_PE_W2, IMG_PE_WA, IMG_PE_WB, IMG_PN_WA, IMG_PN_WX, IMG_PN_W2, IMG_EE_W2, IMG_NE_W2, IMG_ND_W0, IMG_COUNT };
+constexpr size_t IMG_BYTES = 32768;  // one image: a 128 x 128 fp16 operand tile
+static inline const uint8_t* weight_img(const uint8_t* img, int which) { return img + (size_t)which * IMG_BYTES; }
 
 struct EdgeStepArgs {
   const float* base;
@@ -162,10 +164,25 @@ int launch_node_encoder_bwd_tc(const float* g_in, const float* y_raw, const floa
                                const float* pos, const int64_t* types, const pdg_norm_t* nrm, int scale_in, const float* W0,
                                const float* b0, float* cta_grads, const float* gs, float* grad_mean_stress, float* grad_pos, int N,
                                int n_tiles, int grid, const uint8_t* img, cudaStream_t st);
-int launch_decoder_tc(const float* base, const float* yprev, const double* prev_parts, double prev_count, const float* lnw,
-                      const float* lnb, float* x_out, const float* d1, const float* D2, const float* d2, float* hd_out,
-                      float out_scale, float out_shift, float* out, const int* nzflag, int N, int n_tiles, int grid,
-                      const uint8_t* img, cudaStream_t st);
+// decoder: x_T = x_{T-1} + LN(y3_{T-1}); node_decoder
+struct DecArgs {
+  const float* base;
+  const float* yprev;
+  const double* prev_parts;
+  double prev_count;
+  const float* lnw;
+  const float* lnb;
+  float* x_out;   // nullable
+  const float* d1;
+  const float* D2;  // [3][128]
+  const float* d2;  // [3]
+  float* hd_out;  // nullable, fp32 [N_pad][128]
+  float out_scale, out_shift;
+  float* out;     // [N][3]
+  const int* nzflag;
+  int N, n_tiles;
+};
+int launch_decoder_tc(const DecArgs& a, const uint8_t* img, int grid, cudaStream_t st);
 int launch_decoder_bwd_tc(const float* g_out, float gscale, const float* gs, const float* hd, const float* x_T, const float* y3_last,
                           const double* parts_prev, double count_prev, const float* D2, float* gx, float* cta_grads, float* cs3,
                           const int* nzflag, int N, int n_tiles, int grid, const uint8_t* img, cudaStream_t st);
@@ -223,7 +240,7 @@ struct FwdWs {
     const size_t eh = (size_t)E_pad * H * 2;  // fp16 rows / operand-tile images
     for (int t = 0; t < 64; ++t) eimg_[t] = nullptr;
     pack = (float*)take(PackOffsets::TOTAL * sizeof(float));
-    img = (uint8_t*)take((size_t)IMG_COUNT * 32768);
+    img = (uint8_t*)take(IMG_COUNT * IMG_BYTES);
     parts = (double*)take((size_t)(2 + 3 * T) * MAXP * 2 * sizeof(double));
     nzflag = (int*)take(256);
     y_nenc = (float*)take(nb);
@@ -267,5 +284,55 @@ struct FwdWs {
   }
   double* parts_slot(int s) const { return parts + (size_t)s * MAXP * 2; }
 };
+
+// What forward step t of W reads and writes: the node_pre, edge-step and node_update arguments, from W, the parameters P
+// and the plan's receiver / sender views.  Step 0 starts from the encoders' raw outputs; the last step skips the edge
+// update (nothing reads it), and e_t leaves only where the next step or, with `save`, the backward reads it.  A tangent
+// workspace (a forward workspace without `save`) gives the tangent pass its pointers the same way.  Left to the caller
+// are the fields of the 16-bit mode alone: the operand images, node_pre's aggraw_zero and b1, and its e_out rule.
+struct FwdStepArgs {
+  NodePreArgs np;
+  EdgeStepArgs e;
+  NodeUpdArgs u;
+};
+inline FwdStepArgs fwd_step_args(const FwdWs& W, const float* const* P, const int32_t* recv, const int32_t* send,
+                                 const int32_t* rowptr, int t) {
+  const bool first = t == 0, last = t == W.T - 1;
+  const int N = (int)W.N, E = (int)W.E, nt_n = (int)(W.N_pad / TM), nt_e = (int)(W.E_pad / TM);
+  const double cnt_n = (double)N * H, cnt_e = (double)E * H;
+  FwdStepArgs s = {};
+  NodePreArgs& np = s.np;
+  np.base = first ? nullptr : W.x_[t - 1]; np.yprev = first ? W.y_nenc : W.y3_[t - 1];
+  np.prev_parts = W.parts_slot(first ? 0 : slot_ln3(t - 1)); np.prev_count = cnt_n;
+  np.lnw = first ? P[NE_LNW] : P[PN_LNW]; np.lnb = first ? P[NE_LNB] : P[PN_LNB];
+  np.x_out = W.x_[t]; np.Pa = W.Pa_[t]; np.Pb = W.Pb_[t]; np.n_tiles = nt_n;
+  EdgeStepArgs& e = s.e;
+  e.base = first ? nullptr : W.e_[t - 1]; e.yprev = first ? W.y_eenc : W.y2_[t - 1];
+  e.prev_parts = W.parts_slot(first ? 1 : slot_ln2(t - 1)); e.prev_count = cnt_e;
+  e.prev_w = first ? P[EE_LNW] : P[PE_LNW]; e.prev_b = first ? P[EE_LNB] : P[PE_LNB];
+  e.e_out = (W.save || !last) ? W.e_[t] : nullptr;
+  e.Pa = W.Pa_[t]; e.Pb = W.Pb_[t]; e.recv = recv; e.send = send; e.rowptr = rowptr;
+  e.WtE = W.pack + PackOffsets::PE_WET; e.b1 = P[PE_B0]; e.Wt2 = W.pack + PackOffsets::PE_W2T; e.b2 = P[PE_B2];
+  e.y2_out = last ? nullptr : W.y2_[t]; e.aggraw = W.aggraw_[t];
+  e.parts1 = W.parts_slot(slot_ln1(t)); e.parts2 = last ? nullptr : W.parts_slot(slot_ln2(t));
+  e.E = E; e.n_tiles = nt_e;
+  NodeUpdArgs& u = s.u;
+  u.aggraw = W.aggraw_[t]; u.rowptr = rowptr; u.parts1 = W.parts_slot(slot_ln1(t)); u.count1 = cnt_e;
+  u.lnw_e = P[PE_LNW]; u.lnb_e = P[PE_LNB]; u.x_t = W.x_[t]; u.c1 = P[PN_B0]; u.c2 = P[PN_B2];
+  u.hq_out = W.save ? W.hq_[t] : nullptr; u.y3_out = W.y3_[t]; u.parts3 = W.parts_slot(slot_ln3(t));
+  u.N = N; u.n_tiles = nt_n;
+  return s;
+}
+// The decoder's inputs after the last step; x_T and the hidden layer leave only with `save`.  The output, its scale and
+// the zero-load flag are the caller's.
+inline DecArgs fwd_dec_args(const FwdWs& W, const float* const* P) {
+  const int T = W.T;
+  DecArgs d = {};
+  d.base = W.x_[T - 1]; d.yprev = W.y3_[T - 1]; d.prev_parts = W.parts_slot(slot_ln3(T - 1)); d.prev_count = (double)W.N * H;
+  d.lnw = P[PN_LNW]; d.lnb = P[PN_LNB]; d.x_out = W.save ? W.x_[T] : nullptr;
+  d.d1 = P[ND_B0]; d.D2 = P[ND_W2]; d.d2 = P[ND_B2]; d.hd_out = W.save ? W.hd : nullptr;
+  d.N = (int)W.N; d.n_tiles = (int)(W.N_pad / TM);
+  return d;
+}
 
 }  // namespace pdg
