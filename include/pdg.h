@@ -128,7 +128,7 @@ int pdg_forward(const pdg_params_t* params, const pdg_norm_t* norm, const float*
  * range.  Row k has the bits of pdg_forward on instance k's inputs with the same flags; with PDG_FLAG_ZERO_CHECK an
  * instance whose mean_stress is all zeros gives zeros whatever the others hold.  Launches the kernels and memsets of
  * one pdg_forward for any K.  Returns -1 for K outside 1..PDG_FWD_MAX_INSTANCES, precision != PDG_PREC_FP32,
- * PDG_FLAG_SAVE (no derivative follows a batched forward), steps outside 1..62, a negative stride, a workspace that is
+ * PDG_FLAG_SAVE (pdg_forward_batched_saved keeps the state for a derivative), steps outside 1..62, a negative stride, a workspace that is
  * too small and an empty graph.  Replaces torch.func.vmap over the inputs of models.py:288-326. */
 #define PDG_FWD_MAX_INSTANCES 64
 size_t pdg_forward_batched_ws_bytes(int64_t n_nodes, int64_t n_edges, int steps, int flags, int n_instances);
@@ -136,6 +136,19 @@ int pdg_forward_batched(const pdg_params_t* params, const pdg_norm_t* norm, cons
                         const float* pos, int64_t pos_stride, const int64_t* nodes_types, const float* edge_attr,
                         int64_t ea_stride, const void* plan, int64_t n_nodes, int64_t n_edges, int steps, int flags,
                         int precision, void* ws, size_t ws_bytes, int n_instances, float* local_stress, void* stream);
+/* The same forward keeping every instance's state for pdg_vjp_instances: flags must contain PDG_FLAG_SAVE.  Instance k's
+ * workspace is a full fp32 PDG_FLAG_SAVE forward workspace (the layout pdg_ws_offset describes) at byte offset
+ * k * pdg_forward_batched_saved_ws_bytes(n_nodes, n_edges, steps, flags, 1); the total is n_instances times that (0 for
+ * flags without PDG_FLAG_SAVE, K or steps out of range).  The kernels read the packed weights in instance 0's workspace;
+ * afterwards every instance's workspace holds a copy of them (log2(K) device copies), so an adjoint may be given the
+ * workspace from any instance on.
+ * Row k, and every saved tensor of instance k, has the bits of pdg_forward with PDG_FLAG_SAVE on instance k's inputs.
+ * Returns -1 for flags without PDG_FLAG_SAVE and for the other refusals of pdg_forward_batched. */
+size_t pdg_forward_batched_saved_ws_bytes(int64_t n_nodes, int64_t n_edges, int steps, int flags, int n_instances);
+int pdg_forward_batched_saved(const pdg_params_t* params, const pdg_norm_t* norm, const float* mean_stress, int64_t ms_stride,
+                              const float* pos, int64_t pos_stride, const int64_t* nodes_types, const float* edge_attr,
+                              int64_t ea_stride, const void* plan, int64_t n_nodes, int64_t n_edges, int steps, int flags,
+                              int precision, void* ws, size_t ws_bytes, int n_instances, float* local_stress, void* stream);
 
 /* test/debug: byte offset + element count of a saved tensor in a PDG_FLAG_SAVE workspace.
  * what: 0 x_t, 1 e_t, 2 y2_t, 3 Pa_t, 4 Pb_t, 5 aggraw_t, 6 hq_t, 7 y3_t, 8 y_nenc,
@@ -211,6 +224,26 @@ int pdg_vjp_batched(const pdg_params_t* params, const pdg_norm_t* norm, const fl
                     int64_t n_edges, int steps, int flags, int precision, const void* fwd_ws, void* vjp_ws,
                     size_t vjp_ws_bytes, int n_cotangents, const float* grad_local_stress, float* grad_mean_stress,
                     float* grad_pos, float* grad_edge_attr, void* stream);
+
+/* Reverse mode through the batched forward: n_cotangents M (>= 1) cotangents for each of n_instances I (1..
+ * PDG_FWD_MAX_INSTANCES) instances, I * M <= PDG_VJP_MAX_COTANGENTS, in one adjoint pass.  fwd_ws is the workspace of a
+ * pdg_forward_batched_saved of I instances with the same inputs, strides and flags; it is only read.  Cotangent (i, m)
+ * is grad_local_stress [I][M][N][3] row i * M + m and reads instance i's saved state and inputs.  fwd_ws may also start
+ * at any later instance j of such a workspace (fwd_ws + j * the single-instance bytes, inputs from instance j on): the
+ * packed weights are read from its first instance; the outputs are
+ * grad_mean_stress [I][M][N][3], grad_pos [I][M][N][2], grad_edge_attr [I][M][E] (caller's edge order; NULL: not
+ * formed).  An input shared by the instances (stride 0) still gets one row per (i, m): summing them is the caller's.
+ * vjp_ws: pdg_vjp_batched_ws_bytes(n_nodes, n_edges, steps, I * M).  Row (i, m) has the bits of pdg_vjp_batched with
+ * K = 1 (the input gradients of pdg_backward_inputs) on a pdg_forward with PDG_FLAG_SAVE of instance i and cotangent
+ * (i, m).  Launches the kernels of one pdg_vjp_batched for any I and M.  Returns -1 for I outside 1..PDG_FWD_MAX_INSTANCES,
+ * I * M > PDG_VJP_MAX_COTANGENTS, a negative stride and every refusal of pdg_vjp_batched.
+ * Replaces torch reverse-mode AD (torch.func.grad / vjp / jacrev) through torch.func.vmap over models.py:288-326. */
+int pdg_vjp_instances(const pdg_params_t* params, const pdg_norm_t* norm, const float* mean_stress, int64_t ms_stride,
+                      const float* pos, int64_t pos_stride, const int64_t* nodes_types, const float* edge_attr,
+                      int64_t ea_stride, const void* plan, int64_t n_nodes, int64_t n_edges, int steps, int flags,
+                      int precision, const void* fwd_ws, int n_instances, void* vjp_ws, size_t vjp_ws_bytes,
+                      int n_cotangents, const float* grad_local_stress, float* grad_mean_stress, float* grad_pos,
+                      float* grad_edge_attr, void* stream);
 
 /* ---- loss: per-graph NMSE + divergence regulariser, batch means ---------------------
  * Replaces the per-graph Python loop of train() (gnn_train.py:162-202):

@@ -60,6 +60,9 @@ _SIGS = {
     "pdg_forward_batched_ws_bytes": (_sz, [_i64, _i64, _i32, _i32, _i32]),
     "pdg_forward_batched": (_i32, [C.POINTER(PdgParams), C.POINTER(PdgNorm), _vp, _i64, _vp, _i64, _vp, _vp, _i64, _vp,
                                    _i64, _i64, _i32, _i32, _i32, _vp, _sz, _i32, _vp, _vp]),
+    "pdg_forward_batched_saved_ws_bytes": (_sz, [_i64, _i64, _i32, _i32, _i32]),
+    "pdg_forward_batched_saved": (_i32, [C.POINTER(PdgParams), C.POINTER(PdgNorm), _vp, _i64, _vp, _i64, _vp, _vp, _i64,
+                                         _vp, _i64, _i64, _i32, _i32, _i32, _vp, _sz, _i32, _vp, _vp]),
     "pdg_ws_offset": (_i32, [_i64, _i64, _i32, _i32, _i32, _i32, C.POINTER(_sz), C.POINTER(_sz)]),
     "pdg_backward_ws_bytes": (_sz, [_i64, _i64, _i32]),
     "pdg_backward": (_i32, [C.POINTER(PdgParams), C.POINTER(PdgNorm), _vp, _vp, _vp, _vp, _vp, _i64, _i64, _i32, _i32,
@@ -75,6 +78,8 @@ _SIGS = {
     "pdg_vjp_batched_ws_bytes": (_sz, [_i64, _i64, _i32, _i32]),
     "pdg_vjp_batched": (_i32, [C.POINTER(PdgParams), C.POINTER(PdgNorm), _vp, _vp, _vp, _vp, _vp, _i64, _i64, _i32, _i32,
                                _i32, _vp, _vp, _sz, _i32, _vp, _vp, _vp, _vp, _vp]),
+    "pdg_vjp_instances": (_i32, [C.POINTER(PdgParams), C.POINTER(PdgNorm), _vp, _i64, _vp, _i64, _vp, _vp, _i64, _vp,
+                                 _i64, _i64, _i32, _i32, _i32, _vp, _i32, _vp, _sz, _i32, _vp, _vp, _vp, _vp, _vp]),
     "pdg_opdiv_plan_bytes": (_sz, [_i64, _i64]),
     "pdg_opdiv_tmp_bytes": (_sz, [_i64, _i64]),
     "pdg_opdiv_plan_build": (_i32, [_vp, _vp, _i64, _vp, _i64, _i64, _vp, _vp, _sz, _vp]),

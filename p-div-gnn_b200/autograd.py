@@ -2,8 +2,8 @@
 
 Nothing here computes; it validates inputs, builds / caches the device graph plan,
 allocates the workspace from torch's caching allocator (so stream semantics hold) and
-calls ``pdg_forward`` / ``pdg_forward_batched`` / ``pdg_backward_inputs`` / ``pdg_jvp_batched`` / ``pdg_vjp_batched``
-on the current CUDA stream.
+calls ``pdg_forward`` / ``pdg_forward_batched`` / ``pdg_forward_batched_saved`` / ``pdg_backward_inputs`` /
+``pdg_jvp_batched`` / ``pdg_vjp_batched`` / ``pdg_vjp_instances`` on the current CUDA stream.
 """
 from __future__ import annotations
 
@@ -130,11 +130,13 @@ class _EPDFunction(torch.autograd.Function):
     """pdg_forward, pdg_backward_inputs (reverse mode), pdg_vjp_batched (vmapped reverse mode) and pdg_jvp (forward
     mode).  Written in setup_context style so that torch.func.jvp accepts it; the forward workspace reaches ctx as a
     second, non-differentiable output.  `swapped`: parameters other than the cached param_list were in the module
-    (torch.func.functional_call), so a gradient for them would never reach this Function."""
+    (torch.func.functional_call), so a gradient for them would never reach this Function.  `grad_level`: the innermost
+    torch.func level that tracks mean_stress, pos or edge_attr for a reverse-mode derivative (0: none, or plain
+    autograd); the vmap rule tells a derivative inside the vmap from one outside it by it."""
 
     @staticmethod
     def forward(model, plan, mean_stress, pos, types, edge_attr, flags, steps, prec, need_grad, need_tan, swapped,
-                *params):
+                grad_level, *params):
         L = _lib.lib()
         dev = mean_stress.device
         n, e = plan.n_nodes, plan.n_edges
@@ -154,7 +156,8 @@ class _EPDFunction(torch.autograd.Function):
 
     @staticmethod
     def setup_context(ctx, inputs, output):
-        model, plan, mean_stress, pos, types, edge_attr, flags, steps, prec, need_grad, need_tan, swapped, *params = inputs
+        model, plan, mean_stress, pos, types, edge_attr, flags, steps, prec, need_grad, need_tan, swapped, _, *params = \
+            inputs
         _, ws = output
         ctx.mark_non_differentiable(ws)
         # no zero gradient is materialised for the workspace output (a memset of the whole saved state per backward);
@@ -180,26 +183,44 @@ class _EPDFunction(torch.autograd.Function):
 
     @staticmethod
     def vmap(info, in_dims, model, plan, mean_stress, pos, types, edge_attr, flags, steps, prec, need_grad, need_tan,
-             swapped, *params):
+             swapped, grad_level, *params):
         """torch reaches this rule only when a model input or parameter is batched at this vmap level: with unbatched
         primals it skips the level, and batched tangents go to _EPDTangent.vmap.  Batched mean_stress, pos and
         edge_attr (one graph under many loads or shapes) run as instances of pdg_forward_batched: the vmapped dimension
-        moves to the front, unbatched inputs are shared (stride 0).  Inference only, fp32 only."""
-        if need_grad or need_tan:
+        moves to the front, unbatched inputs are shared (stride 0).  fp32 only.
+
+        A reverse-mode derivative taken outside the vmap (torch.func.grad / vjp / jacrev of a function that vmaps the
+        model, or autograd through the vmap) leaves the inputs under this level requiring grad (need_grad is False for
+        batched inputs, whose requires_grad reads False, and True for a shared input that requires grad): the instances
+        then keep their forward state (pdg_forward_batched_saved), and the outer level records _EPDInstances, whose
+        backward runs pdg_vjp_instances.  A derivative inside the vmap is tracked at a level inside this one
+        (grad_level above the level current in this rule) and is refused, whether or not the inputs under this level
+        also require grad for an outer derivative; so are forward mode and a trainable model."""
+        save = torch.is_grad_enabled() and any(_tracked(x) for x in (mean_stress, pos, edge_attr))
+        inside = grad_level > (torch._C._functorch.maybe_current_level() or 0)
+        if need_tan or (need_grad and (not save or inside or any(p.requires_grad for p in params))):
             raise NotImplementedError(
-                "pdivgnn_b200: vmap over mean_stress, pos or edge_attr runs the forward only (under torch.no_grad(), or "
-                "with a model whose parameters and inputs do not require grad); derivatives through it are not "
-                "implemented.  Derivatives at one input point are: batched tangents (torch.func.jacfwd, vmap over "
-                "torch.func.jvp) and batched cotangents (torch.func.jacrev, vmap over torch.func.vjp)")
+                "pdivgnn_b200: vmap over mean_stress, pos or edge_attr runs the forward only when the derivative is "
+                "taken inside the vmap (torch.func.vmap over grad, vjp, jacrev, jvp or jacfwd) or the model's "
+                "parameters require grad.  Reverse-mode derivatives taken outside the vmap work with a frozen model "
+                "(model.requires_grad_(False)): torch.func.grad, vjp or jacrev of a function that vmaps the model, or "
+                "autograd through the vmap.  Derivatives at one input point are: batched tangents (torch.func.jacfwd, "
+                "vmap over torch.func.jvp) and batched cotangents (torch.func.jacrev, vmap over torch.func.vjp)")
         if prec != _lib.PREC_FP32:
             raise NotImplementedError("pdivgnn_b200: vmap over the model's inputs needs precision='fp32'; in the 16-bit "
                                       "mode call the model once per input")
-        if any(d is not None for d in in_dims[12:]):
+        if any(d is not None for d in in_dims[13:]):
             raise NotImplementedError(_BATCHED_PARAMS)
         if in_dims[4] is not None:
             raise NotImplementedError("pdivgnn_b200: vmap over nodes_types is not implemented; the instances of one "
                                       "vmapped forward share the graph and its node types, and differ in mean_stress, "
                                       "pos and edge_attr")
+        if save and swapped:
+            raise NotImplementedError("pdivgnn_b200: reverse-mode derivatives through vmap over the model's inputs need "
+                                      "the model's own parameters; parameters swapped in by torch.func.functional_call "
+                                      "are not supported there")
+        if save:
+            flags |= _lib.FLAG_SAVE
         xs = [x if d is None else x.movedim(d, 0) for x, d in zip((mean_stress, pos, edge_attr), (in_dims[2], in_dims[3], in_dims[5]))]
         out, ws = _EPDInstances.apply((model, plan, types, flags, steps, params), *xs)
         return (out, ws), (0, None)
@@ -238,10 +259,10 @@ class _EPDFunction(torch.autograd.Function):
             allreduce_flat_(flat, dp[1], getattr(model, "_pdg_peer", None))
         grads, off = [], 0
         for i, p in enumerate(params):
-            grads.append(flat[off:off + p.numel()].view(p.shape) if need[12 + i] else None)
+            grads.append(flat[off:off + p.numel()].view(p.shape) if need[13 + i] else None)
             off += p.numel()
         ctx.pdg = None
-        return (None, None, g_ms, g_pos, None, g_ea) + (None,) * 6 + tuple(grads)
+        return (None, None, g_ms, g_pos, None, g_ea) + (None,) * 7 + tuple(grads)
 
     @staticmethod
     def _backward_batched(ctx, grad_out):
@@ -253,14 +274,14 @@ class _EPDFunction(torch.autograd.Function):
         if prec != _lib.PREC_FP32:
             raise NotImplementedError("pdivgnn_b200: batched reverse-mode derivatives (torch.func.jacrev, vmap over vjp) "
                                       "need precision='fp32'; the 16-bit mode's input gradients miss its 2e-2 tolerance")
-        if ctx.pdg_swapped or any(need[12:]):
+        if ctx.pdg_swapped or any(need[13:]):
             raise NotImplementedError("pdivgnn_b200: batched reverse-mode derivatives with respect to the parameters are "
                                       "not implemented (torch.func.jacrev or vmap over vjp of the parameters); those "
                                       "with respect to mean_stress, pos and edge_attr are")
         want = (need[2], need[3], need[5])
         outs = iter(_EPDAdjoint.apply(ctx.pdg, want, grad_out) if any(want) else ())
         g_ms, g_pos, g_ea = (next(outs) if w else None for w in want)
-        return (None, None, g_ms, g_pos, None, g_ea) + (None,) * (6 + len(ctx.pdg[9]))
+        return (None, None, g_ms, g_pos, None, g_ea) + (None,) * (7 + len(ctx.pdg[9]))
 
 
 class _EPDAdjoint(torch.autograd.Function):
@@ -314,6 +335,40 @@ def _tangent_shapes(state):
     return ((plan.n_nodes, 3), (plan.n_nodes, 2), (plan.n_edges,))
 
 
+def _tracked(t):
+    """requires_grad of t below its vmap levels: an input of a nested vmap rule is still batched at the outer levels,
+    and a BatchedTensor reports False whatever it wraps"""
+    while torch._C._functorch.is_batchedtensor(t):
+        t = torch._C._functorch.get_unwrapped(t)
+    return t.requires_grad
+
+
+def _grad_level(t):
+    """The innermost torch.func level at which t is tracked for a reverse-mode derivative: its innermost wrapper that is
+    not a vmap level and requires grad (0: none, or plain autograd only)"""
+    while torch._C._functorch.is_functorch_wrapped_tensor(t):
+        if not torch._C._functorch.is_batchedtensor(t) and t.requires_grad:
+            return torch._C._functorch.maybe_get_level(t)
+        t = torch._C._functorch.get_unwrapped(t)
+    return 0
+
+
+def _instance_args(state, xs):
+    """(K, [(tensor, element stride)] for mean_stress, pos, edge_attr) of pdg_forward_batched and pdg_vjp_instances.  An
+    input of its per-graph shape, or expanded over K (leading stride 0), is passed once with stride 0."""
+    shapes = _tangent_shapes(state)
+    k = next(x.shape[0] for x, s in zip(xs, shapes) if x.dim() == len(s) + 1)
+    args = []
+    for x, s, name in zip(xs, shapes, ("mean_stress", "pos", "edge_attr")):
+        stride = 0
+        if x.dim() == len(s) + 1 and x.stride(0) != 0:
+            x, stride = x.contiguous(), x[0].numel()
+        elif x.dim() == len(s) + 1:
+            x = x[0]
+        args.append((_lib.require_cuda(x, name, torch.float32), stride))
+    return k, args
+
+
 _BATCHED_PARAMS = ("pdivgnn_b200: vmap over the model's parameters (model ensembles through torch.func.functional_call) "
                    "is not implemented; vmap over mean_stress, pos and edge_attr is")
 
@@ -322,7 +377,13 @@ class _EPDInstances(torch.autograd.Function):
     """local_stress of K instances of one graph: pdg_forward_batched, one pass per at most FWD_MAX_INSTANCES instances.
     `state` is (model, plan, nodes_types, flags, steps, params).  An input is of its per-graph shape (the same for every
     instance) or [K, *shape], at least one of them the latter; returns local_stress [K, N, 3] and the workspace.  The
-    vmap rule folds the vmapped dimension into K.  Inference only: there is no backward."""
+    vmap rule folds the vmapped dimension into K.
+
+    Saving mode (PDG_FLAG_SAVE in the state's flags, set by _EPDFunction.vmap for a derivative taken outside the vmap):
+    pdg_forward_batched_saved, and the workspace keeps the saved forward of every instance (pass p's instances at their
+    own offset) until a backward with a plain cotangent, or for as long as the graph lives when the cotangents are
+    vmapped (jacrev, vmap over vjp).  local_stress is then differentiable; its backward forms the input gradients with
+    _EPDInstanceAdjoint (pdg_vjp_instances).  Without it, inference only."""
 
     @staticmethod
     def forward(state, mean_stress, pos, edge_attr):
@@ -330,34 +391,61 @@ class _EPDInstances(torch.autograd.Function):
         model, plan, types, flags, steps, params = state
         dev = types.device
         n, e = plan.n_nodes, plan.n_edges
-        xs, shapes = (mean_stress, pos, edge_attr), _tangent_shapes(state)
-        k = next(x.shape[0] for x, s in zip(xs, shapes) if x.dim() == len(s) + 1)
-        args = []
-        for x, s, name in zip(xs, shapes, ("mean_stress", "pos", "edge_attr")):
-            stride = 0
-            if x.dim() == len(s) + 1 and x.stride(0) != 0:
-                x, stride = x.contiguous(), x[0].numel()
-            elif x.dim() == len(s) + 1:
-                x = x[0]  # one input expanded over K: passed once, with stride 0
-            args.append((_lib.require_cuda(x, name, torch.float32), stride))
+        k, args = _instance_args(state, (mean_stress, pos, edge_attr))
+        save = bool(flags & _lib.FLAG_SAVE)
         cap = _lib.FWD_MAX_INSTANCES
         with torch.cuda.device(dev):
-            ws_bytes = L.pdg_forward_batched_ws_bytes(n, e, steps, flags, min(k, cap))
-            ws = torch.empty(_bucket(ws_bytes), dtype=torch.uint8, device=dev)  # reused by every pass (stream order)
+            if save:  # one saved workspace per instance, all kept
+                iws = L.pdg_forward_batched_saved_ws_bytes(n, e, steps, flags, 1)
+                ws = torch.empty(k * iws, dtype=torch.uint8, device=dev)
+            else:
+                ws_bytes = L.pdg_forward_batched_ws_bytes(n, e, steps, flags, min(k, cap))
+                ws = torch.empty(_bucket(ws_bytes), dtype=torch.uint8, device=dev)  # reused by every pass (stream order)
             out = torch.empty((k, n, 3), dtype=torch.float32, device=dev)
             ps, norm = _params_struct(params), model._norm_struct()
             for i in range(0, k, cap):
                 kk = min(cap, k - i)
                 xp = [_lib.ptr(x[i:i + kk] if st else x) for x, st in args]
-                _lib.check(L.pdg_forward_batched(C.byref(ps), C.byref(norm), xp[0], args[0][1], xp[1], args[1][1],
-                                                 _lib.ptr(types), xp[2], args[2][1], _lib.ptr(plan.buf), n, e, steps,
-                                                 flags, _lib.PREC_FP32, _lib.ptr(ws), ws_bytes, kk, _lib.ptr(out[i:i + kk]),
-                                                 _lib.stream_ptr(dev)), "pdg_forward_batched")
+                fn, name = (L.pdg_forward_batched_saved, "pdg_forward_batched_saved") if save else \
+                    (L.pdg_forward_batched, "pdg_forward_batched")
+                w, wb = (ws[i * iws:(i + kk) * iws], kk * iws) if save else (ws, ws_bytes)
+                _lib.check(fn(C.byref(ps), C.byref(norm), xp[0], args[0][1], xp[1], args[1][1], _lib.ptr(types), xp[2],
+                              args[2][1], _lib.ptr(plan.buf), n, e, steps, flags, _lib.PREC_FP32, _lib.ptr(w), wb, kk,
+                              _lib.ptr(out[i:i + kk]), _lib.stream_ptr(dev)), name)
         return out, ws
 
     @staticmethod
     def setup_context(ctx, inputs, output):
-        ctx.mark_non_differentiable(*output)
+        state, *xs = inputs
+        if not state[3] & _lib.FLAG_SAVE:
+            ctx.mark_non_differentiable(*output)
+            return
+        ctx.mark_non_differentiable(output[1])
+        ctx.set_materialize_grads(False)
+        ctx.pdg = (state, tuple(xs), output[1])
+
+    @staticmethod
+    def backward(ctx, grad_out, _grad_ws):
+        """Rows of every instance from _EPDInstanceAdjoint.  A batched input gets its rows in its own shape [K, ...] (an
+        input expanded over K too: autograd reduces them through the expand); an input shared by every instance gets
+        the sum of its rows.  After a plain cotangent the saved forwards are released, as _EPDFunction releases its
+        own; a vmapped one keeps them, since jacrev may call again (chunk_size)."""
+        if ctx.pdg is None:
+            raise RuntimeError("pdivgnn_b200: a second backward through the vmapped model: its saved forwards were "
+                               "released after the first one (retain_graph does not keep them); run the forward again")
+        state, xs, _ = ctx.pdg
+        want = tuple(ctx.needs_input_grad[1:4])
+        saved = ctx.pdg
+        if grad_out is None or not _lib.is_vmapped(grad_out):
+            ctx.pdg = None
+        if grad_out is None or not any(want):
+            return None, None, None, None
+        rows = iter(_EPDInstanceAdjoint.apply(saved, want, grad_out))
+        grads = []
+        for w, x, s in zip(want, xs, _tangent_shapes(state)):
+            g = next(rows) if w else None
+            grads.append(g.sum(0) if g is not None and x.dim() == len(s) else g)
+        return (None, *grads)
 
     @staticmethod
     def vmap(info, in_dims, state, *xs):
@@ -379,6 +467,69 @@ class _EPDInstances(torch.autograd.Function):
             flat.append(x)
         out, ws = _EPDInstances.apply(state, *flat)
         return (out.reshape(b, k, *out.shape[1:]), ws), (0, None)
+
+
+class _EPDInstanceAdjoint(torch.autograd.Function):
+    """Input gradients of the K instances of a saving _EPDInstances for M cotangents each, pdg_vjp_instances in passes of
+    at most VJP_MAX_COTANGENTS (instance, cotangent) pairs.  `saved` is (state, inputs, workspace) of that forward, `want`
+    the (mean_stress, pos, edge_attr) flags of the gradients to form, `g` the cotangent of local_stress [K, N, 3] or
+    [M, K, N, 3].  Returns the wanted gradients in that order, each [K, *input shape] (or [M, K, *input shape]): the row
+    of every instance, for shared inputs too.  The vmap rule folds the vmapped dimension into M.  There is no backward:
+    second-order derivatives are not implemented."""
+
+    @staticmethod
+    def forward(saved, want, g):
+        L = _lib.lib()
+        state, xs, ws = saved
+        model, plan, types, flags, steps, params = state
+        dev = types.device
+        n, e = plan.n_nodes, plan.n_edges
+        k, args = _instance_args(state, xs)
+        m = g.shape[0] if g.dim() == 4 else None
+        mm = m or 1
+        # rows i * M + j of pdg_vjp_instances: instance-major
+        g = _lib.require_cuda(g.to(torch.float32), "grad_local_stress", torch.float32).reshape(mm, k, n, 3).transpose(0, 1)
+        cap = _lib.VJP_MAX_COTANGENTS
+        ip, mp = max(1, cap // mm), min(mm, cap)  # instances and cotangents per pass
+        iws = L.pdg_forward_batched_saved_ws_bytes(n, e, steps, flags, 1)
+        with torch.cuda.device(dev):
+            outs = [torch.empty((k, mm) + s, dtype=torch.float32, device=dev) if w else None
+                    for w, s in zip(want, _tangent_shapes(state))]
+            vws_bytes = L.pdg_vjp_batched_ws_bytes(n, e, steps, min(k, ip) * mp)
+            vws = torch.empty(_bucket(vws_bytes), dtype=torch.uint8, device=dev)  # reused by every pass (stream order)
+            ps, norm = _params_struct(params), model._norm_struct()
+            for i in range(0, k, ip):
+                ii = min(ip, k - i)
+                xp = [_lib.ptr(x[i:i + ii] if st else x) for x, st in args]
+                for j in range(0, mm, mp):
+                    jj = min(mp, mm - j)
+                    gp = g[i:i + ii, j:j + jj].contiguous()
+                    dst = [o[i:i + ii, j:j + jj] if o is not None else None for o in outs]
+                    tmp = [d if d is None or d.is_contiguous() else torch.empty_like(d) for d in dst]
+                    _lib.check(L.pdg_vjp_instances(C.byref(ps), C.byref(norm), xp[0], args[0][1], xp[1], args[1][1],
+                                                   _lib.ptr(types), xp[2], args[2][1], _lib.ptr(plan.buf), n, e, steps,
+                                                   flags, _lib.PREC_FP32, _lib.ptr(ws[i * iws:]), ii, _lib.ptr(vws),
+                                                   vws_bytes, jj, _lib.ptr(gp), *(_lib.ptr(t) for t in tmp),
+                                                   _lib.stream_ptr(dev)), "pdg_vjp_instances")
+                    for d, t in zip(dst, tmp):
+                        if t is not d:
+                            d.copy_(t)
+        return tuple(o.transpose(0, 1) if m is not None else o[:, 0] for o in outs if o is not None)
+
+    @staticmethod
+    def setup_context(ctx, inputs, output):
+        pass
+
+    @staticmethod
+    def vmap(info, in_dims, saved, want, g):
+        """Moves the vmapped dimension B of the cotangent to the front and merges it with an M that an inner vmap level
+        already folded in ([B, M, K, N, 3] -> [B*M, K, N, 3]: nested vmap flattens)."""
+        b = info.batch_size
+        g = g.unsqueeze(0).expand(b, *g.shape) if in_dims[2] is None else g.movedim(in_dims[2], 0)
+        m = g.shape[1] if g.dim() == 5 else None
+        outs = _EPDInstanceAdjoint.apply(saved, want, g.reshape(b * (m or 1), *g.shape[-3:]))
+        outs = tuple(o.reshape(b, m, *o.shape[1:]) if m is not None else o for o in outs)
+        return outs, (0,) * len(outs)
 
 
 class _EPDTangent(torch.autograd.Function):
@@ -550,8 +701,10 @@ def epd_forward(model, mesh_graph, scale_output: bool, scale_input: bool, zero_c
     # with respect to them is refused here, and a batched backward refuses any swapped parameter (a fresh walk only
     # under a transform)
     swapped = False
+    grad_level = 0
     transformed = torch._C._functorch.maybe_current_level() is not None
     if transformed:
+        grad_level = max(_grad_level(x) for x in (mean_stress, pos, edge_attr))
         fresh = [q for _, q in model.named_parameters()]
         swapped = any(q is not p for q, p in zip(fresh, params))
         if swapped and any(_lib.is_vmapped(q) for q in fresh):
@@ -567,4 +720,4 @@ def epd_forward(model, mesh_graph, scale_output: bool, scale_input: bool, zero_c
         return _forward_graphed(model, plan, mean_stress, pos, types, edge_attr, flags, model.message_passing_steps, prec,
                                 params)
     return _EPDFunction.apply(model, plan, mean_stress, pos, types, edge_attr, flags, model.message_passing_steps, prec,
-                              need_grad, need_tan, swapped, *params)[0]
+                              need_grad, need_tan, swapped, grad_level, *params)[0]

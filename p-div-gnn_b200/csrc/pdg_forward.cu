@@ -771,11 +771,61 @@ extern "C" int pdg_forward(const pdg_params_t* params, const pdg_norm_t* norm, c
   return forward_run<false>(params, norm, mean_stress, 0, pos, 0, nodes_types, edge_attr, 0, plan, W, flags, 1, tcm, local_stress, st);
 }
 
-// K instances of one graph: the workspace holds K fp32 forward workspaces without saved state, one after another
-// (each total is a multiple of 256 bytes, so every instance stays aligned).
+// K instances of one graph: the workspace holds K fp32 forward workspaces, one after another (each total is a multiple of
+// 256 bytes, so every instance stays aligned); pdg_forward_batched keeps no saved state, pdg_forward_batched_saved keeps
+// a full PDG_FLAG_SAVE state per instance for pdg_vjp_instances.
 extern "C" size_t pdg_forward_batched_ws_bytes(int64_t n_nodes, int64_t n_edges, int steps, int flags, int n_instances) {
   if (n_instances < 1 || n_instances > PDG_FWD_MAX_INSTANCES || steps < 1 || steps > 62) return 0;
   return (size_t)n_instances * FwdWs(n_nodes, n_edges, steps, (flags & PDG_FLAG_SAVE) != 0, nullptr, false).total;
+}
+
+extern "C" size_t pdg_forward_batched_saved_ws_bytes(int64_t n_nodes, int64_t n_edges, int steps, int flags, int n_instances) {
+  return (flags & PDG_FLAG_SAVE) ? pdg_forward_batched_ws_bytes(n_nodes, n_edges, steps, flags, n_instances) : 0;
+}
+
+static int forward_instances(const char* fn, bool save, const pdg_params_t* params, const pdg_norm_t* norm,
+                             const float* mean_stress, int64_t ms_stride, const float* pos, int64_t pos_stride,
+                             const int64_t* nodes_types, const float* edge_attr, int64_t ea_stride, const void* plan,
+                             int64_t n_nodes, int64_t n_edges, int steps, int flags, int precision, void* ws, size_t ws_bytes,
+                             int K, float* local_stress, cudaStream_t st) {
+  if (K < 1 || K > PDG_FWD_MAX_INSTANCES) {
+    set_error("%s: n_instances=%d outside 1..%d", fn, K, PDG_FWD_MAX_INSTANCES);
+    return -1;
+  }
+  if (precision != PDG_PREC_FP32) {
+    set_error("%s: only the fp32 mode (PDG_PREC_FP32) runs instances; the 16-bit mode's kernels are "
+              "persistent, one CTA per SM", fn);
+    return -1;
+  }
+  if (!save && (flags & PDG_FLAG_SAVE)) {
+    set_error("%s: PDG_FLAG_SAVE is not supported (the batched forward keeps no state for a backward; "
+              "pdg_forward_batched_saved does)", fn);
+    return -1;
+  }
+  if (save && !(flags & PDG_FLAG_SAVE)) { set_error("%s: flags must contain PDG_FLAG_SAVE", fn); return -1; }
+  if (steps < 1 || steps > 62) { set_error("%s: steps=%d unsupported", fn, steps); return -1; }
+  if (ms_stride < 0 || pos_stride < 0 || ea_stride < 0) {
+    set_error("%s: negative input stride (mean_stress %lld, pos %lld, edge_attr %lld)", fn, (long long)ms_stride,
+              (long long)pos_stride, (long long)ea_stride);
+    return -1;
+  }
+  if (n_nodes <= 0 || n_edges <= 0) { set_error("%s: empty graph", fn); return -1; }
+  const FwdWs W(n_nodes, n_edges, steps, save, ws, false);
+  if (ws_bytes < (size_t)K * W.total) {
+    set_error("%s: workspace %zu < %zu", fn, ws_bytes, (size_t)K * W.total);
+    return -1;
+  }
+  const int rc = forward_run<true>(params, norm, mean_stress, ms_stride, pos, pos_stride, nodes_types, edge_attr, ea_stride,
+                                  plan, W, flags, K, false, local_stress, st);
+  if (rc != 0 || !save) return rc;
+  // The kernels read the packed weights in instance 0's workspace only.  A saved workspace also gives every later
+  // instance a copy, so that an adjoint pass (pdg_vjp_instances) may start at any instance of it: copies that double
+  // the number of packed instances each time, log2(K) of them.
+  const size_t pack_bytes = PackOffsets::TOTAL * sizeof(float);
+  for (int have = 1; have < K; have *= 2)
+    PDG_CUDA_CHECK(cudaMemcpy2DAsync((char*)W.pack + (size_t)have * W.total, W.total, W.pack, W.total, pack_bytes,
+                                     have < K - have ? have : K - have, cudaMemcpyDeviceToDevice, st));
+  return 0;
 }
 
 extern "C" int pdg_forward_batched(const pdg_params_t* params, const pdg_norm_t* norm, const float* mean_stress,
@@ -783,34 +833,19 @@ extern "C" int pdg_forward_batched(const pdg_params_t* params, const pdg_norm_t*
                                    const float* edge_attr, int64_t ea_stride, const void* plan, int64_t n_nodes,
                                    int64_t n_edges, int steps, int flags, int precision, void* ws, size_t ws_bytes,
                                    int n_instances, float* local_stress, void* stream_) {
-  const int K = n_instances;
-  if (K < 1 || K > PDG_FWD_MAX_INSTANCES) {
-    set_error("pdg_forward_batched: n_instances=%d outside 1..%d", K, PDG_FWD_MAX_INSTANCES);
-    return -1;
-  }
-  if (precision != PDG_PREC_FP32) {
-    set_error("pdg_forward_batched: only the fp32 mode (PDG_PREC_FP32) runs instances; the 16-bit mode's kernels are "
-              "persistent, one CTA per SM");
-    return -1;
-  }
-  if (flags & PDG_FLAG_SAVE) {
-    set_error("pdg_forward_batched: PDG_FLAG_SAVE is not supported (the batched forward keeps no state for a backward)");
-    return -1;
-  }
-  if (steps < 1 || steps > 62) { set_error("pdg_forward_batched: steps=%d unsupported", steps); return -1; }
-  if (ms_stride < 0 || pos_stride < 0 || ea_stride < 0) {
-    set_error("pdg_forward_batched: negative input stride (mean_stress %lld, pos %lld, edge_attr %lld)",
-              (long long)ms_stride, (long long)pos_stride, (long long)ea_stride);
-    return -1;
-  }
-  if (n_nodes <= 0 || n_edges <= 0) { set_error("pdg_forward_batched: empty graph"); return -1; }
-  const FwdWs W(n_nodes, n_edges, steps, false, ws, false);
-  if (ws_bytes < (size_t)K * W.total) {
-    set_error("pdg_forward_batched: workspace %zu < %zu", ws_bytes, (size_t)K * W.total);
-    return -1;
-  }
-  return forward_run<true>(params, norm, mean_stress, ms_stride, pos, pos_stride, nodes_types, edge_attr, ea_stride, plan, W,
-                           flags, K, false, local_stress, (cudaStream_t)stream_);
+  return forward_instances("pdg_forward_batched", false, params, norm, mean_stress, ms_stride, pos, pos_stride, nodes_types,
+                           edge_attr, ea_stride, plan, n_nodes, n_edges, steps, flags, precision, ws, ws_bytes, n_instances,
+                           local_stress, (cudaStream_t)stream_);
+}
+
+extern "C" int pdg_forward_batched_saved(const pdg_params_t* params, const pdg_norm_t* norm, const float* mean_stress,
+                                         int64_t ms_stride, const float* pos, int64_t pos_stride, const int64_t* nodes_types,
+                                         const float* edge_attr, int64_t ea_stride, const void* plan, int64_t n_nodes,
+                                         int64_t n_edges, int steps, int flags, int precision, void* ws, size_t ws_bytes,
+                                         int n_instances, float* local_stress, void* stream_) {
+  return forward_instances("pdg_forward_batched_saved", true, params, norm, mean_stress, ms_stride, pos, pos_stride,
+                           nodes_types, edge_attr, ea_stride, plan, n_nodes, n_edges, steps, flags, precision, ws, ws_bytes,
+                           n_instances, local_stress, (cudaStream_t)stream_);
 }
 
 // Test/debug helper: byte offset and element count of a saved tensor inside a forward

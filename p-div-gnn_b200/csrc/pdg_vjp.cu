@@ -39,27 +39,53 @@ struct VjpWs : DataGradBufs {
   }
 };
 
-// ---- LayerNorm-backward scalars {c1, c2, mu, a} of one or two instances (blockIdx.x) for every cotangent (blockIdx.y) ----
-__global__ void __launch_bounds__(FIN_G* H) k_ln_finalize_vjp(LnFinArgs a0, LnFinArgs a1, size_t cws) {
+// Instances (pdg_vjp_instances): every wrapper below is a template on INST.  With INST, cotangent k = blockIdx.y belongs to
+// instance i = k / M: the forward state it reads moves by i * iws bytes (instance i's saved forward workspace) and the
+// model inputs by i * (element stride).  The packed weights stay where they are: every wrapper reads them in the first
+// instance of fwd_ws (pdg_forward_batched_saved leaves a copy in every instance's workspace).
+// Without INST (pdg_vjp_batched) the trailing arguments are not read.
+
+// ---- LayerNorm-backward scalars {c1, c2, mu, a} of one or two LayerNorms (blockIdx.x) for every cotangent (blockIdx.y) ----
+template <bool INST>
+__global__ void __launch_bounds__(FIN_G* H) k_ln_finalize_vjp(LnFinArgs a0, LnFinArgs a1, size_t cws, int M, size_t iws) {
   const LnFinArgs& a = blockIdx.x == 0 ? a0 : a1;
   const size_t off = (size_t)blockIdx.y * cws;
-  ln_finalize_body<false>(copy_at(a.cs, off), a.nparts, a.fwd_parts, a.count, a.lnw, copy_at(a.scal_out, off), nullptr, nullptr);
+  const double* fwd_parts = a.fwd_parts;
+  if constexpr (INST) fwd_parts = copy_at(fwd_parts, (size_t)(blockIdx.y / M) * iws);
+  ln_finalize_body<false>(copy_at(a.cs, off), a.nparts, fwd_parts, a.count, a.lnw, copy_at(a.scal_out, off), nullptr, nullptr);
 }
 
 // ---- decoder, node_update, node_pre, encoders: the bodies of the fp32 backward without weight gradients (pdg_bwd.cuh) for
 // cotangent blockIdx.y ------------------------------------------------------------------------------------------------
+template <bool INST>
 __global__ void __launch_bounds__(NT, 1)
 k_decoder_vjp(const float* __restrict__ g_out, float gscale, const float* __restrict__ hd, const float* __restrict__ y3_last,
               const double* __restrict__ parts_prev, double count_prev, const float* __restrict__ D1,
               const float* __restrict__ D2, float* __restrict__ gx, float* __restrict__ cs3, const int* __restrict__ nzflag,
-              int N, int n_tiles, size_t cws) {
+              int N, int n_tiles, size_t cws, int M, size_t iws) {
   const size_t off = (size_t)blockIdx.y * cws;
+  if constexpr (INST) {
+    const size_t io = (size_t)(blockIdx.y / M) * iws;
+    hd = copy_at(hd, io);
+    y3_last = copy_at(y3_last, io);
+    parts_prev = copy_at(parts_prev, io);
+    nzflag = copy_at(nzflag, io);
+  }
   decoder_bwd_body<false>(g_out + (size_t)blockIdx.y * N * PDG_OUT, gscale, hd, nullptr, y3_last, parts_prev, count_prev, D1, D2,
                           copy_at(gx, off), nullptr, copy_at(cs3, off), nzflag, N, n_tiles);  // g_out: [K][N][3]
 }
 
-__global__ void __launch_bounds__(NT, 1) k_node_update_vjp(NodeUpdBwdArgs a, size_t cws) {
+template <bool INST>
+__global__ void __launch_bounds__(NT, 1) k_node_update_vjp(NodeUpdBwdArgs a, size_t cws, int M, size_t iws) {
   const size_t off = (size_t)blockIdx.y * cws;
+  if constexpr (INST) {
+    const size_t io = (size_t)(blockIdx.y / M) * iws;
+    a.y3 = copy_at(a.y3, io);
+    a.hq = copy_at(a.hq, io);
+    a.aggraw = copy_at(a.aggraw, io);
+    a.x_t = copy_at(a.x_t, io);
+    a.parts1 = copy_at(a.parts1, io);
+  }
   a.gx = copy_at(a.gx, off);
   a.gagg = copy_at(a.gagg, off);
   a.scal3 = copy_at(a.scal3, off);
@@ -67,8 +93,15 @@ __global__ void __launch_bounds__(NT, 1) k_node_update_vjp(NodeUpdBwdArgs a, siz
   node_update_bwd_body<false>(a);
 }
 
-__global__ void __launch_bounds__(NT, 1) k_node_pre_vjp(NodePreBwdArgs a, size_t cws) {
+template <bool INST>
+__global__ void __launch_bounds__(NT, 1) k_node_pre_vjp(NodePreBwdArgs a, size_t cws, int M, size_t iws) {
   const size_t off = (size_t)blockIdx.y * cws;
+  if constexpr (INST) {
+    const size_t io = (size_t)(blockIdx.y / M) * iws;
+    a.x_t = copy_at(a.x_t, io);
+    a.yprev = copy_at(a.yprev, io);
+    a.parts_prev = copy_at(a.parts_prev, io);
+  }
   a.gx = copy_at(a.gx, off);
   a.RA = copy_at(a.RA, off);
   a.RB = copy_at(a.RB, off);
@@ -80,14 +113,26 @@ __global__ void __launch_bounds__(NT, 1) k_node_pre_vjp(NodePreBwdArgs a, size_t
 
 //   node  gi0 = d/d mean_stress [K][N][3], gi1 = d/d pos [K][N][2] (either may be null);
 //   edge  gi0 = d/d edge_attr [K][E] at perm[row] (PyG edge order)
-template <int NODE>
+//   INST: instance i's inputs start s0 (mean_stress or edge_attr) and s1 (pos) elements per instance further on
+template <int NODE, bool INST>
 __global__ void __launch_bounds__(NT, 1)
 k_encoder_vjp(const float* __restrict__ g_in, const float* __restrict__ y_raw, const float* __restrict__ scal,
               const float* __restrict__ lnw, const float* __restrict__ mean_stress, const float* __restrict__ pos,
               const int64_t* __restrict__ types, const float* __restrict__ edge_attr, const int32_t* __restrict__ perm,
               pdg_norm_t nrm, int scale_in, const float* __restrict__ W0, const float* __restrict__ b0,
-              const float* __restrict__ W2, int R, int n_tiles, float* __restrict__ gi0, float* __restrict__ gi1, size_t cws) {
+              const float* __restrict__ W2, int R, int n_tiles, float* __restrict__ gi0, float* __restrict__ gi1, size_t cws,
+              int M, size_t iws, int64_t s0, int64_t s1) {
   const size_t off = (size_t)blockIdx.y * cws;
+  if constexpr (INST) {
+    const unsigned i = blockIdx.y / M;
+    y_raw = copy_at(y_raw, (size_t)i * iws);
+    if (NODE) {
+      mean_stress += i * s0;
+      pos += i * s1;
+    } else {
+      edge_attr += i * s0;
+    }
+  }
   if (gi0 != nullptr) gi0 += (size_t)blockIdx.y * R * (NODE ? 3 : 1);
   if (gi1 != nullptr) gi1 += (size_t)blockIdx.y * R * 2;
   encoder_bwd_body<NODE, false, true>(copy_at(g_in, off), y_raw, copy_at(scal, off), lnw, mean_stress, pos, types, edge_attr, perm,
@@ -100,15 +145,36 @@ k_encoder_vjp(const float* __restrict__ g_in, const float* __restrict__ y_raw, c
 //   per cotangent: dy1 -> T1;  dhm = m1 (dy1 W2) -> DHM, T1, segment sums RA;
 //                  dy2 -> T2;  dhn = m2 (dy2 W2) -> DHN, T2, segment sums RB   (not on the last step);
 //                  dG = dhm + dhn -> T1;  ge = ge + dG We  and the column sums of the LayerNorm that produced e_t
+//   INST: blockIdx.y = i * gpi + g, group g of instance i's K cotangents (a group never spans two instances: G, the masks
+//   and y1 are the instance's own)
 struct EdgeVjpArgs {
-  EdgeBwdArgs e;  // cotangent 0's buffers (gagg, ge, scal1, scal2, DHM, DHN, RA, RB, cs2) and the primal state
+  EdgeBwdArgs e;  // cotangent 0's buffers (gagg, ge, scal1, scal2, DHM, DHN, RA, RB, cs2) and instance 0's primal state
   float* eacc;
   size_t cws;
-  int K, C;
+  int K, C;       // cotangents (of one instance with INST), cotangents per group
+  int gpi;        // INST: groups per instance
+  size_t iws;     // INST: bytes between instance workspaces
 };
 
+template <bool INST>
 __global__ void __launch_bounds__(NT, 1) k_edge_step_vjp(EdgeVjpArgs v) {
   extern __shared__ __align__(16) float smem[];
+  int k0, nk;  // this CTA's cotangents: k0 .. k0 + nk - 1
+  if constexpr (INST) {
+    const int i = blockIdx.y / v.gpi, g = blockIdx.y - i * v.gpi;
+    const size_t io = (size_t)i * v.iws;
+    v.e.e_t = copy_at(v.e.e_t, io);
+    v.e.Pa = copy_at(v.e.Pa, io);
+    v.e.Pb = copy_at(v.e.Pb, io);
+    v.e.y2_t = copy_at(v.e.y2_t, io);
+    v.e.yprev = copy_at(v.e.yprev, io);
+    v.e.parts_prev = copy_at(v.e.parts_prev, io);
+    k0 = i * v.K + g * v.C;
+    nk = min(v.C, v.K - g * v.C);
+  } else {
+    k0 = blockIdx.y * v.C;
+    nk = min(v.C, v.K - k0);
+  }
   const EdgeBwdArgs& a = v.e;
   float* T0 = smem;
   float* T1 = T0 + TM * LDS;
@@ -121,7 +187,6 @@ __global__ void __launch_bounds__(NT, 1) k_edge_step_vjp(EdgeVjpArgs v) {
   unsigned char* seg_row = reinterpret_cast<unsigned char*>(seg_masks + 4);  // [TM + 1]
   float seg_dummy = 0.f;
   const int tid = threadIdx.x, ty = tid >> 4, tx = tid & 15;
-  const int k0 = blockIdx.y * v.C, nk = min(v.C, v.K - k0);  // this CTA's cotangents: k0 .. k0 + nk - 1
   const float mu_prev = ln_stat_block(a.parts_prev, a.count_prev, (float*)smi).mu;
   for (int tile = blockIdx.x; tile < a.n_tiles; tile += gridDim.x) {
     const int row0 = tile * TM;
@@ -302,33 +367,55 @@ extern "C" size_t pdg_vjp_batched_ws_bytes(int64_t n_nodes, int64_t n_edges, int
   return (size_t)n_cotangents * VjpWs(n_nodes, n_edges, steps, nullptr).total;
 }
 
-extern "C" int pdg_vjp_batched(const pdg_params_t* params, const pdg_norm_t* norm, const float* mean_stress, const float* pos,
-                               const int64_t* nodes_types, const float* edge_attr, const void* plan, int64_t n_nodes,
-                               int64_t n_edges, int steps, int flags, int precision, const void* fwd_ws, void* vjp_ws,
-                               size_t vjp_ws_bytes, int n_cotangents, const float* grad_local_stress, float* grad_mean_stress,
-                               float* grad_pos, float* grad_edge_attr, void* stream_) {
-  cudaStream_t st = (cudaStream_t)stream_;
-  const int K = n_cotangents;
-  if (K < 1 || K > PDG_VJP_MAX_COTANGENTS) {
-    set_error("pdg_vjp_batched: n_cotangents=%d outside 1..%d", K, PDG_VJP_MAX_COTANGENTS);
+namespace pdg {
+
+// The adjoint pass of I instances with M cotangents each: cotangent k = i * M + m reads instance i's saved state (its forward
+// workspace at fwd_ws + i * iws) and inputs.  pdg_vjp_batched is I = 1 with INST off; pdg_vjp_instances runs INST.
+template <bool INST>
+static int vjp_run(const char* fn, const pdg_params_t* params, const pdg_norm_t* norm, const float* mean_stress, int64_t ms_stride,
+                   const float* pos, int64_t pos_stride, const int64_t* nodes_types, const float* edge_attr, int64_t ea_stride,
+                   const void* plan, int64_t n_nodes, int64_t n_edges, int steps, int flags, int precision, const void* fwd_ws,
+                   int I, void* vjp_ws, size_t vjp_ws_bytes, int M, const float* grad_local_stress, float* grad_mean_stress,
+                   float* grad_pos, float* grad_edge_attr, cudaStream_t st) {
+  const int K = I * M;  // cotangents of the pass
+  if (M < 1 || M > PDG_VJP_MAX_COTANGENTS) {
+    set_error("%s: n_cotangents=%d outside 1..%d", fn, M, PDG_VJP_MAX_COTANGENTS);
+    return -1;
+  }
+  if (INST && (I < 1 || I > PDG_FWD_MAX_INSTANCES)) {
+    set_error("%s: n_instances=%d outside 1..%d", fn, I, PDG_FWD_MAX_INSTANCES);
+    return -1;
+  }
+  if (K > PDG_VJP_MAX_COTANGENTS) {
+    set_error("%s: n_instances * n_cotangents = %d * %d > %d", fn, I, M, PDG_VJP_MAX_COTANGENTS);
     return -1;
   }
   if (precision != PDG_PREC_FP32) {
-    set_error("pdg_vjp_batched: only the fp32 mode (PDG_PREC_FP32) has a batched reverse-mode derivative; the 16-bit "
-              "mode's input gradients miss its 2e-2 tolerance");
+    set_error("%s: only the fp32 mode (PDG_PREC_FP32) has a batched reverse-mode derivative; the 16-bit "
+              "mode's input gradients miss its 2e-2 tolerance", fn);
     return -1;
   }
-  if (!(flags & PDG_FLAG_SAVE)) { set_error("pdg_vjp_batched: the forward workspace must come from a pdg_forward with PDG_FLAG_SAVE"); return -1; }
-  if (steps < 1 || steps > 62) { set_error("pdg_vjp_batched: steps=%d unsupported", steps); return -1; }
+  if (!(flags & PDG_FLAG_SAVE)) {
+    set_error(INST ? "%s: the forward workspace must come from a pdg_forward_batched_saved (flags with PDG_FLAG_SAVE)"
+                   : "%s: the forward workspace must come from a pdg_forward with PDG_FLAG_SAVE", fn);
+    return -1;
+  }
+  if (steps < 1 || steps > 62) { set_error("%s: steps=%d unsupported", fn, steps); return -1; }
+  if (ms_stride < 0 || pos_stride < 0 || ea_stride < 0) {
+    set_error("%s: negative input stride (mean_stress %lld, pos %lld, edge_attr %lld)", fn, (long long)ms_stride,
+              (long long)pos_stride, (long long)ea_stride);
+    return -1;
+  }
   if (grad_mean_stress == nullptr && grad_pos == nullptr && grad_edge_attr == nullptr) {
-    set_error("pdg_vjp_batched: no output requested (grad_mean_stress, grad_pos and grad_edge_attr are all NULL)");
+    set_error("%s: no output requested (grad_mean_stress, grad_pos and grad_edge_attr are all NULL)", fn);
     return -1;
   }
-  if (n_nodes <= 0 || n_edges <= 0) { set_error("pdg_vjp_batched: empty graph"); return -1; }
-  const FwdWs W(n_nodes, n_edges, steps, true, const_cast<void*>(fwd_ws), false);
+  if (n_nodes <= 0 || n_edges <= 0) { set_error("%s: empty graph", fn); return -1; }
+  const FwdWs W(n_nodes, n_edges, steps, true, const_cast<void*>(fwd_ws), false);  // instance 0
+  const size_t iws = W.total;  // bytes between consecutive instance workspaces
   const VjpWs V(n_nodes, n_edges, steps, vjp_ws);
   const size_t cws = V.total;  // bytes between consecutive cotangent workspaces
-  if (vjp_ws_bytes < (size_t)K * cws) { set_error("pdg_vjp_batched: workspace %zu < %zu", vjp_ws_bytes, (size_t)K * cws); return -1; }
+  if (vjp_ws_bytes < (size_t)K * cws) { set_error("%s: workspace %zu < %zu", fn, vjp_ws_bytes, (size_t)K * cws); return -1; }
   const int N = (int)n_nodes, E = (int)n_edges, T = steps;
   int32_t *perm, *recv, *send, *rowptr, *sptr, *slist;
   pdg_plan_views(const_cast<void*>(plan), n_nodes, n_edges, &perm, &recv, &send, &rowptr, &sptr, &slist);
@@ -336,20 +423,21 @@ extern "C" int pdg_vjp_batched(const pdg_params_t* params, const pdg_norm_t* nor
   int G = num_sms();
   if (G > MAXP) G = MAXP;
   const int grid_n = balanced_grid(nt_n, G), grid_e = balanced_grid(nt_e, G);  // the x-grids of pdg_backward_inputs
-  // Edge kernel: cotangent groups of C over the SMs the x-grid leaves idle (the rule of pdg_jvp_batched)
-  int groups = std::min(K, std::max(1, G / grid_e));
-  const int C = (K + groups - 1) / groups;
-  groups = (K + C - 1) / C;  // no empty group
+  // Edge kernel: each instance's cotangents in groups of C over the SMs the x-grid leaves idle (the rule of
+  // pdg_jvp_batched); a group never spans two instances
+  int groups = std::min(M, std::max(1, G / (grid_e * I)));
+  const int C = (M + groups - 1) / groups;
+  groups = (M + C - 1) / C;  // no empty group
   const double cnt_n = (double)N * H, cnt_e = (double)E * H;
   const float* const* P = params->p;
   const int scale_in = (flags & PDG_FLAG_SCALE_INPUT) ? 1 : 0;
   const bool ig_node = grad_mean_stress != nullptr || grad_pos != nullptr, ig_edge = grad_edge_attr != nullptr;
-  if (set_smem((const void*)k_decoder_vjp, SMEM_V2T)) return -2;
-  if (set_smem((const void*)k_node_update_vjp, SMEM_V2T)) return -2;
-  if (set_smem((const void*)k_edge_step_vjp, SMEM_B3T)) return -2;
-  if (set_smem((const void*)k_node_pre_vjp, SMEM_V2T)) return -2;
-  if (set_smem((const void*)k_encoder_vjp<1>, SMEM_V2T)) return -2;
-  if (set_smem((const void*)k_encoder_vjp<0>, SMEM_V2T)) return -2;
+  if (set_smem((const void*)k_decoder_vjp<INST>, SMEM_V2T)) return -2;
+  if (set_smem((const void*)k_node_update_vjp<INST>, SMEM_V2T)) return -2;
+  if (set_smem((const void*)k_edge_step_vjp<INST>, SMEM_B3T)) return -2;
+  if (set_smem((const void*)k_node_pre_vjp<INST>, SMEM_V2T)) return -2;
+  if (set_smem((const void*)k_encoder_vjp<1, INST>, SMEM_V2T)) return -2;
+  if (set_smem((const void*)k_encoder_vjp<0, INST>, SMEM_V2T)) return -2;
   auto scal = [&](int slot) { return V.scal + slot * 4; };
   const dim3 gn(grid_n, K);
 
@@ -358,8 +446,8 @@ extern "C" int pdg_vjp_batched(const pdg_params_t* params, const pdg_norm_t* nor
     const int* nzf = (flags & PDG_FLAG_ZERO_CHECK) ? W.nzflag : nullptr;
     const float gscale = (flags & PDG_FLAG_SCALE_OUTPUT) ? norm->std_local_stress : 1.f;
     const DecArgs d = fwd_dec_args(W, P);  // what the forward's decoder read and saved
-    k_decoder_vjp<<<gn, NT, SMEM_V2T, st>>>(grad_local_stress, gscale, d.hd_out, d.yprev, d.prev_parts, d.prev_count, P[ND_W0],
-                                            d.D2, V.gx, V.cs3, nzf, N, nt_n, cws);
+    k_decoder_vjp<INST><<<gn, NT, SMEM_V2T, st>>>(grad_local_stress, gscale, d.hd_out, d.yprev, d.prev_parts, d.prev_count,
+                                                  P[ND_W0], d.D2, V.gx, V.cs3, nzf, N, nt_n, cws, M, iws);
   }
   PDG_LAUNCH_CHECK();
   // receiver-side segment sums RA / RB (adjacent) of every cotangent start from zero: one strided memset
@@ -369,13 +457,13 @@ extern "C" int pdg_vjp_batched(const pdg_params_t* params, const pdg_norm_t* nor
     {
       ScopedTimer tm_(KC_VJP_LN_FIN, st);
       LnFinArgs f3{V.cs3, grid_n, W.parts_slot(slot_ln3(t)), cnt_n, P[PN_LNW], scal(slot_ln3(t)), nullptr, nullptr};
-      k_ln_finalize_vjp<<<dim3(1, K), FIN_G * H, 0, st>>>(f3, f3, cws);
+      k_ln_finalize_vjp<INST><<<dim3(1, K), FIN_G * H, 0, st>>>(f3, f3, cws, M, iws);
     }
     PDG_LAUNCH_CHECK();
     const BwdStepArgs s = bwd_step_args(W, P, V, recv, send, rowptr, sptr, slist, t);
     {
       ScopedTimer tm_(KC_VJP_NODE_UPD, st);
-      k_node_update_vjp<<<gn, NT, SMEM_V2T, st>>>(s.u, cws);
+      k_node_update_vjp<INST><<<gn, NT, SMEM_V2T, st>>>(s.u, cws, M, iws);
     }
     PDG_LAUNCH_CHECK();
     {
@@ -383,42 +471,65 @@ extern "C" int pdg_vjp_batched(const pdg_params_t* params, const pdg_norm_t* nor
       LnFinArgs f1{V.cs1, grid_n, W.parts_slot(slot_ln1(t)), cnt_e, P[PE_LNW], scal(slot_ln1(t)), nullptr, nullptr};
       LnFinArgs f2 = f1;
       if (!last) f2 = LnFinArgs{V.cs2, grid_e, W.parts_slot(slot_ln2(t)), cnt_e, P[PE_LNW], scal(slot_ln2(t)), nullptr, nullptr};
-      k_ln_finalize_vjp<<<dim3(last ? 1 : 2, K), FIN_G * H, 0, st>>>(f1, f2, cws);
+      k_ln_finalize_vjp<INST><<<dim3(last ? 1 : 2, K), FIN_G * H, 0, st>>>(f1, f2, cws, M, iws);
     }
     PDG_LAUNCH_CHECK();
-    const EdgeVjpArgs v{s.e, V.eacc, cws, K, C};
+    const EdgeVjpArgs v{s.e, V.eacc, cws, M, C, groups, iws};
     {
       ScopedTimer tm_(KC_VJP_EDGE_STEP, st);
-      k_edge_step_vjp<<<dim3(grid_e, groups), NT, SMEM_B3T, st>>>(v);
+      k_edge_step_vjp<INST><<<dim3(grid_e, I * groups), NT, SMEM_B3T, st>>>(v);
     }
     PDG_LAUNCH_CHECK();
     {
       ScopedTimer tm_(KC_VJP_NODE_PRE, st);
-      k_node_pre_vjp<<<gn, NT, SMEM_V2T, st>>>(s.n, cws);
+      k_node_pre_vjp<INST><<<gn, NT, SMEM_V2T, st>>>(s.n, cws, M, iws);
     }
     PDG_LAUNCH_CHECK();
   }
   // encoders: x_0 = LN(y_nenc), e_0 = LN(y_eenc)
   {
     ScopedTimer tm_(KC_VJP_LN_FIN, st);
-    LnFinArgs fn{V.cs3, grid_n, W.parts_slot(0), cnt_n, P[NE_LNW], scal(0), nullptr, nullptr};
+    LnFinArgs fn_{V.cs3, grid_n, W.parts_slot(0), cnt_n, P[NE_LNW], scal(0), nullptr, nullptr};
     LnFinArgs fe{V.cs2, grid_e, W.parts_slot(1), cnt_e, P[EE_LNW], scal(1), nullptr, nullptr};
-    k_ln_finalize_vjp<<<dim3(2, K), FIN_G * H, 0, st>>>(fn, fe, cws);
+    k_ln_finalize_vjp<INST><<<dim3(2, K), FIN_G * H, 0, st>>>(fn_, fe, cws, M, iws);
   }
   PDG_LAUNCH_CHECK();
   if (ig_node) {
     ScopedTimer tm_(KC_VJP_ENC, st);
-    k_encoder_vjp<1><<<gn, NT, SMEM_V2T, st>>>(V.gx, W.y_nenc, scal(0), P[NE_LNW], mean_stress, pos, nodes_types, nullptr, nullptr,
-                                               *norm, scale_in, P[NE_W0], P[NE_B0], P[NE_W2], N, nt_n, grad_mean_stress, grad_pos,
-                                               cws);
+    k_encoder_vjp<1, INST><<<gn, NT, SMEM_V2T, st>>>(V.gx, W.y_nenc, scal(0), P[NE_LNW], mean_stress, pos, nodes_types, nullptr,
+                                                     nullptr, *norm, scale_in, P[NE_W0], P[NE_B0], P[NE_W2], N, nt_n,
+                                                     grad_mean_stress, grad_pos, cws, M, iws, ms_stride, pos_stride);
   }
   if (ig_node) PDG_LAUNCH_CHECK();
   if (ig_edge) {
     ScopedTimer tm_(KC_VJP_ENC, st);
-    k_encoder_vjp<0><<<dim3(grid_e, K), NT, SMEM_V2T, st>>>(V.ge, W.y_eenc, scal(1), P[EE_LNW], nullptr, nullptr, nullptr, edge_attr,
-                                                            perm, *norm, scale_in, P[EE_W0], P[EE_B0], P[EE_W2], E, nt_e,
-                                                            grad_edge_attr, nullptr, cws);
+    k_encoder_vjp<0, INST><<<dim3(grid_e, K), NT, SMEM_V2T, st>>>(V.ge, W.y_eenc, scal(1), P[EE_LNW], nullptr, nullptr, nullptr,
+                                                                  edge_attr, perm, *norm, scale_in, P[EE_W0], P[EE_B0], P[EE_W2],
+                                                                  E, nt_e, grad_edge_attr, nullptr, cws, M, iws, ea_stride, 0);
   }
   if (ig_edge) PDG_LAUNCH_CHECK();
   return 0;
+}
+
+}  // namespace pdg
+
+extern "C" int pdg_vjp_batched(const pdg_params_t* params, const pdg_norm_t* norm, const float* mean_stress, const float* pos,
+                               const int64_t* nodes_types, const float* edge_attr, const void* plan, int64_t n_nodes,
+                               int64_t n_edges, int steps, int flags, int precision, const void* fwd_ws, void* vjp_ws,
+                               size_t vjp_ws_bytes, int n_cotangents, const float* grad_local_stress, float* grad_mean_stress,
+                               float* grad_pos, float* grad_edge_attr, void* stream_) {
+  return vjp_run<false>("pdg_vjp_batched", params, norm, mean_stress, 0, pos, 0, nodes_types, edge_attr, 0, plan, n_nodes,
+                        n_edges, steps, flags, precision, fwd_ws, 1, vjp_ws, vjp_ws_bytes, n_cotangents, grad_local_stress,
+                        grad_mean_stress, grad_pos, grad_edge_attr, (cudaStream_t)stream_);
+}
+
+extern "C" int pdg_vjp_instances(const pdg_params_t* params, const pdg_norm_t* norm, const float* mean_stress, int64_t ms_stride,
+                                 const float* pos, int64_t pos_stride, const int64_t* nodes_types, const float* edge_attr,
+                                 int64_t ea_stride, const void* plan, int64_t n_nodes, int64_t n_edges, int steps, int flags,
+                                 int precision, const void* fwd_ws, int n_instances, void* vjp_ws, size_t vjp_ws_bytes,
+                                 int n_cotangents, const float* grad_local_stress, float* grad_mean_stress, float* grad_pos,
+                                 float* grad_edge_attr, void* stream_) {
+  return vjp_run<true>("pdg_vjp_instances", params, norm, mean_stress, ms_stride, pos, pos_stride, nodes_types, edge_attr,
+                       ea_stride, plan, n_nodes, n_edges, steps, flags, precision, fwd_ws, n_instances, vjp_ws, vjp_ws_bytes,
+                       n_cotangents, grad_local_stress, grad_mean_stress, grad_pos, grad_edge_attr, (cudaStream_t)stream_);
 }
